@@ -3,6 +3,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...        # the reference's CPU algorithm (oracle port) on the host cores
+    python bench.py --dump-outputs DIR ...      # also write what the last timed step computed, as DIR/<name>.npy
 
 A "step" is one pass of the hot path over the whole workload (all genes x all groups).  `value` is gene x group tests
 per second with the input resident in HBM; `e2e` is the same metric through the public `asymptotic_wilcoxon` call with
@@ -29,6 +30,10 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (which may be read-only)
+
+DUMP_MAX_TESTS = 1 << 20         # --dump-outputs: at most this many tests (32 MB with the index), a fixed sample beyond
+DUMP_SEED = 0
 
 # name: format, test, data kind, description (BASELINE.json config it belongs to)
 WORKLOADS = {
@@ -75,7 +80,16 @@ def parse():
     ap.add_argument("--others", default="auto",
                     help="'auto' (the default line at N=1 carries every other workload), 'none', or a comma list")
     ap.add_argument("--seed", type=int, default=0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the results of the last one as DIR/p_value.npy, statistic.npy, "
+                         "fold_change.npy (float64) and test_index.npy (the flat index group * genes + gene of each "
+                         f"entry, float64): every test, or a fixed seeded sample of {DUMP_MAX_TESTS} of them (rank 0)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the results of the b200 path")
+    return a
 
 
 def shape_of(a, spec):
@@ -310,10 +324,11 @@ class Workload:
             dist.barrier()
         torch.cuda.synchronize(self.dev)
 
-    def timed(self, steps, warmup, min_load_s=0.6, post_load_s=0.3):
+    def timed(self, steps, warmup, min_load_s=0.6, post_load_s=0.3, keep=None):
         """K timed steps (CUDA events, max over ranks) inside a longer stretch of the same load: a step takes a few
         milliseconds, far below nvidia-smi's sampling period, and the SM clock needs tens of milliseconds of load to
-        reach its boost state."""
+        reach its boost state.  ``keep`` (flat test indices on the device): those rows of the last timed step's
+        results are copied to ``self.kept`` before the steps after the timed window overwrite them."""
         import torch
         import torch.distributed as dist
 
@@ -331,6 +346,8 @@ class Workload:
             self.step()
         e1.record()
         launches = self._lib.launch_count() - l0
+        if keep is not None:
+            self.kept = self.results.view(-1, 3).index_select(0, keep)
         t_post = time.perf_counter()
         while time.perf_counter() - t_post < post_load_s:
             self.step()
@@ -535,6 +552,21 @@ def cpu_run(Xhost, labels, reference, sample, threads):
     return P.counts.size * sample / dt, dt
 
 
+def dump_sample(n_tests):
+    """Flat test indices (group * genes + gene) that --dump-outputs writes: all of them, or a fixed seeded sample."""
+    if n_tests <= DUMP_MAX_TESTS:
+        return np.arange(n_tests, dtype=np.int64)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n_tests, DUMP_MAX_TESTS, replace=False)).astype(np.int64)
+
+
+def dump_outputs(directory, kept, index):
+    """``kept[i]`` = (p_value, statistic, fold_change) of test ``index[i]``: one float64 .npy file per column."""
+    os.makedirs(directory, exist_ok=True)
+    for k, name in enumerate(("p_value", "statistic", "fold_change")):
+        np.save(os.path.join(directory, f"{name}.npy"), np.ascontiguousarray(kept[:, k], dtype=np.float64))
+    np.save(os.path.join(directory, "test_index.npy"), index.astype(np.float64))
+
+
 def cpu_sample_size(a, fmt, genes, threads):
     return a.cpu_sample_genes or min(genes, (32 if fmt == "dense" else 256) * threads)
 
@@ -582,11 +614,16 @@ def main():
 
     # ---- headline workload: weak scaling, every rank owns a full-size gene shard
     w = Workload(a.workload, a, dev, rank, world)
+    dump_index = dump_sample(w.n_tests) if a.dump_outputs and rank == 0 else None
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms_step, launches, n_warm = w.timed(a.steps, a.warmup)
+    ms_step, launches, n_warm = w.timed(a.steps, a.warmup, keep=None if dump_index is None else
+                                        torch.from_numpy(dump_index).to(dev))
     clocks = sampler.stop() if rank == 0 else None
+    if dump_index is not None:
+        dump_outputs(a.dump_outputs, w.kept.cpu().numpy(), dump_index)
+        del w.kept
     if clocks is not None:
         clocks["window"] = (f"{n_warm} warm-up steps (>= 0.6 s of the same load) + the {a.steps} timed steps + 0.3 s of the "
                             "same load")

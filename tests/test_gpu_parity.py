@@ -1045,3 +1045,38 @@ def test_packed_upload_rebuilds_the_matrix(monkeypatch, source):
         assert st["raw"] >= 2
     if source in ("pageable", "shard"):
         assert st["raw"] == 0 and st["bytes"] < 0.35 * src.size * 4
+
+
+def test_bench_steps_and_dumped_outputs(tmp_path):
+    """bench.py: `--steps K` times K steps (K times the launches of one), and `--dump-outputs` writes what the last timed
+    step computed -- on the benchmark's own seeded inputs, the oracle's results."""
+    import json
+    import subprocess
+    import sys
+
+    import torch
+
+    import bench
+
+    root = os.path.dirname(os.path.abspath(bench.__file__))
+    cells, genes, perts = 3000, 40, 10
+    args = [sys.executable, os.path.join(root, "bench.py"), "--cells", str(cells), "--genes", str(genes), "--perts",
+            str(perts), "--warmup", "1", "--no-e2e", "--no-cpu-baseline", "--others", "none"]
+    lines = {}
+    for steps in (1, 3):
+        out = subprocess.check_output(args + ["--steps", str(steps), "--dump-outputs", str(tmp_path / str(steps))],
+                                      text=True, cwd=root)
+        lines[steps] = json.loads(out.strip().splitlines()[-1])
+    assert lines[3]["steps"] == 3 and lines[1]["gpu_launches"] > 0
+    assert lines[3]["gpu_launches"] == 3 * lines[1]["gpu_launches"]
+
+    labels, reference = bench.make_labels(0, cells, perts, bench.WORKLOADS["dense_ovo"])
+    X = bench.gen_dense("counts", 17, cells, genes, torch.device("cuda", 0)).cpu().numpy()
+    groups, p, U, fc = oracle.run(X, labels, reference)
+    for steps in (1, 3):
+        d = tmp_path / str(steps)
+        got = [np.load(d / f"{k}.npy") for k in ("p_value", "statistic", "fold_change", "test_index")]
+        assert all(a.dtype == np.float64 and a.shape == (len(groups) * genes,) for a in got)
+        np.testing.assert_array_equal(got[3], np.arange(len(groups) * genes))
+        assert_parity(tuple(a.reshape(len(groups), genes) for a in got[:3]), (p, U, fc),
+                      ref_row=int(np.searchsorted(groups, reference)), what=f"bench --dump-outputs, {steps} steps")
