@@ -1,12 +1,12 @@
 """illico_b200 -- B200-native asymptotic Wilcoxon rank-sum (Mann-Whitney U) tests.
 
 Drop-in for the one hot path of remydubois/illico: ``asymptotic_wilcoxon(adata, ...)`` and the six
-batch dispatchers under it, computed by hand-written sm_100a CUDA kernels behind a C ABI
+batch dispatchers under it, plus ``rank_genes(adata, ...)`` (each group's genes ranked by score, selected on the GPU), computed by hand-written sm_100a CUDA kernels behind a C ABI
 (``include/illico_b200.h``).  There is no CPU fallback.
 """
 __version__ = "0.1.0"
 
-__all__ = ["asymptotic_wilcoxon", "register_into_reference", "__version__"]
+__all__ = ["asymptotic_wilcoxon", "rank_genes", "register_into_reference", "__version__"]
 
 
 def __getattr__(name):
@@ -15,6 +15,13 @@ def __getattr__(name):
         from .asymptotic_wilcoxon import asymptotic_wilcoxon as fn
 
         globals()["asymptotic_wilcoxon"] = fn  # rebind: the submodule import bound the module to this name
+        return fn
+    if name == "rank_genes":
+        from .asymptotic_wilcoxon import asymptotic_wilcoxon as aw
+        from .ranking import rank_genes as fn
+
+        # (importing .ranking imports the .asymptotic_wilcoxon submodule, which binds the module to that name)
+        globals().update(asymptotic_wilcoxon=aw, rank_genes=fn)
         return fn
     if name == "register_into_reference":
         from .registry import register_into_reference as fn

@@ -10,7 +10,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libillico_b200.so")
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 ALTERNATIVES = {"two-sided": 0, "less": 1, "greater": 2}
 TIES_DENSE, TIES_SPARSE = 0, 1
 
@@ -33,7 +33,15 @@ class Flags(C.Structure):
     """``illico_flags_t``"""
 
     _fields_ = [("is_log1p", _i32), ("use_continuity", _i32), ("tie_correct", _i32), ("alternative", _i32),
-                ("tie_order", _i32), ("n_cols_hint", _i32), ("group_sums", _vp)]
+                ("tie_order", _i32), ("n_cols_hint", _i32), ("group_sums", _vp), ("scores", _vp),
+                ("score_group_stride", _i64)]
+
+    def replace(self, **fields) -> "Flags":
+        """A copy with some fields changed."""
+        out = Flags.from_buffer_copy(self)
+        for k, v in fields.items():
+            setattr(out, k, v)
+        return out
 
 
 class Debug(C.Structure):
@@ -87,6 +95,8 @@ SIGNATURES = {
     "illico_unpack_rows_f32": (C.c_int, [_vp, _vp, _vp, _i64, _i32, _vp, _i64, _vp]),
     "illico_bh_workspace_bytes": (_sz, [_i32, _i32]),
     "illico_bh_adjust": (C.c_int, [_vp, _i64, _i64, _i32, _i32, _vp, _vp, _sz, _vp]),
+    "illico_top_genes_workspace_bytes": (_sz, [_i32, _i32]),
+    "illico_top_genes": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _sz, _vp]),
     "illico_compute_pval_batch": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
 }
 

@@ -113,6 +113,7 @@ def asymptotic_wilcoxon(
     return_array: bool = False,
     p_adjust: bool = False,
     log2_fold_change: bool = False,
+    score: bool = False,
 ):
     """Asymptotic Mann-Whitney / Wilcoxon rank-sum tests for every (group, gene) on B200 GPUs.
 
@@ -128,9 +129,46 @@ def asymptotic_wilcoxon(
                    (the reference's thread pool over gene batches, ``asymptotic_wilcoxon.py:212-249``, across GPUs);
       ``return_array``  return ``(groups, var_names, results[G, N, 3])`` and skip the DataFrame;
       ``p_adjust`` / ``log2_fold_change``  add the columns ``p_adj`` (Benjamini-Hochberg over the genes of each group,
-                   what ``scanpy.tl.rank_genes_groups`` reports as ``pvals_adj``) and ``log2_fold_change``.
+                   what ``scanpy.tl.rank_genes_groups`` reports as ``pvals_adj``) and ``log2_fold_change``;
+      ``score``    add the column ``score``: the signed z of the normal approximation, ``(n_r n_t / 2 - U) / sigma`` with
+                   the p-value's (tie-corrected) sigma and no continuity correction -- positive when the group ranks above
+                   the reference / rest, 0 on the reference row and where p = 1 (scanpy's wilcoxon ``scores``).  Written
+                   by the kernels next to the p-value.
+    With ``return_array`` and an optional column, the result is ``(groups, var_names, results, {name: [G, N] array})``.
     """
     del precompile  # kernels are compiled ahead of time
+    run = _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, alternative, use_continuity,
+                     tie_correct, layer, device, devices, score=score, on_device=False)
+    out = run.results
+    extra = {}
+    if p_adjust:
+        extra["p_adj"] = _bh_adjust(out, run.device)
+    if log2_fold_change:
+        with np.errstate(divide="ignore", invalid="ignore"):
+            extra["log2_fold_change"] = np.log2(out[:, :, 2])
+    if score:
+        extra["score"] = run.scores
+    if return_array:
+        if extra:
+            return run.groups, np.asarray(adata.var_names), out, extra
+        return run.groups, np.asarray(adata.var_names), out
+    return _result_frame(run.groups, adata.var_names, out, extra)
+
+
+class _Run:
+    """What ``_run_tests`` delivers: the groups (``np.unique`` order), the group container, the first GPU, and the results
+    ``[G, N, 3]`` / score plane ``[G, N]`` (None unless asked for) -- pinned host arrays, or tensors on that GPU."""
+
+    def __init__(self, groups, grpc, device, results, scores):
+        self.groups, self.grpc, self.device, self.results, self.scores = groups, grpc, device, results, scores
+
+
+def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, alternative, use_continuity, tie_correct,
+               layer, device, devices, score: bool, on_device: bool) -> _Run:
+    """Every (group, gene) test of ``adata``: validation, upload, group plan, one gene shard per GPU, batches, backed
+    streaming.  ``on_device=False``: each shard's slabs are copied into pinned host arrays (``asymptotic_wilcoxon``).
+    ``on_device=True``: they stay on the GPUs and meet in ``[G, N, 3]`` / ``[G, N]`` tensors on the first one
+    (device-to-device copies; with one shard its own tensors are the result)."""
     X = adata.layers[layer] if layer is not None else adata.X
     if isinstance(X, (sparse.csr_array, sparse.csc_array)):
         X = sparse.csr_matrix(X) if isinstance(X, sparse.csr_array) else sparse.csc_matrix(X)
@@ -191,6 +229,7 @@ def asymptotic_wilcoxon(
                 engine = Engine(shared["grpc"], sh.device, host_plan=shared["host_plan"])
                 flags = flags_for()
                 res = torch.empty((engine.n_groups, sh.ub - sh.lb, 3), dtype=torch.float64, device=sh.device)
+                sc = torch.empty((engine.n_groups, sh.ub - sh.lb), dtype=torch.float64, device=sh.device) if score else None
                 if data_handler.in_ram:
                     M.ready()
                     if fmt == CSR and not engine.check_csr_sorted(M):
@@ -202,11 +241,17 @@ def asymptotic_wilcoxon(
                         )
                     off = bounds[0] - sh.lb      # gene g of the run is column g + off of the device matrix
                     for lb, ub in _batches(sh.lb, sh.ub, batch_size, engine, True):
-                        engine.run_batch(M, lb + off, ub + off, flags, res, lb - sh.lb)
+                        engine.run_batch(M, lb + off, ub + off, flags, res, lb - sh.lb, scores=sc)
                 else:
                     _run_backed(data_handler, _batches(sh.lb, sh.ub, batch_size, engine, False), engine, flags, res,
-                                max(1, int(n_threads)), gene0=sh.lb)
-                hostio.d2h_slab(shared["host"], res, sh.lb)
+                                max(1, int(n_threads)), gene0=sh.lb, scores=sc)
+                if on_device and len(shards) == 1:
+                    shared["out"], shared["out_scores"] = res, sc
+                else:
+                    kind = "d2d" if on_device else "d2h"
+                    hostio.d2h_slab(shared["out"], res, sh.lb, kind)
+                    if sc is not None:
+                        hostio.d2h_slab(shared["out_scores"], sc, sh.lb, kind)
                 torch.cuda.current_stream(sh.device).synchronize()
         except BaseException as e:  # re-raised on the calling thread
             sh.error = e
@@ -231,7 +276,12 @@ def asymptotic_wilcoxon(
 
         shared["grpc"], shared["host_plan"] = grpc, build_plan(grpc, _seg_max())
         G = int(grpc.counts.size)
-        shared["host"] = torch.empty((G, n_genes, 3), dtype=torch.float64, pin_memory=True)
+        if not on_device:
+            shared["out"] = torch.empty((G, n_genes, 3), dtype=torch.float64, pin_memory=True)
+            shared["out_scores"] = torch.empty((G, n_genes), dtype=torch.float64, pin_memory=True) if score else None
+        elif len(shards) > 1:
+            shared["out"] = torch.empty((G, n_genes, 3), dtype=torch.float64, device=devs[0])
+            shared["out_scores"] = torch.empty((G, n_genes), dtype=torch.float64, device=devs[0]) if score else None
     except BaseException:
         shared["error"] = True
         plan_ready.set()
@@ -247,18 +297,10 @@ def asymptotic_wilcoxon(
     for sh in shards:
         if sh.error is not None:
             raise sh.error
-    out = shared["host"].numpy()
-    extra = {}
-    if p_adjust:
-        extra["p_adj"] = _bh_adjust(out, shards[0].device)
-    if log2_fold_change:
-        with np.errstate(divide="ignore", invalid="ignore"):
-            extra["log2_fold_change"] = np.log2(out[:, :, 2])
-    if return_array:
-        if extra:
-            return unique_raw_groups, np.asarray(adata.var_names), out, extra
-        return unique_raw_groups, np.asarray(adata.var_names), out
-    return _result_frame(unique_raw_groups, adata.var_names, out, extra)
+    out, scores = shared["out"], shared["out_scores"]
+    if not on_device:
+        out, scores = out.numpy(), (scores.numpy() if scores is not None else None)
+    return _Run(unique_raw_groups, grpc, shards[0].device, out, scores)
 
 
 def _bh_adjust(out: np.ndarray, device) -> np.ndarray:
@@ -334,7 +376,8 @@ class _PinnedSlot:
         return view
 
 
-def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, results, n_readers: int, gene0: int = 0) -> None:
+def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, results, n_readers: int, gene0: int = 0,
+                scores=None) -> None:
     """Out-of-core input (BASELINE config 4): gene batches stream disk -> pinned ring -> HBM -> kernels.
 
     Reader threads slice the next batches from the backed container straight into pinned staging buffers (a ring of
@@ -420,7 +463,7 @@ def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, resu
             if data.dtype != torch.float32:
                 data, raw = _to_f32_or_wide(data)
             M = DeviceMatrix(fmt, tuple(shape), data, dv["indices"], dv["indptr"], raw=raw)
-        engine.run_batch(M, bounds[0], bounds[1], flags, results, lb - gene0)
+        engine.run_batch(M, bounds[0], bounds[1], flags, results, lb - gene0, scores=scores)
 
     try:
         while done < n_readers:

@@ -161,10 +161,14 @@ int64_t illico_profile_report(char* out, int64_t cap) {
 int illico_memcpy2d_async(void* dst, size_t dpitch, const void* src, size_t spitch, size_t width_bytes, size_t height,
                           int kind, void* stream) {
     if (!dst || !src) { set_error("illico_memcpy2d_async: NULL pointer"); return 1; }
-    if (kind != 1 && kind != 2) { set_error("illico_memcpy2d_async: kind must be 1 (host to device) or 2 (device to host)"); return 1; }
+    if (kind < 1 || kind > 3) {
+        set_error("illico_memcpy2d_async: kind must be 1 (host to device), 2 (device to host) or 3 (device to device)");
+        return 1;
+    }
     if (width_bytes == 0 || height == 0) return 0;
-    ILLICO_CUDA_OK(cudaMemcpy2DAsync(dst, dpitch, src, spitch, width_bytes, height,
-                                     kind == 1 ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+    // device to device: cudaMemcpyDefault lets the driver route a copy between two GPUs (peer or staged)
+    const cudaMemcpyKind k = kind == 1 ? cudaMemcpyHostToDevice : kind == 2 ? cudaMemcpyDeviceToHost : cudaMemcpyDefault;
+    ILLICO_CUDA_OK(cudaMemcpy2DAsync(dst, dpitch, src, spitch, width_bytes, height, k, (cudaStream_t)stream));
     return 0;
 }
 

@@ -10,6 +10,11 @@
 
 namespace illico {
 
+// sigma = sqrt(n_ref * n_tgt * (n_ref + n_tgt + 1) / 12.0 * tie_corr)
+__device__ __forceinline__ double pval_sigma(double prod12, double tie_corr) {
+    return __dsqrt_rn(__dmul_rn(prod12, tie_corr));
+}
+
 // The part of compute_pval after the quantities that only depend on the group sizes: nrnt = float(n_ref * n_tgt),
 // mu = nrnt / 2, prod12 = float(n_ref * n_tgt * (n_ref + n_tgt + 1)) / 12.0, tie_corr = 1 - tie_sum / float(n (n-1) (n+1)).
 // The fused epilogue takes those from a per-group table (same operations, so the same bits, evaluated once per group
@@ -17,8 +22,7 @@ namespace illico {
 __device__ __forceinline__ double pval_core(double nrnt, double mu, double prod12, double tie_corr, double U, double cc,
                                             int alternative) {
     if (!(tie_corr > 1.0e-9)) return 1.0;
-    // sigma = sqrt(n_ref * n_tgt * (n_ref + n_tgt + 1) / 12.0 * tie_corr)
-    const double sigma = __dsqrt_rn(__dmul_rn(prod12, tie_corr));
+    const double sigma = pval_sigma(prod12, tie_corr);
     const double sqrt2 = 1.4142135623730951;  // math.sqrt(2.0)
     if (alternative == ILLICO_TWO_SIDED) {
         const double other = __dsub_rn(nrnt, U);
@@ -36,6 +40,23 @@ __device__ __forceinline__ double pval_core(double nrnt, double mu, double prod1
         const double z = __ddiv_rn(__dadd_rn(delta, cc), sigma);
         return __dmul_rn(0.5, erfc(__ddiv_rn(-z, sqrt2)));
     }
+}
+
+// Signed effect score (illico_flags_t::scores): (mu - U) / sigma with the p-value's sigma, no continuity correction --
+// the z of the normal approximation, positive when the group ranks above the reference / rest.  0 where the p-value is 1
+// (tie correction <= 1e-9); NaN where sigma = 0 otherwise (a one-versus-rest run with a single group, where p is NaN).
+__device__ __forceinline__ double score_core(double mu, double prod12, double tie_corr, double U) {
+    if (!(tie_corr > 1.0e-9)) return 0.0;
+    return __ddiv_rn(__dsub_rn(mu, U), pval_sigma(prod12, tie_corr));
+}
+
+// score_core from the group sizes and the tie sum, with compute_pval's operations
+__device__ __forceinline__ double compute_score(long long n_ref, long long n_tgt, long long n, double tie_sum, double U,
+                                                double mu) {
+    const double denom = (double)(n * (n - 1) * (n + 1));
+    const double tie_corr = __dsub_rn(1.0, __ddiv_rn(tie_sum, denom));
+    const double prod12 = __ddiv_rn((double)(n_ref * n_tgt * (n_ref + n_tgt + 1)), 12.0);
+    return score_core(mu, prod12, tie_corr, U);
 }
 
 __device__ __forceinline__ double compute_pval(long long n_ref, long long n_tgt, long long n, double tie_sum,

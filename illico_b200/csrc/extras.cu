@@ -5,6 +5,8 @@
 //                              (reference tests/test_asymptotic_wilcoxon.py:30-60).  Same operation order as
 //                              statsmodels' multipletests(method="fdr_bh"): p_sorted / (k / N), reverse running minimum,
 //                              clipped at 1.
+//   illico_top_genes           ranks the genes of each group by score (stable radix sort of order-preserving keys carrying
+//                              the gene index) and gathers the first k genes' records: scanpy's rank_genes_groups order.
 //   illico_compute_pval_batch  evaluates the epilogue's compute_pval (epilogue.cuh; reference illico/utils/math.py:64-118)
 //                              on arrays of arguments, so the known-answer vectors of tests/golden/primitives.npz can be
 //                              checked against the device code itself.
@@ -76,6 +78,56 @@ __global__ void __launch_bounds__(BH_THREADS) bh_adjust_kernel(const double* __r
     }
 }
 
+// Per-group ranking (illico_top_genes): one CTA per group (grid-strided), like bh_adjust_kernel.  The key of gene j is the
+// order-preserving u64 image of its score, complemented so that an ascending sort puts the largest score first; NaN keys
+// are all-ones (after every number).  The gene indices ride along as the payload: they go in ascending, and the sort is
+// stable, so equal scores stay in index order.
+__device__ __forceinline__ unsigned long long score_key_desc(double x, int by_abs) {
+    if (x != x) return ~0ull;
+    if (by_abs) x = fabs(x);
+    if (x == 0.0) x = 0.0;                                              // -0.0 sorts as +0.0
+    const unsigned long long u = (unsigned long long)__double_as_longlong(x);
+    const unsigned long long asc = (u >> 63) ? ~u : (u | 0x8000000000000000ull);
+    return ~asc;
+}
+
+__global__ void __launch_bounds__(BH_THREADS) top_genes_kernel(const double* __restrict__ score, long long score_stride,
+                                                               const double* __restrict__ res, long long res_stride,
+                                                               const double* __restrict__ padj, int G, int N, int k, int by_abs,
+                                                               int* __restrict__ out_gene, double* __restrict__ out_rec,
+                                                               unsigned long long* __restrict__ slab) {
+    __shared__ uint32_t hist[BH_NW * 256];
+    __shared__ uint32_t aux[RADIX_AUX_WORDS];
+    const int tid = threadIdx.x;
+    unsigned long long* A = slab + (long long)blockIdx.x * 3 * N;
+    unsigned long long* B = A + N;
+    uint32_t* IA = reinterpret_cast<uint32_t*>(B + N);
+    uint32_t* IB = IA + N;
+    for (int g = blockIdx.x; g < G; g += gridDim.x) {
+        const double* sg = score + (long long)g * score_stride;
+        for (int j = tid; j < N; j += BH_THREADS) {
+            A[j] = score_key_desc(sg[j], by_abs);
+            IA[j] = (uint32_t)j;
+        }
+        __syncthreads();
+        const unsigned long long* S = block_radix_sort_t<unsigned long long, uint32_t>(A, B, N, hist, aux, IA, IB);
+        const uint32_t* idx = (S == A) ? IA : IB;
+        const double* rg = res + (long long)g * res_stride;
+        for (int r = tid; r < k; r += BH_THREADS) {
+            const int j = (int)idx[r];
+            const long long o = (long long)g * k + r;
+            out_gene[o] = j;
+            double* rec = out_rec + o * 5;
+            rec[0] = sg[j];
+            rec[1] = rg[3 * (long long)j];
+            rec[2] = rg[3 * (long long)j + 1];
+            rec[3] = rg[3 * (long long)j + 2];
+            rec[4] = padj ? padj[(long long)g * N + j] : NAN;
+        }
+        __syncthreads();
+    }
+}
+
 __global__ void compute_pval_batch_kernel(const long long* n_ref, const long long* n_tgt, const long long* n, const double* tie,
                                           const double* U, const double* mu, const double* cc, const int* alt, double* out,
                                           long long count) {
@@ -137,6 +189,34 @@ int illico_bh_adjust(const double* p_values, int64_t group_stride, int64_t gene_
     cudaStream_t st = (cudaStream_t)stream;
     ILLICO_LAUNCH("bh_adjust_kernel", st,
                   bh_adjust_kernel<<<ctas, BH_THREADS, 0, st>>>(p_values, group_stride, gene_stride, n_groups, n_genes, p_adj, slab));
+    ILLICO_CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
+size_t illico_top_genes_workspace_bytes(int32_t n_groups, int32_t n_genes) {
+    long long ctas = n_groups < 148 * 2 ? n_groups : 148 * 2;
+    if (ctas < 1) ctas = 1;
+    // per CTA: two u64 key buffers and two u32 index buffers of n_genes
+    return (size_t)ctas * 3 * (size_t)(n_genes > 0 ? n_genes : 1) * sizeof(unsigned long long) + 256;
+}
+
+int illico_top_genes(const double* scores, int64_t score_group_stride, const double* results, int64_t result_group_stride,
+                     const double* p_adj, int32_t n_groups, int32_t n_genes, int32_t k, int32_t by_abs, int32_t* out_gene,
+                     double* out_rec, void* workspace, size_t workspace_bytes, void* stream) {
+    if (!scores || !results || !out_gene || !out_rec || !workspace) { set_error("illico_top_genes: NULL argument"); return 1; }
+    if (n_groups <= 0 || n_genes <= 0) return 0;
+    if (k < 1 || k > n_genes) { set_error("illico_top_genes: k = %d outside [1, %d]", k, n_genes); return 1; }
+    if (workspace_bytes < illico_top_genes_workspace_bytes(n_groups, n_genes)) {
+        set_error("illico_top_genes: workspace too small");
+        return 1;
+    }
+    const int ctas = n_groups < 148 * 2 ? n_groups : 148 * 2;
+    unsigned long long* slab =
+        reinterpret_cast<unsigned long long*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
+    cudaStream_t st = (cudaStream_t)stream;
+    ILLICO_LAUNCH("top_genes_kernel", st,
+                  top_genes_kernel<<<ctas, BH_THREADS, 0, st>>>(scores, score_group_stride, results, result_group_stride, p_adj,
+                                                                n_groups, n_genes, k, by_abs ? 1 : 0, out_gene, out_rec, slab));
     ILLICO_CUDA_OK(cudaGetLastError());
     return 0;
 }

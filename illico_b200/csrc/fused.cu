@@ -815,7 +815,9 @@ __global__ void __launch_bounds__(256) fused_group_kernel(const illico_plan_t pl
 // its divisions by the group sizes are multiplications by precomputed reciprocals; everything that feeds the p-value
 // keeps the reference's IEEE operations.
 constexpr int EPI_GROUPS = 16;   // groups per thread
-template <bool OVO, bool WIDE>
+// SCORE: also writes the score plane (illico_flags_t::scores); a separate instantiation, so that the default call's
+// epilogue is the same code as without the plane.
+template <bool OVO, bool WIDE, bool SCORE>
 __global__ void __launch_bounds__(256, 3) fused_epilogue_kernel(int b, const illico_plan_t pl, const illico_flags_t fl, Gtab gt,
                                                              int bs, double* __restrict__ results, long long gstride,
                                                              long long* dbg_u2, double* dbg_tie, long long* dbg_tie_exact,
@@ -868,6 +870,7 @@ __global__ void __launch_bounds__(256, 3) fused_epilogue_kernel(int b, const ill
         if (OVO && g == ref) {
             // control row: (1, -1, fold change of the control against itself), as ovo_kernel writes it
             o[0] = 1.0; o[1] = -1.0; o[2] = (ovo_mean_r == 0.0) ? INFINITY : ovo_mean_r / ovo_mean_r;
+            if (SCORE) fl.scores[(long long)g * fl.score_group_stride + j] = 0.0;
             if (dbg_u2) dbg_u2[di] = -2;
             if (dbg_tie) dbg_tie[di] = 0.0;
             if (dbg_tie_exact) dbg_tie_exact[di] = 0;
@@ -910,6 +913,7 @@ __global__ void __launch_bounds__(256, 3) fused_epilogue_kernel(int b, const ill
             U = (double)u2 * 0.5;
             const double tie_corr = __dsub_rn(1.0, __ddiv_rn(fl.tie_correct ? tie : 0.0, gcs[GC_DENOM][k]));
             p = pval_core(gcs[GC_NRNT][k], gcs[GC_MU][k], gcs[GC_PROD12][k], tie_corr, U, cc, fl.alternative);
+            if (SCORE) fl.scores[(long long)g * fl.score_group_stride + j] = score_core(gcs[GC_MU][k], gcs[GC_PROD12][k], tie_corr, U);
             fc = (ovo_mean_r == 0.0) ? INFINITY : (sum * gcs[GC_INV_NT][k]) * ovo_inv_mean_r;
             if (dbg_u2) dbg_u2[di] = (long long)u2;
             if (dbg_tie) dbg_tie[di] = tie;
@@ -919,6 +923,8 @@ __global__ void __launch_bounds__(256, 3) fused_epilogue_kernel(int b, const ill
             const long long u2 = 2 * n_r * n_t + n_t * (n_t + 1) - (long long)R2;
             U = (double)u2 * 0.5;
             p = pval_core(gcs[GC_NRNT][k], gcs[GC_MU][k], gcs[GC_PROD12][k], ovr_tie_corr, U, cc, fl.alternative);
+            if (SCORE)
+                fl.scores[(long long)g * fl.score_group_stride + j] = score_core(gcs[GC_MU][k], gcs[GC_PROD12][k], ovr_tie_corr, U);
             // rest-of-cells mean: exactly zero when this group holds every non-zero of the gene (the reference's total is
             // the sum of the per-group sums, so its `total - sum` is an exact 0 there; a total accumulated in another
             // order could leave an ulp and turn the +inf fold change into 1e16)
@@ -1405,11 +1411,15 @@ int run_fused(const float* X, long long ld, int gene_lb, int b, const illico_pla
     ILLICO_LAUNCH("fused_group_kernel", stream, fused_group_kernel<OVO><<<(plan->n_groups + 255) / 256, 256, 0, stream>>>(*plan, gt));
     ILLICO_LAUNCH("fused_gene_kernel", stream, fused_gene_kernel<OVO><<<(b + 127) / 128, 128, 0, stream>>>(b, *plan, *flags, gt, bs, nullptr, nullptr));
     ILLICO_CUDA_OK(cudaGetLastError());
-    ILLICO_LAUNCH("fused_epilogue_kernel", stream, fused_epilogue_kernel<OVO, false><<<dim3((unsigned)((b + 255) / 256), (unsigned)((plan->n_groups + EPI_GROUPS - 1) / EPI_GROUPS)), 256, 0, stream>>>(
+    const bool score = flags->scores != nullptr;
+    auto epi = score ? fused_epilogue_kernel<OVO, false, true> : fused_epilogue_kernel<OVO, false, false>;
+    ILLICO_LAUNCH("fused_epilogue_kernel", stream, epi<<<dim3((unsigned)((b + 255) / 256), (unsigned)((plan->n_groups + EPI_GROUPS - 1) / EPI_GROUPS)), 256, 0, stream>>>(
             b, *plan, *flags, gt, bs, results, gstride, nullptr, nullptr, nullptr, list_share_1024()));
-    if (wide_on)
-        ILLICO_LAUNCH("fused_wide_epilogue_kernel", stream, fused_epilogue_kernel<OVO, true><<<dim3((unsigned)((b + 255) / 256), (unsigned)((plan->n_groups + EPI_GROUPS - 1) / EPI_GROUPS)), 256, 0, stream>>>(
+    if (wide_on) {
+        auto wepi = score ? fused_epilogue_kernel<OVO, true, true> : fused_epilogue_kernel<OVO, true, false>;
+        ILLICO_LAUNCH("fused_wide_epilogue_kernel", stream, wepi<<<dim3((unsigned)((b + 255) / 256), (unsigned)((plan->n_groups + EPI_GROUPS - 1) / EPI_GROUPS)), 256, 0, stream>>>(
                 b, *plan, *flags, gt, bs, results, gstride, nullptr, nullptr, nullptr, list_share_1024()));
+    }
     ILLICO_CUDA_OK(cudaGetLastError());
 
     // 4. genes handed back: listed on the device, staged from the matrix by a persistent kernel, ranked by the general
@@ -1516,7 +1526,8 @@ int run_fused_csr(const float* data, const int32_t* indices, const long long* in
     }
     ILLICO_LAUNCH("fused_group_kernel", stream, fused_group_kernel<OVO><<<(plan->n_groups + 255) / 256, 256, 0, stream>>>(*plan, gt));
     ILLICO_LAUNCH("fused_gene_kernel", stream, fused_gene_kernel<OVO><<<(b + 127) / 128, 128, 0, stream>>>(b, *plan, *flags, gt, bs, nullptr, nullptr));
-    ILLICO_LAUNCH("fused_epilogue_kernel", stream, fused_epilogue_kernel<OVO, false><<<dim3((unsigned)((b + 255) / 256), (unsigned)((G + EPI_GROUPS - 1) / EPI_GROUPS)), 256, 0, stream>>>(
+    auto epi = flags->scores ? fused_epilogue_kernel<OVO, false, true> : fused_epilogue_kernel<OVO, false, false>;
+    ILLICO_LAUNCH("fused_epilogue_kernel", stream, epi<<<dim3((unsigned)((b + 255) / 256), (unsigned)((G + EPI_GROUPS - 1) / EPI_GROUPS)), 256, 0, stream>>>(
             b, *plan, *flags, gt, bs, results, gstride, nullptr, nullptr, nullptr, 128));   // (the CSR pass stops at an eighth)
     ILLICO_CUDA_OK(cudaGetLastError());
 

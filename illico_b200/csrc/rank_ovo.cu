@@ -267,6 +267,7 @@ __device__ __noinline__ double ordered_pair_tie(const uint32_t* A, int nA, const
     return acc;
 }
 
+template <bool SCORE>
 __device__ __forceinline__ void finalize_group(const OvoParams& P, const RefInfo& R, int j, int g, long long m,
                                                unsigned long long u2, unsigned long long tie_nz, double sum,
                                                const uint32_t* gkeys = nullptr, int gstride = 1) {
@@ -289,6 +290,7 @@ __device__ __forceinline__ void finalize_group(const OvoParams& P, const RefInfo
     const double* gc = P.gc + g;
     const double tie_corr = __dsub_rn(1.0, __ddiv_rn(P.flags.tie_correct ? tie : 0.0, gc[3 * P.Gs]));
     const double p = pval_core(gc[1 * P.Gs], gc[0], gc[2 * P.Gs], tie_corr, U, cc, P.flags.alternative);
+    if (SCORE) P.flags.scores[(long long)g * P.flags.score_group_stride + jo] = score_core(gc[0], gc[2 * P.Gs], tie_corr, U);
     const double fc = (R.mean == 0.0) ? INFINITY : (sum * gc[4 * P.Gs]) * R.inv_mean;
     double* o = P.results + (long long)g * P.gstride + (long long)jo * 3;
     o[0] = p; o[1] = U; o[2] = fc;
@@ -311,7 +313,8 @@ __global__ void __launch_bounds__(256) ovo_group_consts_kernel(const illico_plan
     gc[4 * Gs + g] = 1.0 / (double)n_t;
 }
 
-template <int OVO_THREADS, int MIN_CTAS, bool LOG1P>
+// SCORE: also writes the score plane (illico_flags_t::scores), in an instantiation of its own
+template <int OVO_THREADS, int MIN_CTAS, bool LOG1P, bool SCORE>
 __global__ void __launch_bounds__(OVO_THREADS, MIN_CTAS) ovo_kernel(const OvoParams P) {
     constexpr int NT = OVO_THREADS;
     constexpr int OVO_NW = OVO_THREADS / 32;
@@ -613,6 +616,7 @@ __global__ void __launch_bounds__(OVO_THREADS, MIN_CTAS) ovo_kernel(const OvoPar
                     const int jo = P.gene_map ? P.gene_map[j] : j;
                     double* o = P.results + (long long)g * P.gstride + (long long)jo * 3;
                     o[0] = 1.0; o[1] = -1.0; o[2] = (R.mean == 0.0) ? INFINITY : R.mean / R.mean;
+                    if (SCORE) P.flags.scores[(long long)g * P.flags.score_group_stride + jo] = 0.0;
                     const long long di = (long long)g * P.n_cols + jo;
                     if (P.dbg_u2) P.dbg_u2[di] = -2;
                     if (P.dbg_tie) P.dbg_tie[di] = 0.0;
@@ -705,7 +709,7 @@ __global__ void __launch_bounds__(OVO_THREADS, MIN_CTAS) ovo_kernel(const OvoPar
                             rank_value(R, f2key(v), bq, u2, tie);
                             sum += (double)bq * fc_val<LOG1P>(v);
                         }
-                        finalize_group(P, R, j, g, m, u2, tie, sum);
+                        finalize_group<SCORE>(P, R, j, g, m, u2, tie, sum);
                         done = true;
                     }
                 } else if (!table && !big_pair && m <= STREAM_MAX) {
@@ -791,7 +795,7 @@ __global__ void __launch_bounds__(OVO_THREADS, MIN_CTAS) ovo_kernel(const OvoPar
                             take4(q4, min(4, c - 4 * i4));
                         }
                     }
-                    finalize_group(P, R, j, g, m, u2, tie, sum);
+                    finalize_group<SCORE>(P, R, j, g, m, u2, tie, sum);
                     done = true;
                 }
                 if (!done) {  // a whole warp (or the CTA) ranks this group by sorting it
@@ -840,7 +844,7 @@ __global__ void __launch_bounds__(OVO_THREADS, MIN_CTAS) ovo_kernel(const OvoPar
                 u2 = warp_sum_u64(u2);
                 tie = warp_sum_u64(tie);
                 sum = warp_sum_f64(sum);
-                if (lane == 0) finalize_group(P, R, j, g, m, u2, tie, sum, buf, 1);
+                if (lane == 0) finalize_group<SCORE>(P, R, j, g, m, u2, tie, sum, buf, 1);
                 __syncwarp();
             }
             __syncthreads();
@@ -873,7 +877,7 @@ __global__ void __launch_bounds__(OVO_THREADS, MIN_CTAS) ovo_kernel(const OvoPar
                 u2 = block_sum<unsigned long long>(u2, redu);
                 tie = block_sum<unsigned long long>(tie, redu);
                 sum = block_sum<double>(sum, redd);
-                if (tid == 0) finalize_group(P, R, j, g, m, u2, tie, sum, gk, 1);
+                if (tid == 0) finalize_group<SCORE>(P, R, j, g, m, u2, tie, sum, gk, 1);
                 __syncthreads();
             }
             __syncthreads();
@@ -896,7 +900,7 @@ size_t ovo_workspace_bytes(const illico_plan_t* plan, int n_ctas) {
     return ovo_head_bytes(plan) + (size_t)n_ctas * 4 * (size_t)plan->max_group_size * sizeof(uint32_t);
 }
 
-template <int NT, int MIN_CTAS, bool LOG1P>
+template <int NT, int MIN_CTAS, bool LOG1P, bool SCORE>
 static int launch_ovo_t(OvoParams& P, const illico_plan_t* plan, void* workspace, size_t workspace_bytes, int sms,
                         int max_smem, cudaStream_t stream) {
     constexpr int NW = NT / 32;
@@ -911,7 +915,7 @@ static int launch_ovo_t(OvoParams& P, const illico_plan_t* plan, void* workspace
     const size_t need = fixed + (size_t)(REF_CAP + scratch_words) * 4;
     if (need > (size_t)max_smem) { set_error("ovo_kernel needs %zu bytes of shared memory", need); return 1; }
     P.scratch_words = scratch_words;
-    auto kern = ovo_kernel<NT, MIN_CTAS, LOG1P>;
+    auto kern = ovo_kernel<NT, MIN_CTAS, LOG1P, SCORE>;
     ILLICO_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
     int occ = 0;
     ILLICO_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, need));
@@ -963,12 +967,17 @@ int launch_ovo_mapped(const float* ir_vals, const uint32_t* ir_cnt, int n_genes,
     P.dbg_tie_exact = dbg ? (long long*)dbg->tie_exact : nullptr;
     P.bucket_index = env_int("ILLICO_OVO_BUCKETS", 1);
     static const int nt = env_int("ILLICO_OVO_THREADS", 256);
+    const int v = (flags->is_log1p ? 1 : 0) | (flags->scores ? 2 : 0);
     if (nt == 512) {
-        if (flags->is_log1p) return launch_ovo_t<512, 2, true>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
-        return launch_ovo_t<512, 2, false>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
+        if (v == 0) return launch_ovo_t<512, 2, false, false>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
+        if (v == 1) return launch_ovo_t<512, 2, true, false>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
+        if (v == 2) return launch_ovo_t<512, 2, false, true>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
+        return launch_ovo_t<512, 2, true, true>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
     }
-    if (flags->is_log1p) return launch_ovo_t<256, 3, true>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
-    return launch_ovo_t<256, 3, false>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
+    if (v == 0) return launch_ovo_t<256, 3, false, false>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
+    if (v == 1) return launch_ovo_t<256, 3, true, false>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
+    if (v == 2) return launch_ovo_t<256, 3, false, true>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
+    return launch_ovo_t<256, 3, true, true>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
 }
 
 int launch_ovo(const float* ir_vals, const uint32_t* ir_cnt, int n_genes, const illico_plan_t* plan,

@@ -86,6 +86,8 @@ __device__ __forceinline__ double zero_block_term_f64(long long n0) {
     return __dsub_rn(c, x);
 }
 
+// SCORE: also writes the score plane (illico_flags_t::scores), in an instantiation of its own
+template <bool SCORE>
 __global__ void __launch_bounds__(OVR_THREADS, 2) ovr_kernel(const OvrParams P) {
     extern __shared__ __align__(16) uint32_t smem[];
     const int tid = threadIdx.x, lane = tid & 31;
@@ -396,6 +398,8 @@ __global__ void __launch_bounds__(OVR_THREADS, 2) ovr_kernel(const OvrParams P) 
             const double U = (double)u2 / 2.0;
             const double mu = (double)(n_r * n_t) / 2.0;
             const double p = compute_pval(n_r, n_t, n, P.flags.tie_correct ? tie : 0.0, U, mu, cc, P.flags.alternative);
+            if (SCORE)
+                P.flags.scores[(long long)g * P.flags.score_group_stride + jo] = compute_score(n_r, n_t, n, P.flags.tie_correct ? tie : 0.0, U, mu);
             double* o = P.results + (long long)g * P.gstride + (long long)jo * 3;
             o[0] = p; o[1] = U; o[2] = sum;
             my_total += sum;
@@ -433,6 +437,7 @@ __global__ void __launch_bounds__(OVR_THREADS, 2) ovr_kernel(const OvrParams P) 
 // A segment with more than 255 stored values could overflow an 8-bit bin: such a gene keeps 16-bit bins only
 // and its second pass re-reads the values (the round-1 two-pass scheme).  A gene with more distinct values is
 // appended to `todo` for the general kernel.
+template <bool SCORE>
 __global__ void __launch_bounds__(T_THREADS, 8) ovr_table_kernel(const OvrParams P) {
     __shared__ uint32_t tkey[T_SLOTS];      // raw float bits, 0 = empty
     __shared__ uint32_t gcount[T_SLOTS];    // multiplicity in the whole column
@@ -645,6 +650,8 @@ __global__ void __launch_bounds__(T_THREADS, 8) ovr_table_kernel(const OvrParams
             const double U = (double)u2 / 2.0;
             const double mu = (double)(n_r * n_t) / 2.0;
             const double p = compute_pval(n_r, n_t, n, P.flags.tie_correct ? tie : 0.0, U, mu, cc, P.flags.alternative);
+            if (SCORE)
+                P.flags.scores[(long long)g * P.flags.score_group_stride + jo] = compute_score(n_r, n_t, n, P.flags.tie_correct ? tie : 0.0, U, mu);
             const double mu_t = sum * (1.0 / (double)n_t);   // (the fused epilogue's form: every path gives the same bits)
             // exactly zero when the group holds every non-zero of the gene (see fused_epilogue_kernel)
             const double mu_r = (nnz_g == nnz) ? 0.0 : (total - sum) / (double)(n - n_t);
@@ -736,9 +743,11 @@ int launch_ovr_mapped(const float* ir_vals, const uint32_t* ir_cnt, int n_genes,
     P.sort_cap = sort_cap;
     const size_t need = fixed + (size_t)2 * sort_cap * 4;
 
-    ILLICO_CUDA_OK(cudaFuncSetAttribute(ovr_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
+    auto kern = flags->scores ? ovr_kernel<true> : ovr_kernel<false>;
+    auto tkern = flags->scores ? ovr_table_kernel<true> : ovr_table_kernel<false>;
+    ILLICO_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
     int occ = 0;
-    ILLICO_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, ovr_kernel, OVR_THREADS, need));
+    ILLICO_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, OVR_THREADS, need));
     if (occ < 1) { set_error("ovr_kernel does not fit: %zu bytes of shared memory", need); return 1; }
     int grid = sms * occ;
     if (grid > n_genes) grid = n_genes;
@@ -762,7 +771,7 @@ int launch_ovr_mapped(const float* ir_vals, const uint32_t* ir_cnt, int n_genes,
         P.todo = todo; P.todo_count = todo_count;
         ILLICO_CUDA_OK(cudaMemsetAsync(todo_count, 0, sizeof(int), stream));
         int tocc = 0;
-        ILLICO_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&tocc, ovr_table_kernel, T_THREADS, 0));
+        ILLICO_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&tocc, tkern, T_THREADS, 0));
         if (tocc > T_MAX_CTAS_PER_SM) tocc = T_MAX_CTAS_PER_SM;
         int tgrid = sms * (tocc > 0 ? tocc : 1);
         if (tgrid > n_genes) tgrid = n_genes;
@@ -774,12 +783,12 @@ int launch_ovr_mapped(const float* ir_vals, const uint32_t* ir_cnt, int n_genes,
             P.table_rec = reinterpret_cast<uint4*>(reinterpret_cast<char*>(workspace) + slabs);
             P.table_rec_stride = (long long)(rec_cta / 16);
         }
-        ILLICO_LAUNCH("ovr_table_kernel", stream, ovr_table_kernel<<<tgrid, T_THREADS, 0, stream>>>(P));
+        ILLICO_LAUNCH("ovr_table_kernel", stream, tkern<<<tgrid, T_THREADS, 0, stream>>>(P));
         ILLICO_CUDA_OK(cudaGetLastError());
     } else {
         P.todo = nullptr; P.todo_count = nullptr;
     }
-    ILLICO_LAUNCH("ovr_kernel", stream, ovr_kernel<<<grid, OVR_THREADS, need, stream>>>(P));
+    ILLICO_LAUNCH("ovr_kernel", stream, kern<<<grid, OVR_THREADS, need, stream>>>(P));
     ILLICO_CUDA_OK(cudaGetLastError());
     return 0;
 }

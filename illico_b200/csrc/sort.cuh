@@ -3,6 +3,8 @@
 // Ranking never moves payloads: the rank kernels sort KEYS ONLY (the order-preserving image of the
 // non-zero values) and look ranks up by binary search, so group labels stay where they were staged.
 #pragma once
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace illico {
@@ -12,12 +14,16 @@ namespace illico {
 //   aux  : [40] uint32
 constexpr int RADIX_AUX_WORDS = 40;
 
-// Stable LSD radix sort of `n` keys, 8-bit digits, ping-pong between `a` (input) and `b`.
-// Pointers may be shared or global (generic addressing).  Passes in which every key has the same
-// digit are skipped (integer-valued floats have two constant low bytes).  Returns the buffer that
-// holds the sorted keys.  Must be called by all threads of the block.
-template <typename KeyT>
-static __device__ __noinline__ KeyT* block_radix_sort_t(KeyT* a, KeyT* b, int n, uint32_t* hist, uint32_t* aux) {
+// Stable LSD radix sort of `n` keys, 8-bit digits, ping-pong between `a` (input) and `b`, optionally carrying one
+// payload per key (ValT, ping-pong between `va` and `vb`: it moves with its key).  Pointers may be shared or global
+// (generic addressing).  Passes in which every key has the same digit are skipped (integer-valued floats have two constant
+// low bytes).  Returns the buffer that holds the sorted keys; the payloads are in `va` if that is `a`, else in `vb`.
+// Must be called by all threads of the block.
+struct NoPayload {};
+template <typename KeyT, typename ValT>
+static __device__ __forceinline__ KeyT* block_radix_sort_impl(KeyT* a, KeyT* b, ValT* va, ValT* vb, int n, uint32_t* hist,
+                                                              uint32_t* aux) {
+    constexpr bool PAY = !std::is_same<ValT, NoPayload>::value;
     const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5, NW = blockDim.x >> 5;
     const unsigned lt = (1u << lane) - 1u;
     if (n <= 1) return a;
@@ -76,14 +82,29 @@ static __device__ __noinline__ KeyT* block_radix_sort_t(KeyT* a, KeyT* b, int n,
             unsigned peers = __match_any_sync(FULL, d);
             uint32_t pos = valid ? myhist[d] + __popc(peers & lt) : 0u;
             if (valid) b[pos] = key;
+            if constexpr (PAY) {
+                if (valid) vb[pos] = va[i];
+            }
             __syncwarp();
             if (valid && lane == __ffs(peers) - 1) myhist[d] += __popc(peers);
             __syncwarp();
         }
         __syncthreads();
         KeyT* t = a; a = b; b = t;
+        if constexpr (PAY) {
+            ValT* tv = va; va = vb; vb = tv;
+        }
     }
     return a;
+}
+template <typename KeyT>
+static __device__ __noinline__ KeyT* block_radix_sort_t(KeyT* a, KeyT* b, int n, uint32_t* hist, uint32_t* aux) {
+    return block_radix_sort_impl<KeyT, NoPayload>(a, b, nullptr, nullptr, n, hist, aux);
+}
+template <typename KeyT, typename ValT>
+static __device__ __noinline__ KeyT* block_radix_sort_t(KeyT* a, KeyT* b, int n, uint32_t* hist, uint32_t* aux, ValT* va,
+                                                        ValT* vb) {
+    return block_radix_sort_impl<KeyT, ValT>(a, b, va, vb, n, hist, aux);
 }
 static __device__ __forceinline__ uint32_t* block_radix_sort(uint32_t* a, uint32_t* b, int n, uint32_t* hist, uint32_t* aux) {
     return block_radix_sort_t<uint32_t>(a, b, n, hist, aux);

@@ -166,10 +166,11 @@ class Engine:
 
     # ---- one gene batch ----------------------------------------------------------------------------------
     def run_batch(self, M: DeviceMatrix, lb: int, ub: int, flags: _lib.Flags, results: torch.Tensor,
-                  result_gene0: int, debug: dict | None = None) -> None:
+                  result_gene0: int, debug: dict | None = None, scores: torch.Tensor | None = None) -> None:
         """Enqueues stage + rank for genes ``[lb, ub)`` of ``M``; writes ``results[:, result_gene0 + k, :]``.
 
-        ``results`` is a device tensor ``[G, N_total, 3]`` float64 (contiguous).
+        ``results`` is a device tensor ``[G, N_total, 3]`` float64 (contiguous).  ``scores``, a device tensor ``[G, N_total]``
+        float64 (contiguous), also receives the signed score of every test at ``scores[:, result_gene0 + k]``.
         """
         b = ub - lb
         if b <= 0:
@@ -181,10 +182,13 @@ class Engine:
         with torch.cuda.device(self.device):
             M.ready()
         if M.raw is not None:
-            return self._run_batch_wide(M, lb, ub, flags, results, result_gene0, debug)
+            return self._run_batch_wide(M, lb, ub, flags, results, result_gene0, debug, scores)
         t = self._ensure_buffers(b)
         G, Ntot = results.shape[0], results.shape[1]
         assert results.dtype == torch.float64 and results.is_contiguous() and G == self.n_groups
+        if scores is not None:
+            assert scores.dtype == torch.float64 and scores.is_contiguous() and tuple(scores.shape) == (G, Ntot)
+            flags = flags.replace(scores=scores.data_ptr() + result_gene0 * 8, score_group_stride=Ntot)
         stream = torch.cuda.current_stream(self.device)
         st = stream.cuda_stream
         for x in (t.ir_vals, t.ir_cnt, t.ws):   # a thread may enqueue on different streams over time: keep the allocator informed
@@ -208,14 +212,13 @@ class Engine:
                         gstride, dbg_ref, st)
             else:
                 if M.fmt == "csr" and flags.n_cols_hint != M.shape[1]:
-                    flags = _lib.Flags(flags.is_log1p, flags.use_continuity, flags.tie_correct, flags.alternative, flags.tie_order,
-                                       int(M.shape[1]), flags.group_sums)
+                    flags = flags.replace(n_cols_hint=int(M.shape[1]))
                 fn = getattr(self.lib, f"illico_{test}_{M.fmt}_f32")
                 rc = fn(M.data.data_ptr(), M.indices.data_ptr(), M.indptr.data_ptr(), lb, b, C.byref(self.plan),
                         C.byref(flags), C.byref(buf), out_ptr, gstride, dbg_ref, st)
         _lib.check(rc, f"illico_{test}_{M.fmt}_f32")
 
-    def _run_batch_wide(self, M: DeviceMatrix, lb: int, ub: int, flags: _lib.Flags, results, result_gene0, debug):
+    def _run_batch_wide(self, M: DeviceMatrix, lb: int, ub: int, flags: _lib.Flags, results, result_gene0, debug, scores=None):
         """float64 input (values float32 cannot hold): every sub-batch is recoded on the device to order-preserving
         float32 codes in the input's own layout (exact ranks, U, ties, p) and the fold change uses float64 group sums
         computed from the original values -- ``illico_recode_{dense,csr,csc}`` (csrc/recode.cu), then the ordinary
@@ -265,10 +268,9 @@ class Engine:
                                                     ws.data_ptr(), ws.numel(), st)
                     sub, sub_lb = DeviceMatrix(CSR, M.shape, codes, M.indices, M.indptr), a
                 _lib.check(rc, f"illico_recode_{M.fmt}")
-            f2 = _lib.Flags(flags.is_log1p, flags.use_continuity, flags.tie_correct, flags.alternative, flags.tie_order,
-                            0, sums.data_ptr())
+            f2 = flags.replace(n_cols_hint=0, group_sums=sums.data_ptr())
             dbg = {} if debug is not None else None
-            self.run_batch(sub, sub_lb, sub_lb + b, f2, results, result_gene0 + (a - lb), dbg)
+            self.run_batch(sub, sub_lb, sub_lb + b, f2, results, result_gene0 + (a - lb), dbg, scores)
             if debug is not None:
                 for k, v in dbg.items():
                     debug.setdefault("_parts", {}).setdefault(k, []).append(v)

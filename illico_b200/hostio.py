@@ -100,7 +100,7 @@ def bind_thread_to_device_node(index: int) -> None:
 # ---- strided copies through the C ABI (cudaMemcpy2DAsync) -------------------------------------------------------------
 def copy2d_async(dst_ptr: int, dpitch: int, src_ptr: int, spitch: int, width_bytes: int, height: int, kind: str, stream) -> None:
     lib = _lib.load()
-    rc = lib.illico_memcpy2d_async(dst_ptr, dpitch, src_ptr, spitch, width_bytes, height, {"h2d": 1, "d2h": 2}[kind],
+    rc = lib.illico_memcpy2d_async(dst_ptr, dpitch, src_ptr, spitch, width_bytes, height, {"h2d": 1, "d2h": 2, "d2d": 3}[kind],
                                    stream.cuda_stream)
     _lib.check(rc, "illico_memcpy2d_async")
 
@@ -417,14 +417,18 @@ def h2d_1d(dst: torch.Tensor, src: np.ndarray, n_threads: int | None = None) -> 
     return p
 
 
-def d2h_slab(host: torch.Tensor, dev_slab: torch.Tensor, gene_lb: int) -> None:
-    """Enqueues ``host[:, gene_lb:gene_lb + nb, :] = dev_slab`` (``host`` pinned ``[G, N, 3]`` float64, ``dev_slab``
-    contiguous ``[G, nb, 3]`` on a GPU) on the current stream of the slab's device: one strided device-to-host copy."""
-    G, N, three = host.shape
+def d2h_slab(host: torch.Tensor, dev_slab: torch.Tensor, gene_lb: int, kind: str = "d2h") -> None:
+    """Enqueues ``host[:, gene_lb:gene_lb + nb] = dev_slab`` (``host`` pinned ``[G, N, ...]``, ``dev_slab`` contiguous
+    ``[G, nb, ...]`` of the same dtype on a GPU; the results ``[G, N, 3]`` or the score plane ``[G, N]``) on the current
+    stream of the slab's device: one strided device-to-host copy.  ``kind="d2d"``: ``host`` is a device tensor instead
+    (possibly on another GPU)."""
+    G, N = host.shape[:2]
     nb = dev_slab.shape[1]
-    assert three == 3 and dev_slab.shape[0] == G and dev_slab.is_contiguous() and host.is_contiguous()
+    assert dev_slab.shape[0] == G and dev_slab.shape[2:] == host.shape[2:] and dev_slab.dtype == host.dtype
+    assert dev_slab.is_contiguous() and host.is_contiguous()
     if nb == 0:
         return
+    rec = host[0, 0].numel() * host.element_size()      # bytes per (group, gene)
     cur = torch.cuda.current_stream(dev_slab.device)
-    copy2d_async(host.data_ptr() + gene_lb * 24, N * 24, dev_slab.data_ptr(), nb * 24, nb * 24, G, "d2h", cur)
+    copy2d_async(host.data_ptr() + gene_lb * rec, N * rec, dev_slab.data_ptr(), nb * rec, nb * rec, G, kind, cur)
 

@@ -66,7 +66,7 @@
 extern "C" {
 #endif
 
-#define ILLICO_ABI_VERSION 2
+#define ILLICO_ABI_VERSION 3
 
 enum illico_alternative { ILLICO_TWO_SIDED = 0, ILLICO_LESS = 1, ILLICO_GREATER = 2 };
 
@@ -108,6 +108,13 @@ typedef struct illico_flags {
      * instead of sums of the staged values: the host stages ORDER-PRESERVING float32 codes of values that
      * float32 cannot hold (float64 / large integers), which keeps U, ties and p exact. */
     const double* group_sums;
+    /* Optional signed effect score of every test (device, NULL = not written): (mu - U) / sigma with mu = n_r n_t / 2 and
+     * the sigma of the p-value (tie-corrected iff tie_correct; no continuity correction, whatever the alternative) --
+     * positive when the group ranks above the reference / rest; 0 where the tie correction is <= 1e-9 (p = 1) and on the
+     * one-versus-reference control row.  Points at element [group 0, first gene of the batch], like `results`;
+     * score_group_stride = doubles between consecutive groups. */
+    double* scores;
+    int64_t score_group_stride;
 } illico_flags_t;
 
 /* Optional per-test debug outputs for bit-exact parity checks (any pointer may be NULL). */
@@ -130,7 +137,8 @@ double illico_last_fused_ms(void);
 int64_t illico_profile_report(char* out, int64_t cap);
 
 /* ---- column shards in, result slabs out -------------------------------------------------------------
- * Strided asynchronous copy (cudaMemcpy2DAsync) on `stream`: kind 1 = host to device, 2 = device to host.  The host side
+ * Strided asynchronous copy (cudaMemcpy2DAsync) on `stream`: kind 1 = host to device, 2 = device to host, 3 = device to
+ * device (the two sides may be on different GPUs: how the shards' slabs of a ranking run meet on one GPU).  The host side
  * should be page-locked for the copy to be asynchronous.  This is how a GPU receives its gene shard X[:, lb:ub] of a
  * C-order host matrix (height = n_cells rows of width_bytes = 4 (ub - lb), spitch = 4 n_genes) and how it delivers its
  * slab results[:, lb:ub, :] into the one host array of the reference's layout (illico/asymptotic_wilcoxon.py:210,
@@ -288,6 +296,17 @@ int illico_unpack_rows_f32(const uint32_t* mask, const uint32_t* row_off, const 
 size_t illico_bh_workspace_bytes(int32_t n_groups, int32_t n_genes);
 int illico_bh_adjust(const double* p_values, int64_t group_stride, int64_t gene_stride, int32_t n_groups, int32_t n_genes,
                      double* p_adj, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Per-group ranking of the genes (scanpy rank_genes_groups' order): group g's n_genes scores
+ * scores[g * score_group_stride + j] sorted descending (by_abs != 0: by |score|), ties by gene index ascending, NaN after
+ * every number, -0.0 equal to +0.0.  The first k (1 <= k <= n_genes) gene indices go to out_gene [n_groups, k] (int32) and
+ * their records (score, p_value, statistic, fold_change, p_adj) to out_rec [n_groups, k, 5] (float64), gathered from the
+ * score plane, results[g * result_group_stride + 3 j ..] and p_adj[g * n_genes + j] (NULL: NaN).  Stable LSD radix sort,
+ * one CTA per group; workspace from illico_top_genes_workspace_bytes. */
+size_t illico_top_genes_workspace_bytes(int32_t n_groups, int32_t n_genes);
+int illico_top_genes(const double* scores, int64_t score_group_stride, const double* results, int64_t result_group_stride,
+                     const double* p_adj, int32_t n_groups, int32_t n_genes, int32_t k, int32_t by_abs, int32_t* out_gene,
+                     double* out_rec, void* workspace, size_t workspace_bytes, void* stream);
 
 /* The device epilogue's compute_pval (illico/utils/math.py:64-118) on arrays of arguments (device pointers): lets the
  * known-answer vectors of the reference's primitive be checked against the GPU code itself. */
