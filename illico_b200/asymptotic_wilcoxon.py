@@ -194,7 +194,7 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
     # NVLink (repartition.py), instead of every GPU receiving the whole matrix
     prep = None
     if fmt == CSR and len(shards) > 1 and data_handler.in_ram and isinstance(X, sparse.csr_matrix) \
-            and X.data.dtype == np.float32 and os.environ.get("ILLICO_CSR_REPARTITION", "1") != "0":
+            and X.data.dtype == np.float32:
         from . import repartition
 
         if repartition.peer_access_ok([sh.device for sh in shards]):

@@ -270,7 +270,7 @@ template <int ROWS, int STAGES, int BUF, int MINB, bool OVO>
 __global__ void __launch_bounds__(FUSED_THREADS, MINB) fused_pass_kernel(const float* __restrict__ X, long long ld, int gene_lb,
                                                                          int b, const illico_plan_t pl, int groups_per_cta,
                                                                          Gtab gt, int bs, unsigned long long* __restrict__ rec,
-                                                                         long long gstride, int share_1024, int backoff) {
+                                                                         long long gstride, int share_1024) {
     using L = FusedLayout<ROWS, STAGES, BUF>;
     static_assert(32 % ROWS == 0 && BUF > ROWS, "layout");
     extern __shared__ __align__(128) unsigned char smem[];
@@ -325,7 +325,7 @@ __global__ void __launch_bounds__(FUSED_THREADS, MINB) fused_pass_kernel(const f
                 if (q * ROWS >= nrows) break;
                 const int slot = k % STAGES;
                 const uint32_t full = bars + 8 * slot, empty = bars + 8 * (STAGES + slot);
-                if (backoff) mbar_wait_backoff(empty, ((k / STAGES) & 1) ^ 1); else mbar_wait(empty, ((k / STAGES) & 1) ^ 1);
+                mbar_wait(empty, ((k / STAGES) & 1) ^ 1);
                 const int rows_here = min(ROWS, nrows - q * ROWS);
                 if (lane == 0) mbar_expect_tx(full, (uint32_t)rows_here * row_bytes);
                 __syncwarp();
@@ -1088,162 +1088,6 @@ __global__ void __launch_bounds__(CSRF_THREADS, 1) fused_csr_pass_kernel(const f
     }
 }
 
-// ---- the same pass with the shared-memory atomics taken out ------------------------------------------------------------
-// fused_csr_pass_kernel gives every warp whole rows, so two warps may count in the same gene's histogram at once and every
-// update is a shared-memory atomic -- the unit that bounds the kernel (2 cycles per lane, profiles/README.md).  Here a warp
-// owns a RANGE OF GENES of the tile (CSR2_RANGE columns) for all the rows of the segment: the histogram words it touches
-// are its own, updates are plain LDS / STS, and the warps never synchronise until the records are written.  The price is
-// finding where the warp's columns begin in every row.  Column indices ascend inside a row and are spread about evenly, so
-// the position is guessed by interpolation (row extent x column / matrix width) and a 64-entry window around the guess is
-// loaded (two coalesced loads, neighbouring warps share the lines); the window holds the boundary in all but a few per
-// cent of the cases, otherwise it is moved, and a row far off the guess falls back to a binary search.  Four rows are in
-// flight per warp (window loads, then entry loads, issued together).
-constexpr int CSR2_WARPS = 16;
-constexpr int CSR2_THREADS = CSR2_WARPS * 32;
-// (genes per warp: template parameter RANGE; 256 -> tiles of 4096 genes, 96 KB of shared memory, two CTAs per SM)
-
-// first entry of a row (n entries at `idx`) whose column is >= c_lo, given the 64-entry window at ws (w0 / w1 = the lane's
-// two entries, INT_MAX past the row's end).  Positions are relative to the row's start.  Warp-uniform.
-__device__ __forceinline__ int csr2_find_start(const int32_t* __restrict__ idx, int n, int ws, int w0, int w1, int c_lo, int lane) {
-    int lo_known = 0, hi_known = n;                    // entries before lo_known are < c_lo; the one at hi_known is >= c_lo
-    for (int it = 0; it < 3; ++it) {
-        const unsigned g0 = __ballot_sync(FULL, w0 >= c_lo), g1 = __ballot_sync(FULL, w1 >= c_lo);
-        if (!(g0 & 1u)) {                              // the window starts below the boundary
-            if (g0) return ws + __ffs(g0) - 1;
-            if (g1) return ws + 32 + __ffs(g1) - 1;
-            lo_known = ws + 64;                        // ... and ends below it
-            if (lo_known >= hi_known) return hi_known;
-            ws = lo_known;
-        } else {
-            if (ws <= lo_known) return ws;             // nothing below the window is left to look at
-            hi_known = ws;
-            ws = max(ws - 64, lo_known);
-        }
-        w0 = (ws + lane < n) ? __ldg(idx + ws + lane) : 0x7fffffff;
-        w1 = (ws + 32 + lane < n) ? __ldg(idx + ws + 32 + lane) : 0x7fffffff;
-    }
-    while (lo_known < hi_known) {                      // a row far off the guess
-        const int mid = (lo_known + hi_known) >> 1;
-        if (__ldg(idx + mid) < c_lo) lo_known = mid + 1; else hi_known = mid;
-    }
-    return lo_known;
-}
-
-template <bool OVO, bool IDENT, int RANGE, int CSR2_ROWS>
-__global__ void __launch_bounds__(CSR2_THREADS, (RANGE > 256 ? 1 : 2)) fused_csr_pass2_kernel(
-        const float* __restrict__ data, const int32_t* __restrict__ indices, const long long* __restrict__ indptr, int gene_lb, int b,
-        int n_cols, const illico_plan_t pl, Gtab gt, int bs, unsigned long long* __restrict__ rec, long long gstride) {
-    constexpr int TILE = CSR2_WARPS * RANGE;
-    extern __shared__ __align__(16) uint32_t hist[];             // u16 [genes of the tile][12]
-    const int t = threadIdx.x, lane = t & 31, w = t >> 5;
-    const int s = blockIdx.y, g = pl.seg_group[s];
-    const int j_lo = blockIdx.x * TILE, ng = min(TILE, b - j_lo);
-    __shared__ int stop;
-    if (t == 0) stop = 8 * *reinterpret_cast<volatile int*>(gt.n_bad) > b;   // many genes handed back: the general path redoes the batch
-    for (int i = t; i < ng * 6; i += CSR2_THREADS) hist[i] = 0u;
-    __syncthreads();
-    if (stop) return;
-    const int r_lo = w * RANGE, r_n = min(RANGE, ng - r_lo);
-    if (r_n > 0) {
-        const int c_lo = gene_lb + j_lo + r_lo, c_hi = c_lo + r_n;
-        const float frac = (float)c_lo / (float)max(n_cols, 1);
-        const uint32_t hist_w = (uint32_t)__cvta_generic_to_shared(hist) + (uint32_t)r_lo * 24u;
-        float* gkey_w = gt.key + j_lo + r_lo;
-        unsigned char* gbad_w = gt.bad + j_lo + r_lo;
-        const int p0 = pl.seg_pos[s], p1 = pl.seg_pos[s + 1];
-        // one stored value of gene jj (inside the warp's range): its slot's counter, or the gene is handed back
-        auto count = [&](int jj, float v) {
-            int q;
-            if (IDENT) {                                          // raw counts: the table is 1 .. 12, never changed
-                const float tt = __fadd_rn(v, ROUND_MAGIC);
-                q = (int)(__float_as_uint(tt) - (ROUND_MAGIC_BITS + 1u));
-                if (!((__fsub_rn(tt, ROUND_MAGIC) == v) && ((unsigned)q < (unsigned)DCAP))) q = -1;
-            } else {
-                q = min(max((int)v - 1, 0), DCAP - 1);
-                if (__ldcg(gkey_w + (long long)q * bs + jj) != v) q = gbad_w[jj] ? -1 : gtab_slot(gkey_w + jj, bs, v);
-            }
-            if (q >= 0) {
-                const uint32_t a = hist_w + (uint32_t)jj * 24u + (uint32_t)q * 2u;
-                asm volatile("{ .reg .u32 h; ld.shared.u16 h, [%0]; add.u32 h, h, 1; st.shared.u16 [%0], h; }" ::"r"(a) : "memory");
-            } else {                                              // hand the gene back, counted once
-                const int j = j_lo + r_lo + jj;
-                const unsigned bit = 1u << (8 * (j & 3));
-                const unsigned old = atomicOr(reinterpret_cast<unsigned*>(gt.bad + (j & ~3)), bit);
-                if (!(old & bit)) atomicAdd(gt.n_bad, 1);
-            }
-        };
-        for (int pb = p0; pb < p1; pb += 32) {
-            if (8 * *reinterpret_cast<volatile int*>(gt.n_bad) > b) break;   // continuous data: stop before the miss path is walked
-            long long my_e0 = 0;                                  // lane k: start and length of row pb + k
-            int my_n = 0;
-            if (pb + lane < p1) { const long long r = pl.perm[pb + lane]; my_e0 = indptr[r]; my_n = (int)(indptr[r + 1] - my_e0); }
-            const int nr = min(32, p1 - pb);
-            for (int k0 = 0; k0 < nr; k0 += CSR2_ROWS) {
-                const int32_t* idx[CSR2_ROWS];
-                const float* val[CSR2_ROWS];
-                int n[CSR2_ROWS], ws[CSR2_ROWS], w0[CSR2_ROWS], w1[CSR2_ROWS];
-#pragma unroll
-                for (int u = 0; u < CSR2_ROWS; ++u) {
-                    const int k = min(k0 + u, 31);
-                    const long long e0 = __shfl_sync(FULL, my_e0, k);
-                    n[u] = (k0 + u < nr) ? __shfl_sync(FULL, my_n, k) : 0;
-                    idx[u] = indices + e0;
-                    val[u] = data + e0;
-                    ws[u] = max(min((int)((float)n[u] * frac) - 32, n[u] - 64), 0);
-                    w0[u] = (ws[u] + lane < n[u]) ? __ldg(idx[u] + ws[u] + lane) : 0x7fffffff;
-                    w1[u] = (ws[u] + 32 + lane < n[u]) ? __ldg(idx[u] + ws[u] + 32 + lane) : 0x7fffffff;
-                }
-                int st[CSR2_ROWS];
-#pragma unroll
-                for (int u = 0; u < CSR2_ROWS; ++u) st[u] = csr2_find_start(idx[u], n[u], ws[u], w0[u], w1[u], c_lo, lane);
-                int ci[CSR2_ROWS];
-                float cv[CSR2_ROWS];
-#pragma unroll
-                for (int u = 0; u < CSR2_ROWS; ++u) {
-                    const int e = st[u] + lane;
-                    ci[u] = (e < n[u]) ? __ldcs(idx[u] + e) : 0x7fffffff;
-                    cv[u] = (e < n[u]) ? __ldcs(val[u] + e) : 0.0f;
-                }
-#pragma unroll
-                for (int u = 0; u < CSR2_ROWS; ++u) {
-                    for (;;) {
-                        if (ci[u] < c_hi && cv[u] != 0.0f) count(ci[u] - c_lo, cv[u]);       // explicitly stored zeros are zeros
-                        if (__shfl_sync(FULL, ci[u], 31) >= c_hi) break;                   // (ascending: the range ends in this chunk)
-                        st[u] += 32;
-                        const int e = st[u] + lane;
-                        ci[u] = (e < n[u]) ? __ldcs(idx[u] + e) : 0x7fffffff;
-                        cv[u] = (e < n[u]) ? __ldcs(val[u] + e) : 0.0f;
-                    }
-                }
-            }
-        }
-    }
-    __syncthreads();
-    const bool multi = pl.group_seg[g + 1] - pl.group_seg[g] > 1;
-    for (int jj = t; jj < ng; jj += CSR2_THREADS) {
-        const int j = j_lo + jj;
-        uint32_t wd[6];
-#pragma unroll
-        for (int k = 0; k < 6; ++k) wd[k] = hist[jj * 6 + k];
-        if (OVO && g == pl.ref_group) {
-            // the control's histogram is the table's multiplicity column
-#pragma unroll
-            for (int q = 0; q < DCAP; ++q) {
-                const uint32_t cq = (wd[q >> 1] >> (16 * (q & 1))) & 0xffffu;
-                if (cq) atomicAdd(gt.mult + (long long)q * bs + j, cq);
-            }
-        } else if (!multi) {
-            unsigned long long* o = rec + (long long)g * gstride + (long long)j * 3;
-#pragma unroll
-            for (int k = 0; k < 3; ++k) o[k] = (unsigned long long)wd[2 * k] | ((unsigned long long)wd[2 * k + 1] << 32);
-        } else {
-            uint32_t* o = reinterpret_cast<uint32_t*>(rec + (long long)g * gstride + (long long)j * 3);
-#pragma unroll
-            for (int k = 0; k < 6; ++k) if (wd[k]) atomicAdd(o + k, wd[k]);   // u16 pairs: no carry, a group has < 65536 cells
-        }
-    }
-}
-
 // one-versus-rest: the whole gene's histogram = the sum of its groups' records
 __global__ void __launch_bounds__(256) fused_hist_sum_kernel(int b, int G, int groups_per_block, Gtab gt, int bs,
                                                              const unsigned long long* __restrict__ rec, long long gstride) {
@@ -1317,19 +1161,8 @@ int list_share_1024() {
 
 thread_local float g_last_fused_ms = -1.0f;   // >= 0: the last dispatcher call of this thread enqueued a fused pass
 
-template <int ROWS, int STAGES, int BUF, int MINB, bool OVO>
-int launch_pass_t(const float* X, long long ld, int gene_lb, int b, const illico_plan_t* plan, int gpc, Gtab gt, int bs,
-                  double* results, long long gstride, cudaStream_t stream) {
-    using L = FusedLayout<ROWS, STAGES, BUF>;
-    auto kern = fused_pass_kernel<ROWS, STAGES, BUF, MINB, OVO>;
-    ILLICO_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::BYTES));
-    const dim3 grid((unsigned)((b + FUSED_LANES - 1) / FUSED_LANES), (unsigned)((plan->n_groups + gpc - 1) / gpc));
-    ILLICO_LAUNCH("fused_pass_kernel", stream, kern<<<grid, FUSED_THREADS, L::BYTES, stream>>>(X, ld, gene_lb, b, *plan, gpc, gt, bs,
-                                                    reinterpret_cast<unsigned long long*>(results), gstride, list_share_1024(),
-                                                    env_int("ILLICO_FUSED_BACKOFF", 0)));
-    ILLICO_CUDA_OK(cudaGetLastError());
-    return 0;
-}
+constexpr int PASS_ROWS = 1536;          // rows a CTA of the passes streams: groups per CTA = PASS_ROWS / average group size
+constexpr int OVR_SAMPLE_CELLS = 16384;  // one-versus-rest: cells staged to seed the tables
 
 // The whole fused path for one gene batch, enqueued without a single host read-back.
 // 0 = enqueued, 1 = error, -1 = not applicable (the caller runs the general path).
@@ -1358,7 +1191,7 @@ int run_fused(const float* X, long long ld, int gene_lb, int b, const illico_pla
         long long avg = plan->n_cells / plan->n_segments;
         if (avg < 1) avg = 1;
         seg_lo = 0;
-        seg_hi = (int)((env_int("ILLICO_OVR_FUSED_SAMPLE", 16384) + avg - 1) / avg);
+        seg_hi = (int)((OVR_SAMPLE_CELLS + avg - 1) / avg);
         if (seg_hi < 1) seg_hi = 1;
         if (seg_hi > plan->n_segments) seg_hi = plan->n_segments;
     }
@@ -1378,22 +1211,24 @@ int run_fused(const float* X, long long ld, int gene_lb, int b, const illico_pla
     // 2. the pass over the matrix (CTAs whose genes were all handed back by the table step leave at once)
     long long avg_g = plan->n_cells / plan->n_groups;
     if (avg_g < 1) avg_g = 1;
-    int gpc = (int)(env_int("ILLICO_FUSED_ROWS", 1536) / avg_g);
+    int gpc = (int)(PASS_ROWS / avg_g);
     if (gpc < 1) gpc = 1;
-    // ring / buffer shapes measured at the K562 shape (profiles/README.md): stages of 8 rows, a 16-entry group buffer,
-    // 3 CTAs per SM; the 5-stage ring (74 KB of shared memory per CTA) is 6-7 % faster than the 4-stage one
-    int rc;
-    if (env_int("ILLICO_FUSED_STAGES", 5) != 4)
-        rc = launch_pass_t<8, 5, 16, 3, OVO>(X, ld, gene_lb, b, plan, gpc, gt, bs, results, gstride, stream);
-    else
-        rc = launch_pass_t<8, 4, 16, 3, OVO>(X, ld, gene_lb, b, plan, gpc, gt, bs, results, gstride, stream);
-    if (rc) return rc;
+    {
+        // ring / buffer shapes measured at the K562 shape (profiles/README.md): stages of 8 rows, a 16-entry group buffer,
+        // 3 CTAs per SM; the 5-stage ring (74 KB of shared memory per CTA) is 6-7 % faster than the 4-stage one
+        using L = FusedLayout<8, 5, 16>;
+        auto kern = fused_pass_kernel<8, 5, 16, 3, OVO>;
+        ILLICO_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::BYTES));
+        const dim3 grid((unsigned)((b + FUSED_LANES - 1) / FUSED_LANES), (unsigned)((plan->n_groups + gpc - 1) / gpc));
+        ILLICO_LAUNCH("fused_pass_kernel", stream, kern<<<grid, FUSED_THREADS, L::BYTES, stream>>>(X, ld, gene_lb, b, *plan, gpc, gt, bs,
+                                                        reinterpret_cast<unsigned long long*>(results), gstride, list_share_1024()));
+        ILLICO_CUDA_OK(cudaGetLastError());
+    }
     if (wide_on) {
         // (a 6-stage ring -- 112 KB per CTA, the most two CTAs per SM leave room for -- makes the pass 3 % faster and the
-        // whole step 9 % slower: measured, scripts/exp/wide3.sh)
-        const bool six = env_int("ILLICO_WIDE_STAGES", 5) == 6;
-        auto kern = six ? fused_wide_pass_kernel<8, 6, 2> : fused_wide_pass_kernel<8, 5, 2>;
-        const int wide_smem = six ? WideLayout<8, 6>::BYTES : WideLayout<8, 5>::BYTES;
+        // whole step 9 % slower: measured, and removed after commit 216d8fd)
+        auto kern = fused_wide_pass_kernel<8, 5, 2>;
+        const int wide_smem = WideLayout<8, 5>::BYTES;
         ILLICO_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, wide_smem));
         // persistent: two CTAs per SM, each a tile of 256 genes walking every gy-th chunk of groups
         const int tiles = (b + FUSED_LANES - 1) / FUSED_LANES, chunks = (plan->n_groups + gpc - 1) / gpc;
@@ -1489,24 +1324,9 @@ int run_fused_csr(const float* data, const int32_t* indices, const long long* in
     {
         // (An atomics-free variant -- the whole CTA applies one row at a time, plain LDS/STS -- measured 1.5-2.7 x
         // slower: 150 CTA-wide barriers per segment cost more than the shared atomics they avoid.  Counting part of the
-        // updates in a per-SM global histogram with L2 reductions instead of shared atomics measured 1.4-1.9 x slower.)
-        // 1 = warp per row, shared-memory atomics (default); 2 = warp per gene range without atomics.  Measured at the K562
-        // shape (scripts/exp/csr2.sh): 1.15 ms against 1.57 ms (8 rows in flight: 1.62 ms; 512-gene ranges, one CTA per SM:
-        // 2.54 ms) -- finding the range's start in every row costs about 105 instructions per 24-entry row piece, more than
-        // the atomics it saves.
-        const int pass_kind = env_int("ILLICO_CSR_PASS", 1);
-        if (pass_kind >= 2) {
-            const bool ident = !flags->is_log1p;                 // fused_seed_kernel seeded the slots with 1 .. 12
-            const int range = 256;
-            auto kern2 = ident ? fused_csr_pass2_kernel<OVO, true, 256, 4> : fused_csr_pass2_kernel<OVO, false, 256, 4>;
-            const int tile = CSR2_WARPS * range;
-            const size_t smem2 = (size_t)(b < tile ? b : tile) * 24;
-            ILLICO_CUDA_OK(cudaFuncSetAttribute(kern2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-            const dim3 grid2((unsigned)((b + tile - 1) / tile), (unsigned)plan->n_segments);
-            const int n_cols = flags->n_cols_hint > gene_lb + b ? flags->n_cols_hint : gene_lb + b;
-            ILLICO_LAUNCH("fused_csr_pass_kernel", stream, kern2<<<grid2, CSR2_THREADS, smem2, stream>>>(data, indices, indptr, gene_lb, b, n_cols, *plan, gt, bs, rec, gstride));
-            ILLICO_CUDA_OK(cudaGetLastError());
-        } else {
+        // updates in a per-SM global histogram with L2 reductions instead of shared atomics measured 1.4-1.9 x slower.
+        // A warp per gene range without atomics measured 1.57 ms against 1.15 ms at the K562 shape: finding the range's
+        // start in every row costs more than the atomics it saves; it was removed after commit 216d8fd.)
         auto kern = fused_csr_pass_kernel<OVO>;
         const int tile = b < CSRF_TILE ? b : CSRF_TILE;
         const size_t smem = (size_t)tile * 24;
@@ -1514,7 +1334,6 @@ int run_fused_csr(const float* data, const int32_t* indices, const long long* in
         const dim3 grid((unsigned)((b + CSRF_TILE - 1) / CSRF_TILE), (unsigned)plan->n_segments);
         ILLICO_LAUNCH("fused_csr_pass_kernel", stream, kern<<<grid, CSRF_THREADS, smem, stream>>>(data, indices, indptr, gene_lb, b, *plan, gt, bs, rec, gstride));
         ILLICO_CUDA_OK(cudaGetLastError());
-        }
     }
     g_last_fused_ms = 0.0f;
     // (when the pass stopped early -- an eighth of the genes flagged: continuous data -- the kernels below work on

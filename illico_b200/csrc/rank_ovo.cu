@@ -27,8 +27,6 @@
 #include "epilogue.cuh"
 #include "sort.cuh"
 
-#include <stdlib.h>
-
 namespace illico {
 
 constexpr int WARP_CAP = 1024;     // keys per warp buffer in the warp tier
@@ -43,6 +41,8 @@ constexpr int MBINS = 64;          // groups of a chunk are handed to the thread
 constexpr int HCAP = 4096;         // slots of the hash that finds the distinct values of a large control
 constexpr int REF_CAP = 1536;      // control keys sorted in shared memory (larger controls: the CTA's global slab)
 constexpr int GCN = 5;             // per-group constants of the p-value (see ovo_group_consts_kernel)
+constexpr int OVO_THREADS = 256;   // threads per CTA of ovo_kernel
+constexpr int OVO_MIN_CTAS = 3;    // CTAs per SM it is compiled for
 
 struct OvoParams {
     const float* ir_vals;
@@ -59,7 +59,6 @@ struct OvoParams {
     const int* n_genes_dev;  // optional: number of genes decided on the device (a hand-back list), else n_genes
     const int* gene_map;     // optional: staged gene j is column gene_map[j] of the results / debug / group-sum arrays
     int n_cols;              // width of the debug / group-sum arrays (= n_genes unless gene_map is set)
-    int bucket_index;        // 1 = searches go through the bucket index of the search table
     const double* gc;        // [GCN][Gs] per-group constants (ovo_group_consts_kernel)
     int Gs;
     long long* dbg_u2;
@@ -314,8 +313,8 @@ __global__ void __launch_bounds__(256) ovo_group_consts_kernel(const illico_plan
 }
 
 // SCORE: also writes the score plane (illico_flags_t::scores), in an instantiation of its own
-template <int OVO_THREADS, int MIN_CTAS, bool LOG1P, bool SCORE>
-__global__ void __launch_bounds__(OVO_THREADS, MIN_CTAS) ovo_kernel(const OvoParams P) {
+template <bool LOG1P, bool SCORE>
+__global__ void __launch_bounds__(OVO_THREADS, OVO_MIN_CTAS) ovo_kernel(const OvoParams P) {
     constexpr int NT = OVO_THREADS;
     constexpr int OVO_NW = OVO_THREADS / 32;
     extern __shared__ __align__(16) uint32_t smem[];
@@ -520,7 +519,7 @@ __global__ void __launch_bounds__(OVO_THREADS, MIN_CTAS) ovo_kernel(const OvoPar
         // ---- bucket index of the search table
         R.bk_s = (uint32_t)__cvta_generic_to_shared(bkidx);
         R.bk_T = -1; R.kmin = 0u; R.bk_shift = 0; R.bk_last = 0;
-        if (R.st_n > 1 && P.bucket_index) {
+        if (R.st_n > 1) {
             const uint32_t kmin = st_key[0], span = st_key[D - 1] - kmin;
             int shift = max(0, 22 - __clz(span));                         // span >> shift < 1024
             if ((span >> shift) > (uint32_t)(GROUP_CHUNK - 2)) ++shift;   // ... and at most GROUP_CHUNK - 1 buckets
@@ -885,11 +884,6 @@ __global__ void __launch_bounds__(OVO_THREADS, MIN_CTAS) ovo_kernel(const OvoPar
     }
 }
 
-static int env_int(const char* name, int dflt) {
-    const char* v = getenv(name);
-    return v ? atoi(v) : dflt;
-}
-
 // ------------------------------------------------------------------------------------------------------
 // workspace: [gene counter | per-group constants | per-CTA slabs]
 static size_t ovo_head_bytes(const illico_plan_t* plan) {
@@ -900,10 +894,10 @@ size_t ovo_workspace_bytes(const illico_plan_t* plan, int n_ctas) {
     return ovo_head_bytes(plan) + (size_t)n_ctas * 4 * (size_t)plan->max_group_size * sizeof(uint32_t);
 }
 
-template <int NT, int MIN_CTAS, bool LOG1P, bool SCORE>
+template <bool LOG1P, bool SCORE>
 static int launch_ovo_t(OvoParams& P, const illico_plan_t* plan, void* workspace, size_t workspace_bytes, int sms,
                         int max_smem, cudaStream_t stream) {
-    constexpr int NW = NT / 32;
+    constexpr int NT = OVO_THREADS, NW = NT / 32;
     // shared memory: control buffer + scratch + fixed part.  Genes whose control has more non-zeros than REF_CAP
     // keep the control in the CTA's global slab.
     const size_t fixed = (size_t)(NW * 256 + RADIX_AUX_WORDS + 2 * GROUP_CHUNK + 8 + MBINS) * 4 + 32 * 8 * 2 + DT_CAP * 16 + DT_HASH * 8 +
@@ -915,7 +909,7 @@ static int launch_ovo_t(OvoParams& P, const illico_plan_t* plan, void* workspace
     const size_t need = fixed + (size_t)(REF_CAP + scratch_words) * 4;
     if (need > (size_t)max_smem) { set_error("ovo_kernel needs %zu bytes of shared memory", need); return 1; }
     P.scratch_words = scratch_words;
-    auto kern = ovo_kernel<NT, MIN_CTAS, LOG1P, SCORE>;
+    auto kern = ovo_kernel<LOG1P, SCORE>;
     ILLICO_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
     int occ = 0;
     ILLICO_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, need));
@@ -965,19 +959,11 @@ int launch_ovo_mapped(const float* ir_vals, const uint32_t* ir_cnt, int n_genes,
     P.n_genes_dev = n_genes_dev; P.gene_map = gene_map; P.n_cols = n_cols;
     P.dbg_u2 = dbg ? (long long*)dbg->u2 : nullptr; P.dbg_tie = dbg ? dbg->tie_sum : nullptr;
     P.dbg_tie_exact = dbg ? (long long*)dbg->tie_exact : nullptr;
-    P.bucket_index = env_int("ILLICO_OVO_BUCKETS", 1);
-    static const int nt = env_int("ILLICO_OVO_THREADS", 256);
     const int v = (flags->is_log1p ? 1 : 0) | (flags->scores ? 2 : 0);
-    if (nt == 512) {
-        if (v == 0) return launch_ovo_t<512, 2, false, false>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
-        if (v == 1) return launch_ovo_t<512, 2, true, false>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
-        if (v == 2) return launch_ovo_t<512, 2, false, true>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
-        return launch_ovo_t<512, 2, true, true>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
-    }
-    if (v == 0) return launch_ovo_t<256, 3, false, false>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
-    if (v == 1) return launch_ovo_t<256, 3, true, false>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
-    if (v == 2) return launch_ovo_t<256, 3, false, true>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
-    return launch_ovo_t<256, 3, true, true>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
+    if (v == 0) return launch_ovo_t<false, false>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
+    if (v == 1) return launch_ovo_t<true, false>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
+    if (v == 2) return launch_ovo_t<false, true>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
+    return launch_ovo_t<true, true>(P, plan, workspace, workspace_bytes, sms, max_smem, stream);
 }
 
 int launch_ovo(const float* ir_vals, const uint32_t* ir_cnt, int n_genes, const illico_plan_t* plan,

@@ -19,8 +19,6 @@
 #include "epilogue.cuh"
 #include "sort.cuh"
 
-#include <stdlib.h>
-
 namespace illico {
 
 constexpr int OVR_THREADS = 512;
@@ -45,7 +43,7 @@ struct OvrParams {
     long long gstride;
     unsigned long long* slab;  // global scratch, slab_qwords (8-byte words) per CTA
     long long slab_qwords;
-    int sort_cap;              // keys per shared-memory sort buffer (path S)
+    int sort_cap;              // keys per shared-memory sort buffer (path S): HASH_CAP
     long long* dbg_u2;
     double* dbg_tie;
     long long* dbg_tie_exact;
@@ -56,8 +54,6 @@ struct OvrParams {
     int* todo_count;
     uint4* table_rec;          // table kernel: per-CTA [n_segments][2] segment records (NULL: second pass re-reads the values)
     long long table_rec_stride;  // uint4 per CTA
-    int bucket_index;          // 1 = ranks of path S go through a bucket index of the sorted keys
-    int hash_max;              // most distinct values path H takes (<= MAX_DISTINCT); more: path S
 };
 
 __device__ __forceinline__ uint32_t hash_slot(uint32_t key) { return (key * 2654435761u) >> 20; }  // 12 bits
@@ -161,13 +157,13 @@ __global__ void __launch_bounds__(OVR_THREADS, 2) ovr_kernel(const OvrParams P) 
                     if (act && key == HASH_EMPTY) key = 1u;  // only a NaN payload maps here
                     const unsigned peers = __match_any_sync(FULL, key);
                     if (act && lane == __ffs(peers) - 1 && !*(volatile int*)&sc[1])
-                        hash_insert(hkeys, hvals, &sc[0], &sc[1], key, __popc(peers), P.hash_max);
+                        hash_insert(hkeys, hvals, &sc[0], &sc[1], key, __popc(peers), MAX_DISTINCT);
                 }
             }
         }
         nnz = (long long)block_sum<unsigned long long>(my_nnz, redu);  // syncs
         n0 = n - nnz;
-        path_s = sc[1] != 0 || sc[0] > P.hash_max;
+        path_s = sc[1] != 0 || sc[0] > MAX_DISTINCT;
         __syncthreads();
 
         if (!path_s) {
@@ -255,7 +251,7 @@ __global__ void __launch_bounds__(OVR_THREADS, 2) ovr_kernel(const OvrParams P) 
             // ---- bucket index of the sorted keys (they sit in the global slab: region0 is free): the key range is cut
             // into equal buckets, bk[b] = first position of bucket b or later, so a rank reads its bucket's bounds from
             // shared memory and halves a few times in L2 instead of 15 times
-            bk_on = !in_smem && nnz > 1 && nnz < 65536 && P.bucket_index;
+            bk_on = !in_smem && nnz > 1 && nnz < 65536;
             if (bk_on) {
                 uint16_t* bk = reinterpret_cast<uint16_t*>(smem);
                 const int cap = 4 * HASH_CAP - 2;                                   // u16 entries in region0, one spare
@@ -714,10 +710,9 @@ int launch_ovr_mapped(const float* ir_vals, const uint32_t* ir_cnt, int n_genes,
                       const illico_plan_t* plan, const illico_flags_t* flags, double* results, long long gstride, void* workspace,
                       size_t workspace_bytes, const illico_debug_t* dbg, cudaStream_t stream) {
     if (n_genes <= 0) return 0;
-    int dev = 0, sms = 0, max_smem = 0;
+    int dev = 0, sms = 0;
     ILLICO_CUDA_OK(cudaGetDevice(&dev));
     ILLICO_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    ILLICO_CUDA_OK(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
 
     OvrParams P;
     P.ir_vals = ir_vals; P.ir_cnt = ir_cnt; P.n_genes = n_genes; P.plan = *plan; P.flags = *flags;
@@ -725,23 +720,12 @@ int launch_ovr_mapped(const float* ir_vals, const uint32_t* ir_cnt, int n_genes,
     P.n_genes_dev = n_genes_dev; P.gene_map = gene_map; P.n_cols = n_cols;
     P.dbg_u2 = dbg ? (long long*)dbg->u2 : nullptr; P.dbg_tie = dbg ? dbg->tie_sum : nullptr;
     P.dbg_tie_exact = dbg ? (long long*)dbg->tie_exact : nullptr;
-    { const char* benv = getenv("ILLICO_OVR_BUCKETS"); P.bucket_index = benv ? atoi(benv) : 1; }
-    { const char* henv = getenv("ILLICO_OVR_HASH_MAX"); P.hash_max = henv ? atoi(henv) : MAX_DISTINCT; }
-    if (P.hash_max > MAX_DISTINCT) P.hash_max = MAX_DISTINCT;
-    if (P.hash_max < 1) P.hash_max = 1;
 
-    // two CTAs per SM: ~113 KB each.  Fixed part: histogram / distinct table 16 KB + scalars.
+    // Fixed part: histogram / distinct table 16 KB + scalars.  Path S sorts in shared memory only up to HASH_CAP keys
+    // (the hash table's footprint); what is not carved out stays L1 cache for the scattered reads of the group slots.
     const size_t fixed = (size_t)(OVR_NW * 256 + RADIX_AUX_WORDS + 8) * 4 + 32 * 8 * 2 + 8 + 64;
-    const size_t per_cta = (size_t)(max_smem + 1024) / 2 - 1024;
-    // Path S sorts in shared memory only up to sort_cap keys (default: the hash table's footprint); what is not
-    // carved out stays L1 cache for the scattered reads of the group slots.
-    int sort_cap = (int)((per_cta - fixed) / 8) & ~3;
-    const char* sc_env = getenv("ILLICO_OVR_SORT_CAP");
-    const int want = sc_env ? atoi(sc_env) : HASH_CAP;
-    if (sort_cap > want) sort_cap = want;
-    if (sort_cap < HASH_CAP) sort_cap = HASH_CAP;
-    P.sort_cap = sort_cap;
-    const size_t need = fixed + (size_t)2 * sort_cap * 4;
+    P.sort_cap = HASH_CAP;
+    const size_t need = fixed + (size_t)2 * HASH_CAP * 4;
 
     auto kern = flags->scores ? ovr_kernel<true> : ovr_kernel<false>;
     auto tkern = flags->scores ? ovr_table_kernel<true> : ovr_table_kernel<false>;
@@ -764,10 +748,8 @@ int launch_ovr_mapped(const float* ir_vals, const uint32_t* ir_cnt, int n_genes,
         if (grid < 1) { set_error("rank workspace too small: %zu bytes", workspace_bytes); return 1; }
     }
     P.slab = (unsigned long long*)workspace; P.slab_qwords = (long long)slab_q;
-    const char* tenv = getenv("ILLICO_OVR_TABLE");
-    const bool use_table = flags->group_sums == nullptr && !(tenv && atoi(tenv) == 0);
     P.table_rec = nullptr; P.table_rec_stride = 0;
-    if (use_table) {
+    if (flags->group_sums == nullptr) {
         P.todo = todo; P.todo_count = todo_count;
         ILLICO_CUDA_OK(cudaMemsetAsync(todo_count, 0, sizeof(int), stream));
         int tocc = 0;
@@ -778,8 +760,7 @@ int launch_ovr_mapped(const float* ir_vals, const uint32_t* ir_cnt, int n_genes,
         // segment-record area of the table kernel: behind the general kernel's slabs (both kernels may be resident)
         const size_t slabs = ((size_t)grid * slab_q * 8 + 255) & ~(size_t)255;
         const size_t rec_cta = ovr_table_rec_bytes(plan);
-        const char* renv = getenv("ILLICO_OVR_RECORDS");
-        if (!(renv && atoi(renv) == 0) && workspace_bytes >= slabs + (size_t)tgrid * rec_cta) {
+        if (workspace_bytes >= slabs + (size_t)tgrid * rec_cta) {
             P.table_rec = reinterpret_cast<uint4*>(reinterpret_cast<char*>(workspace) + slabs);
             P.table_rec_stride = (long long)(rec_cta / 16);
         }

@@ -12,8 +12,6 @@
 // element exactly once with warp-coalesced row segments and writes only the ~10 % that are non-zero.
 #include "common.cuh"
 
-#include <stdlib.h>
-
 namespace illico {
 
 constexpr int STAGE_WARPS = 8;
@@ -493,15 +491,13 @@ int launch_stage_dense(const float* X, long long ld, int gene_lb, int b, const i
     const int S = plan->n_segments;
     long long avg = plan->n_cells / S;
     if (avg < 1) avg = 1;
-    const char* rows_env = getenv("ILLICO_STAGE_ROWS");
     // ~512 cells per CTA: enough CTAs (tens of waves) that the last partial wave costs a few percent
-    int segs_per_cta = (int)((rows_env ? atoi(rows_env) : 512) / avg);
+    int segs_per_cta = (int)(512 / avg);
     if (segs_per_cta < 1) segs_per_cta = 1;
     if (segs_per_cta > STAGE_MAX_SEGS) segs_per_cta = STAGE_MAX_SEGS;
     long long gy = (S + segs_per_cta - 1) / segs_per_cta;
     // two genes per lane (64-bit loads) when the batch is 8-byte aligned
-    const char* v2 = getenv("ILLICO_STAGE_VEC");
-    const bool vec2 = (!v2 || atoi(v2) == 2) && ((reinterpret_cast<uintptr_t>(X) & 7) == 0) && (ld % 2 == 0) &&
+    const bool vec2 = ((reinterpret_cast<uintptr_t>(X) & 7) == 0) && (ld % 2 == 0) &&
                       (gene_lb % 2 == 0) && (b % 2 == 0);
     const int gpc = STAGE_WARPS * 32 * (vec2 ? 2 : 1);
     const unsigned gx = (unsigned)((b + gpc - 1) / gpc);

@@ -8,7 +8,7 @@
 // permuted cell rows and issues one bulk copy per row piece (`cp.async.bulk.shared.global`, SASS UBLKCP: 4 * GENES
 // bytes, global -> shared, completion counted on an mbarrier); the eight consumer warps read the rows from shared
 // memory.  The bytes in flight per SM are then a property of the ring (STAGES * ROWS * row piece per CTA), not of
-// the consumers' registers or issue slots, and a consumer spends one LDS per VEC elements instead of an address
+// the consumers' registers or issue slots, and a consumer spends one LDS per element instead of an address
 // computation, a shuffle and a global load.  The compaction is lane-private as before, but the lane's buffer holds
 // 8 + ROWS entries and is inspected once per ring stage instead of once per element, which removes the divergent
 // flush branch from the per-element path (it was a third of the old kernel's instructions).
@@ -50,13 +50,13 @@ __device__ __forceinline__ void flush_sector(float* dst, uint32_t buf) {
                  : "memory");
 }
 
-template <int VEC, int ROWS, int STAGES>
+template <int ROWS, int STAGES>
 struct TmaLayout {
-    static constexpr int GENES = TMA_CONSUMERS * VEC;         // genes per CTA
+    static constexpr int GENES = TMA_CONSUMERS;               // genes per CTA: one per consumer lane
     static constexpr int ROW_BYTES = GENES * 4;               // bytes of one row piece
     static constexpr int STAGE_BYTES = ROWS * ROW_BYTES;
     static constexpr int ENTRIES = 8 + ROWS;                  // lane buffer: < 8 left over + one stage's appends
-    static constexpr int WBUF_BYTES = VEC * TMA_CONSUMERS * ENTRIES * 4;
+    static constexpr int WBUF_BYTES = TMA_CONSUMERS * ENTRIES * 4;
     static constexpr int RING_OFF = 0;
     static constexpr int WBUF_OFF = STAGES * STAGE_BYTES;
     static constexpr int BAR_OFF = WBUF_OFF + WBUF_BYTES;     // 2 * STAGES mbarriers
@@ -64,17 +64,17 @@ struct TmaLayout {
     static size_t bytes(int segs_per_cta) { return (size_t)CNT_OFF + (size_t)segs_per_cta * GENES * 2; }
 };
 
-template <int VEC, int ROWS, int STAGES, int MINB>
+template <int ROWS, int STAGES, int MINB>
 __global__ void __launch_bounds__(TMA_THREADS, MINB) stage_dense_tma_kernel(const float* __restrict__ X, long long ld, int gene_lb,
                                                                       int b, const illico_plan_t pl,
                                                                       float* __restrict__ ir_vals,
                                                                       uint32_t* __restrict__ ir_cnt, int segs_per_cta, int seg_lo,
-                                                                      int seg_hi, int no_store, int tiles_x, int tiles_y,
+                                                                      int seg_hi, int tiles_x, int tiles_y,
                                                                       const int* __restrict__ mode_dev, int want_mode) {
     // A decision taken on the device (hand-back of the fused paths): the host enqueued this launch without knowing
     // whether it is needed.  Such launches are persistent (a fixed 1-D grid walking the tiles), so a no costs microseconds.
     if (mode_dev && *mode_dev != want_mode) return;
-    using L = TmaLayout<VEC, ROWS, STAGES>;
+    using L = TmaLayout<ROWS, STAGES>;
     static_assert(32 % ROWS == 0, "a 32-row group of the permutation holds whole stages");
     extern __shared__ __align__(128) unsigned char smem[];
     const uint32_t smem_a = (uint32_t)__cvta_generic_to_shared(smem);
@@ -82,7 +82,7 @@ __global__ void __launch_bounds__(TMA_THREADS, MINB) stage_dense_tma_kernel(cons
     uint16_t* cnt_tile = reinterpret_cast<uint16_t*>(smem + L::CNT_OFF);
     const int t = threadIdx.x, lane = t & 31, w = t >> 5;
     const int S = pl.n_segments;
-    // tiles: (256 * VEC genes) x (segs_per_cta segments).  A 2-D grid gives every CTA its own tile; a 1-D (persistent)
+    // tiles: (256 genes) x (segs_per_cta segments).  A 2-D grid gives every CTA its own tile; a 1-D (persistent)
     // grid walks them.  The ring's stage counters run on across tiles, so the producer fills the ring with the next
     // tile's rows while the consumers finish the current one.
     const int n_tiles = tiles_x * tiles_y;
@@ -137,69 +137,46 @@ __global__ void __launch_bounds__(TMA_THREADS, MINB) stage_dense_tma_kernel(cons
         return;
     }
 
-    // ---------------- consumer warps: lane = VEC adjacent genes
+    // ---------------- consumer warps: lane = gene
     int k = 0;                                                           // stage counter (runs on across tiles)
     for (int tile = tile0; tile < n_tiles; tile += tile_step) {
     const int bx = tile % tiles_x, by = tile / tiles_x;
     const int s_begin = seg_lo + by * segs_per_cta, s_end = min(seg_hi, s_begin + segs_per_cta);
     const int p_begin = pl.seg_pos[s_begin], p_end = pl.seg_pos[s_end];
     const int g0 = bx * L::GENES;
-    const int jb = g0 + t * VEC;
-    bool act[VEC];
-    float* gene_base[VEC];
-    uint32_t done[VEC], off[VEC], buf[VEC];
-#pragma unroll
-    for (int e = 0; e < VEC; ++e) {
-        act[e] = jb + e < b && !no_store;
-        gene_base[e] = ir_vals + (long long)(act[e] ? jb + e : 0) * pl.slot_cap;
-        done[e] = 0;
-        off[e] = 0;
-        buf[e] = smem_a + L::WBUF_OFF + ((e * TMA_CONSUMERS + t) * L::ENTRIES) * 4;
-    }
+    const int j = g0 + t;
+    const bool act = j < b;
+    float* const gene_base = ir_vals + (long long)(act ? j : 0) * pl.slot_cap;
+    uint32_t done = 0, off = 0;
+    const uint32_t buf = smem_a + L::WBUF_OFF + t * L::ENTRIES * 4;
     int s = s_begin;
     int seg_end = pl.seg_pos[s + 1];
     int seg_off = pl.seg_base[s];
     // closes segment s: the lane's leftovers leave as one or two padded sectors, the count goes to the tile
     auto finalize = [&]() {
-#pragma unroll
-        for (int e = 0; e < VEC; ++e) {
-            if (act[e]) {
-                float* dst = gene_base[e] + seg_off + done[e];
-                for (uint32_t o = 0; o < off[e]; o += 32u) flush_sector(dst + (o >> 2), buf[e] + o);
-            }
-            cnt_tile[(s - s_begin) * L::GENES + t * VEC + e] = (uint16_t)(done[e] + (off[e] >> 2));
-            done[e] = 0;
-            off[e] = 0;
+        if (act) {
+            float* dst = gene_base + seg_off + done;
+            for (uint32_t o = 0; o < off; o += 32u) flush_sector(dst + (o >> 2), buf + o);
         }
+        cnt_tile[(s - s_begin) * L::GENES + t] = (uint16_t)(done + (off >> 2));
+        done = 0;
+        off = 0;
     };
-    const unsigned char* my_ring = smem + L::RING_OFF + t * VEC * 4;
+    const unsigned char* my_ring = smem + L::RING_OFF + t * 4;
     for (int p = p_begin; p < p_end; p += ROWS, ++k) {
         const int slot = k % STAGES;
         mbar_wait(bars + 8 * slot, (k / STAGES) & 1);
         const int nr = min(ROWS, p_end - p);
         const unsigned char* src = my_ring + slot * L::STAGE_BYTES;
-        auto load_row = [&](float (&r)[VEC], int u) {
-            if (VEC == 4) {
-                const float4 q = *reinterpret_cast<const float4*>(src + u * L::ROW_BYTES);
-                r[0] = q.x; r[1 % VEC] = q.y; r[2 % VEC] = q.z; r[3 % VEC] = q.w;
-            } else if (VEC == 2) {
-                const float2 q = *reinterpret_cast<const float2*>(src + u * L::ROW_BYTES);
-                r[0] = q.x; r[1 % VEC] = q.y;
-            } else {
-                r[0] = *reinterpret_cast<const float*>(src + u * L::ROW_BYTES);
-            }
-        };
+        auto load_row = [&](int u) { return *reinterpret_cast<const float*>(src + u * L::ROW_BYTES); };
         if (p + ROWS <= seg_end) {
             // the whole stage lies inside the current segment (the usual case): the stage's rows first
             // (independent shared loads), then the dependent appends
-            float v[ROWS][VEC];
+            float v[ROWS];
 #pragma unroll
-            for (int u = 0; u < ROWS; ++u) load_row(v[u], u);
+            for (int u = 0; u < ROWS; ++u) v[u] = load_row(u);
 #pragma unroll
-            for (int u = 0; u < ROWS; ++u) {
-#pragma unroll
-                for (int e = 0; e < VEC; ++e) append_nz(off[e], v[u][e], buf[e]);
-            }
+            for (int u = 0; u < ROWS; ++u) append_nz(off, v[u], buf);
         } else {
             // a segment ends inside this stage (or the CTA's rows do): row by row
 #pragma unroll 1
@@ -210,28 +187,22 @@ __global__ void __launch_bounds__(TMA_THREADS, MINB) stage_dense_tma_kernel(cons
                     seg_end = pl.seg_pos[s + 1];
                     seg_off = pl.seg_base[s];
                 }
-                float r[VEC];
-                load_row(r, u);
-#pragma unroll
-                for (int e = 0; e < VEC; ++e) append_nz(off[e], r[e], buf[e]);
+                append_nz(off, load_row(u), buf);
             }
         }
         __syncwarp();
         if (lane == 0) mbar_arrive(bars + 8 * (STAGES + slot));          // this warp is done with the stage
         // once per stage: full sectors leave, the (< 8) leftovers move to the front of the lane's buffer
-#pragma unroll
-        for (int e = 0; e < VEC; ++e) {
-            if (off[e] >= 32u) {
-                const uint32_t full_bytes = off[e] & ~31u;
-                if (act[e]) {
-                    float* dst = gene_base[e] + seg_off + done[e];
-                    for (uint32_t o = 0; o < full_bytes; o += 32u) flush_sector(dst + (o >> 2), buf[e] + o);
-                }
-                sts128(buf[e], lds128(buf[e] + full_bytes));
-                if (ROWS >= 8) sts128(buf[e] + 16, lds128(buf[e] + full_bytes + 16));
-                done[e] += full_bytes >> 2;
-                off[e] -= full_bytes;
+        if (off >= 32u) {
+            const uint32_t full_bytes = off & ~31u;
+            if (act) {
+                float* dst = gene_base + seg_off + done;
+                for (uint32_t o = 0; o < full_bytes; o += 32u) flush_sector(dst + (o >> 2), buf + o);
             }
+            sts128(buf, lds128(buf + full_bytes));
+            if (ROWS >= 8) sts128(buf + 16, lds128(buf + full_bytes + 16));
+            done += full_bytes >> 2;
+            off -= full_bytes;
         }
     }
     for (;;) {                                                           // closes the last segment (and empty ones after it)
@@ -239,15 +210,12 @@ __global__ void __launch_bounds__(TMA_THREADS, MINB) stage_dense_tma_kernel(cons
         if (++s >= s_end) break;
         seg_off = pl.seg_base[s];
     }
-    // counts: thread t writes the consecutive segments of genes t, t + 256, ... (contiguous runs per gene)
+    // counts: thread t writes the consecutive segments of gene t (contiguous runs per gene)
     asm volatile("bar.sync 1, %0;" ::"r"(TMA_CONSUMERS) : "memory");
     const int nseg = s_end - s_begin;
-    for (int g = t; g < L::GENES; g += TMA_CONSUMERS) {
-        const int j = g0 + g;
-        if (j < b) {
-            uint32_t* dst = ir_cnt + (long long)j * S + s_begin;
-            for (int ls = 0; ls < nseg; ++ls) dst[ls] = cnt_tile[ls * L::GENES + g];
-        }
+    if (act) {
+        uint32_t* dst = ir_cnt + (long long)j * S + s_begin;
+        for (int ls = 0; ls < nseg; ++ls) dst[ls] = cnt_tile[ls * L::GENES + t];
     }
     asm volatile("bar.sync 1, %0;" ::"r"(TMA_CONSUMERS) : "memory");   // the count tile is free for the next tile
     }
@@ -258,17 +226,19 @@ int env_int(const char* name, int dflt) {
     return v ? atoi(v) : dflt;
 }
 
-template <int VEC, int ROWS, int STAGES, int MINB>
+constexpr int STAGE_ROWS = 512;   // rows a CTA stages: segments per CTA = STAGE_ROWS / average segment size
+
+template <int ROWS, int STAGES, int MINB>
 int launch_t(const float* X, long long ld, int gene_lb, int b, const illico_plan_t* plan, float* ir_vals, uint32_t* ir_cnt,
              int segs_per_cta, int seg_lo, int seg_hi, cudaStream_t stream, const int* mode_dev, int want_mode) {
-    using L = TmaLayout<VEC, ROWS, STAGES>;
+    using L = TmaLayout<ROWS, STAGES>;
     const unsigned gx = (unsigned)((b + L::GENES - 1) / L::GENES);
     const unsigned gy = (unsigned)((seg_hi - seg_lo + segs_per_cta - 1) / segs_per_cta);
     const size_t smem = L::bytes(segs_per_cta);
-    auto kern = stage_dense_tma_kernel<VEC, ROWS, STAGES, MINB>;
+    auto kern = stage_dense_tma_kernel<ROWS, STAGES, MINB>;
     ILLICO_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     dim3 grid(gx, gy);
-    if (mode_dev || env_int("ILLICO_STAGE_PERSIST", 0)) {   // decided on the device: persistent 1-D grid
+    if (mode_dev) {   // decided on the device: persistent 1-D grid
         int occ = 0;
         ILLICO_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, TMA_THREADS, smem));
         long long ctas = 148ll * (occ > 0 ? occ : 1);
@@ -278,7 +248,6 @@ int launch_t(const float* X, long long ld, int gene_lb, int b, const illico_plan
     }
     ILLICO_LAUNCH("stage_dense_tma_kernel", stream,
                   kern<<<grid, TMA_THREADS, smem, stream>>>(X, ld, gene_lb, b, *plan, ir_vals, ir_cnt, segs_per_cta, seg_lo, seg_hi,
-                                                            env_int("ILLICO_STAGE_TMA_NOSTORE", 0),   // (measurement aid: read path alone)
                                                             (int)gx, (int)gy, mode_dev, want_mode));
     ILLICO_CUDA_OK(cudaGetLastError());
     return 0;
@@ -304,26 +273,18 @@ int launch_stage_dense_tma_if(const float* X, long long ld, int gene_lb, int b, 
     if (seg_lo < 0 || seg_hi > S || seg_lo >= seg_hi) { set_error("segment range [%d, %d) out of bounds", seg_lo, seg_hi); return 1; }
     long long avg = plan->n_cells / S;
     if (avg < 1) avg = 1;
-    int segs_per_cta = segs_per_cta_req > 0 ? segs_per_cta_req : (int)(env_int("ILLICO_STAGE_ROWS", 512) / avg);
+    int segs_per_cta = segs_per_cta_req > 0 ? segs_per_cta_req : (int)(STAGE_ROWS / avg);
     if (segs_per_cta < 1) segs_per_cta = 1;
     if (segs_per_cta > TMA_MAX_SEGS) segs_per_cta = TMA_MAX_SEGS;
     if (!mode_dev && (S + segs_per_cta - 1) / segs_per_cta > 65535) return -1;      // caller falls back to the plain kernel
     // Ring configurations measured at the K562 shape (profiles/README.md): one gene per lane (1 KB row pieces) is the
-    // fastest and has the smallest footprint.
-    switch (env_int("ILLICO_STAGE_TMA_CFG", 0)) {
-        case 1: return launch_t<2, 4, 4, 2>(X, ld, gene_lb, b, plan, ir_vals, ir_cnt, segs_per_cta, seg_lo, seg_hi, stream, mode_dev, want_mode);
-        case 2: return launch_t<2, 8, 4, 2>(X, ld, gene_lb, b, plan, ir_vals, ir_cnt, segs_per_cta, seg_lo, seg_hi, stream, mode_dev, want_mode);
-        case 3: return launch_t<4, 4, 3, 2>(X, ld, gene_lb, b, plan, ir_vals, ir_cnt, segs_per_cta, seg_lo, seg_hi, stream, mode_dev, want_mode);
-        case 4: return launch_t<1, 8, 4, 3>(X, ld, gene_lb, b, plan, ir_vals, ir_cnt, segs_per_cta, seg_lo, seg_hi, stream, mode_dev, want_mode);
-        case 5: return launch_t<1, 8, 6, 2>(X, ld, gene_lb, b, plan, ir_vals, ir_cnt, segs_per_cta, seg_lo, seg_hi, stream, mode_dev, want_mode);
-        default: break;
-    }
-    // measured (scripts/exp/stage_persist.sh, continuous K562 shape): 72 registers / 3 CTAs per SM 2.01 ms as a 2-D grid and
-    // 2.14 ms persistent; 96 registers / 2 CTAs per SM with a 6-stage ring 2.05 / 2.09 ms; 56 registers / 4 CTAs per SM
-    // spills in the per-element loop and takes 3.4 ms
-    if (mode_dev || env_int("ILLICO_STAGE_PERSIST", 0))
-        return launch_t<1, 8, 6, 2>(X, ld, gene_lb, b, plan, ir_vals, ir_cnt, segs_per_cta, seg_lo, seg_hi, stream, mode_dev, want_mode);
-    return launch_t<1, 8, 4, 3>(X, ld, gene_lb, b, plan, ir_vals, ir_cnt, segs_per_cta, seg_lo, seg_hi, stream, mode_dev, want_mode);
+    // fastest and has the smallest footprint.  Measured on the continuous K562 shape: 72 registers / 3 CTAs per SM
+    // 2.01 ms as a 2-D grid and 2.14 ms persistent; 96 registers / 2 CTAs per SM with a 6-stage ring 2.05 / 2.09 ms;
+    // 56 registers / 4 CTAs per SM spills in the per-element loop and takes 3.4 ms.  A launch decided on the device
+    // has to be persistent, and takes the 6-stage ring.
+    if (mode_dev)
+        return launch_t<8, 6, 2>(X, ld, gene_lb, b, plan, ir_vals, ir_cnt, segs_per_cta, seg_lo, seg_hi, stream, mode_dev, want_mode);
+    return launch_t<8, 4, 3>(X, ld, gene_lb, b, plan, ir_vals, ir_cnt, segs_per_cta, seg_lo, seg_hi, stream, mode_dev, want_mode);
 }
 
 int launch_stage_dense_tma(const float* X, long long ld, int gene_lb, int b, const illico_plan_t* plan, float* ir_vals,

@@ -211,8 +211,6 @@ class Engine:
                 rc = fn(M.data.data_ptr(), M.ld, lb, b, C.byref(self.plan), C.byref(flags), C.byref(buf), out_ptr,
                         gstride, dbg_ref, st)
             else:
-                if M.fmt == "csr" and flags.n_cols_hint != M.shape[1]:
-                    flags = flags.replace(n_cols_hint=int(M.shape[1]))
                 fn = getattr(self.lib, f"illico_{test}_{M.fmt}_f32")
                 rc = fn(M.data.data_ptr(), M.indices.data_ptr(), M.indptr.data_ptr(), lb, b, C.byref(self.plan),
                         C.byref(flags), C.byref(buf), out_ptr, gstride, dbg_ref, st)
@@ -268,7 +266,7 @@ class Engine:
                                                     ws.data_ptr(), ws.numel(), st)
                     sub, sub_lb = DeviceMatrix(CSR, M.shape, codes, M.indices, M.indptr), a
                 _lib.check(rc, f"illico_recode_{M.fmt}")
-            f2 = flags.replace(n_cols_hint=0, group_sums=sums.data_ptr())
+            f2 = flags.replace(group_sums=sums.data_ptr())
             dbg = {} if debug is not None else None
             self.run_batch(sub, sub_lb, sub_lb + b, f2, results, result_gene0 + (a - lb), dbg, scores)
             if debug is not None:

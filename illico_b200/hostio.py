@@ -203,7 +203,7 @@ def h2d_2d(dst: torch.Tensor, src: np.ndarray, n_threads: int | None = None, all
     # 0.075 s); eight links carry 186 GB/s and win.  A pageable source has to be touched by the CPU anyway.
     feeding = int(os.environ.get("LOCAL_WORLD_SIZE", "1") or 1) * max(1, CONCURRENT_UPLOADS)
     if allow_pack and (not pinned_src or feeding <= 4 or os.environ.get("ILLICO_PACK_UPLOAD") == "1") and _pack_wanted(src, n, b):
-        return _h2d_2d_packed(dst, src, pinned_src, n_threads)
+        return _h2d_2d_packed(dst, src, n_threads)
     if pinned_src:
         if src.strides[0] == b * item:      # contiguous: one linear asynchronous copy
             with warnings.catch_warnings():
@@ -281,12 +281,13 @@ def _pack_wanted(src: np.ndarray, n: int, b: int) -> bool:
     return float(np.count_nonzero(sample)) <= 0.3 * sample.size
 
 
-def _h2d_2d_packed(dst: torch.Tensor, src: np.ndarray, pinned_src: bool, n_threads: int | None) -> Pending:
+def _h2d_2d_packed(dst: torch.Tensor, src: np.ndarray, n_threads: int | None) -> Pending:
     """The upload of a mostly-zero float32 matrix with the host threads squeezing the row chunks (bit mask + non-zero
     values, ``illico_host_pack_rows_f32``) instead of copying them: the packed chunk crosses PCIe (about 1/8 of the bytes
     at 10 % density) and ``illico_unpack_rows_f32`` rebuilds the rows in the destination.  The threads share one queue
-    of chunks.  (``ILLICO_PACK_DMA_WORKER=1``: when the source is pinned an extra worker takes chunks off the same queue
-    and sends them as they are -- plain DMA, two in flight; measured slower, see below.)"""
+    of chunks.  (A worker sending chunks of a pinned source as they are, beside the squeeze threads, measured slower on
+    the K562 matrix: the squeeze threads slow down ten-fold while plain DMA out of the same pinned pages is running;
+    0.17 s against 0.10 s with the threads alone.)"""
     lib = _lib.load()
     device = dst.device
     n, b = src.shape
@@ -299,7 +300,7 @@ def _h2d_2d_packed(dst: torch.Tensor, src: np.ndarray, pinned_src: bool, n_threa
     counter = iter(range(n_chunks))
     counter_lock = threading.Lock()
     pending = Pending(device, ring=ring)
-    final_events = [None] * (T + 1)
+    final_events = [None] * T
     cur = torch.cuda.current_stream(device)
     dev_index = device.index if device.index is not None else torch.cuda.current_device()
     start_event = torch.cuda.Event()
@@ -363,37 +364,7 @@ def _h2d_2d_packed(dst: torch.Tensor, src: np.ndarray, pinned_src: bool, n_threa
         except BaseException as e:  # surfaced by finish()
             pending.error = e
 
-    def dma_worker():
-        """Pinned sources: chunks sent as they are, two in flight, while the other threads squeeze theirs."""
-        try:
-            with torch.cuda.device(device):
-                st = torch.cuda.Stream(device=device)
-                st.wait_event(start_event)
-                inflight = []
-                while True:
-                    if len(inflight) == 2:
-                        inflight.pop(0).synchronize()
-                    c = take()
-                    if c is None:
-                        break
-                    r0 = c * rows_per_chunk
-                    r1 = min(n, r0 + rows_per_chunk)
-                    copy2d_async(dst_ptr + r0 * row_bytes, row_bytes, src_ptr + r0 * src_stride, src_stride, row_bytes, r1 - r0, "h2d", st)
-                    ev = torch.cuda.Event()
-                    ev.record(st)
-                    inflight.append(ev)
-                    final_events[T] = ev
-                    stats["raw"] += 1
-                    stats["bytes"] += (r1 - r0) * row_bytes
-        except BaseException as e:
-            pending.error = e
-
     threads = [threading.Thread(target=worker, args=(t,), daemon=True) for t in range(T)]
-    # (off by default: measured on the K562 matrix, scripts/exp/pack_chunks.py, the squeeze threads slow down ten-fold
-    # while plain DMA out of the same pinned pages is running, and the DMA worker ends up with most chunks: 0.17 s
-    # against 0.10 s with the threads alone)
-    if pinned_src and os.environ.get("ILLICO_PACK_DMA_WORKER", "0") == "1":
-        threads.append(threading.Thread(target=dma_worker, daemon=True))
     pending.threads, pending.events = threads, final_events
     for th in threads:
         th.start()

@@ -103,7 +103,7 @@ typedef struct illico_flags {
     int32_t tie_correct;    /* 0 -> tie sum := 0 in the p-value (ovr/dense_ovr.py:70) */
     int32_t alternative;    /* enum illico_alternative */
     int32_t tie_order;      /* enum illico_tie_order */
-    int32_t n_cols_hint;    /* CSR dispatchers: number of columns of the whole matrix (0 = unknown; only guides a search) */
+    int32_t n_cols_hint;    /* unused (kept so that the layout stays as in ABI version 3); pass 0 */
     /* Optional [n_groups, n_genes_batch] float64 expression sums (device).  When set, the fold change uses them
      * instead of sums of the staged values: the host stages ORDER-PRESERVING float32 codes of values that
      * float32 cannot hold (float64 / large integers), which keeps U, ties and p exact. */

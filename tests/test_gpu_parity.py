@@ -1006,8 +1006,7 @@ def test_native_recoding_of_float64_values(fmt):
 def test_packed_upload_rebuilds_the_matrix(monkeypatch, source):
     """hostio._h2d_2d_packed (csrc/hostpack.c + unpack_rows_kernel): a mostly-zero float32 matrix squeezed on the host
     (bit mask + values), sent packed and rebuilt in HBM is the matrix, bit for bit -- NaN kept, -0.0 a zero; pinned
-    sources (with the plain-DMA worker taking chunks off the same queue), column shards of a wider matrix, and chunks too
-    dense to squeeze (sent as they are)."""
+    sources, column shards of a wider matrix, and chunks too dense to squeeze (sent as they are)."""
     import torch
 
     from illico_b200 import hostio
@@ -1015,7 +1014,6 @@ def test_packed_upload_rebuilds_the_matrix(monkeypatch, source):
     monkeypatch.setenv("ILLICO_STAGE_CHUNK_MB", "4")
     monkeypatch.setattr(hostio, "CHUNK_BYTES", 4 << 20)
     monkeypatch.setenv("ILLICO_PACK_UPLOAD", "1")
-    monkeypatch.setenv("ILLICO_PACK_DMA_WORKER", "1")
     rng = np.random.RandomState(4)
     n, N = 9000, 2117
     X = (rng.poisson(1.0, (n, N)) * (rng.rand(n, N) < 0.12)).astype(np.float32)

@@ -39,6 +39,20 @@ def test_product_never_imports_oracle():
                 assert "liboracle" not in src, f
 
 
+def test_environment_switches_match_design_table():
+    """Every environment variable the package reads is listed in DESIGN.md's switch table, and the table lists no
+    variable the package no longer reads."""
+    read = set()
+    for dirpath, _, files in os.walk(os.path.join(ROOT, "illico_b200")):
+        for f in files:
+            if f.endswith((".py", ".cu", ".cuh", ".c", ".h")):
+                read |= set(re.findall(r"[\"'](ILLICO_[A-Z0-9_]+)[\"']", open(os.path.join(dirpath, f)).read()))
+    design = open(os.path.join(ROOT, "DESIGN.md")).read()
+    table = design.split("### Environment switches", 1)[1].split("\n#", 1)[0]
+    rows = [line.split("|")[1] for line in table.splitlines() if line.startswith("| `")]
+    listed = set(re.findall(r"`(ILLICO_[A-Z0-9_]+)`", "".join(rows)))
+    assert read == listed, f"read but not listed: {sorted(read - listed)}; listed but not read: {sorted(listed - read)}"
+
 def test_no_gpu_means_loud_failure():
     import torch
 
