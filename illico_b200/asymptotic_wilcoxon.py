@@ -25,7 +25,7 @@ from scipy import sparse
 
 from . import hostio
 from .engine import CSR, DeviceMatrix, Engine, make_flags, require_cuda
-from .groups import encode_and_count_groups
+from .groups import encode_and_count_groups, seg_max_from_env
 from .registry import DataHandler, data_handler_registry
 
 __all__ = ["asymptotic_wilcoxon"]
@@ -175,6 +175,7 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
     data_handler = data_handler_registry.get(X)  # KeyError for unsupported containers, like the reference
     if devices is None and device is None and isinstance(X, torch.Tensor) and X.is_cuda:
         device = X.device          # a device-resident matrix is ranked where it lives
+    seg_max = seg_max_from_env()   # an invalid ILLICO_B200_SEG_MAX fails before any device work
     devs = _device_list(device, devices)
     n_cells, n_genes = X.shape
     fmt = data_handler.kernel_data_format().value
@@ -274,7 +275,7 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
             raise ValueError(f"{grpc.encoded_groups.size} group labels for {n_cells} cells")
         from .groups import build_plan
 
-        shared["grpc"], shared["host_plan"] = grpc, build_plan(grpc, _seg_max())
+        shared["grpc"], shared["host_plan"] = grpc, build_plan(grpc, seg_max)
         G = int(grpc.counts.size)
         if not on_device:
             shared["out"] = torch.empty((G, n_genes, 3), dtype=torch.float64, pin_memory=True)
@@ -324,15 +325,6 @@ def _bh_adjust(out: np.ndarray, device) -> np.ndarray:
         torch.cuda.current_stream(device).synchronize()
     del C
     return host.numpy()
-
-
-def _seg_max() -> int:
-    import os
-
-    try:
-        return int(os.environ.get("ILLICO_B200_SEG_MAX", 512))
-    except ValueError:
-        return 512
 
 
 def _result_frame(groups, var_names, out: np.ndarray, extra: dict | None = None) -> pd.DataFrame:

@@ -347,6 +347,9 @@ __global__ void __launch_bounds__(OVO_THREADS, OVO_MIN_CTAS) ovo_kernel(const Ov
     uint32_t* gA = slab;            // block-tier group buffers (global)
     uint32_t* gB = slab + maxg;
     __shared__ int mmax3[3];
+    __shared__ int ref_nnz_s;  // the control's non-zeros (thread 0's prefix over its segments)
+    // control segments whose offsets hist[] holds at a time (+1 entry: the start of the next chunk)
+    constexpr int REF_SEG_CHUNK = OVO_NW * 256 - 1;
 
     const int ref_s0 = pl.group_seg[ref], ref_s1 = pl.group_seg[ref + 1];
     if (tid < 8) counters[tid] = 0;
@@ -368,15 +371,20 @@ __global__ void __launch_bounds__(OVO_THREADS, OVO_MIN_CTAS) ovo_kernel(const Ov
         const float* vals = P.ir_vals + (long long)j * pl.slot_cap;
 
         // ================= phase 1: the control, once per gene =================
-        // offsets of the control's segments (few): serial prefix by thread 0 into hist[] (free now)
+        // offsets of the control's segments: serial prefix by thread 0 into hist[] (free now).  hist[] holds the offsets
+        // of the first REF_SEG_CHUNK segments and the start of the next one; the sort path refills it for the others.
         if (tid == 0) {
             uint32_t acc = 0;
-            for (int s = ref_s0; s < ref_s1; ++s) { hist[s - ref_s0] = acc; acc += cnt[s]; }
-            hist[ref_s1 - ref_s0] = acc;
+            for (int s = ref_s0; s < ref_s1; ++s) {
+                if (s - ref_s0 <= REF_SEG_CHUNK) hist[s - ref_s0] = acc;
+                acc += cnt[s];
+            }
+            if (ref_s1 - ref_s0 <= REF_SEG_CHUNK) hist[ref_s1 - ref_s0] = acc;
+            ref_nnz_s = (int)acc;
             counters[6] = 0;
         }
         __syncthreads();
-        const int nref_nz = (int)hist[ref_s1 - ref_s0];
+        const int nref_nz = ref_nnz_s;
         const bool ref_smem = nref_nz <= REF_CAP;
         RefInfo R;
         R.nnz = nref_nz;
@@ -466,16 +474,28 @@ __global__ void __launch_bounds__(OVO_THREADS, OVO_MIN_CTAS) ovo_kernel(const Ov
             // ---- sort path: control keys in shared memory when they fit, else in this CTA's global slab
             uint32_t* rA = ref_smem ? refA : slab + 2ll * maxg;
             uint32_t* rB = ref_smem ? scratch : slab + 3ll * maxg;
-            for (int s = ref_s0 + w; s < ref_s1; s += OVO_NW) {
-                const uint32_t off = hist[s - ref_s0];
-                const int c = (int)cnt[s];
-                const float* src = vals + pl.seg_base[s];
-                for (int i = lane; i < c; i += 32) {
-                    const float v = src[i];
-                    uint32_t key = f2key(v);
-                    if (key == 0u) key = 1u;
-                    rA[off + i] = key;
-                    rsum += fc_val<LOG1P>(v);
+            for (int c0 = ref_s0; c0 < ref_s1; c0 += REF_SEG_CHUNK) {
+                const int c1 = min(ref_s1, c0 + REF_SEG_CHUNK);
+                if (c0 > ref_s0) {   // (CTA-uniform) offsets of the next chunk, from the start hist[REF_SEG_CHUNK] left
+                    __syncthreads();
+                    if (tid == 0) {
+                        uint32_t acc = hist[REF_SEG_CHUNK];
+                        for (int s = c0; s < c1; ++s) { hist[s - c0] = acc; acc += cnt[s]; }
+                        hist[c1 - c0] = acc;
+                    }
+                    __syncthreads();
+                }
+                for (int s = c0 + w; s < c1; s += OVO_NW) {
+                    const uint32_t off = hist[s - c0];
+                    const int c = (int)cnt[s];
+                    const float* src = vals + pl.seg_base[s];
+                    for (int i = lane; i < c; i += 32) {
+                        const float v = src[i];
+                        uint32_t key = f2key(v);
+                        if (key == 0u) key = 1u;
+                        rA[off + i] = key;
+                        rsum += fc_val<LOG1P>(v);
+                    }
                 }
             }
             __syncthreads();

@@ -542,6 +542,8 @@ int launch_stage_csr_if(const float* data, const int32_t* indices, const long lo
     if (segs_per_cta > CSR_MAX_SEGS) segs_per_cta = CSR_MAX_SEGS;
     const long long gy = (S + segs_per_cta - 1) / segs_per_cta;
     if (gy > 65535) { set_error("too many segments (%d) for one CSR staging launch", S); return 1; }
+    // (a partial check only: it catches plans whose groups were not cut at all.  The guarantee that every segment has
+    // fewer than 65536 cells is the plan's own -- HostPlan refuses longer segments, see seg_pos in illico_b200.h)
     if (plan->max_group_size >= 65536 && plan->n_segments == plan->n_groups) {
         set_error("segments of 65536 or more cells are not supported by the CSR staging kernel");
         return 1;

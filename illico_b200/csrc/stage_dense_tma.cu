@@ -260,6 +260,8 @@ bool stage_dense_tma_ok(const float* X, long long ld, int gene_lb, int b, const 
     if (env_int("ILLICO_STAGE_TMA", 1) == 0) return false;
     if ((reinterpret_cast<uintptr_t>(X) & 15) || (ld & 3) || (gene_lb & 3)) return false;
     if (gene_lb + ((b + 3) & ~3) > ld) return false;            // the last piece would leave the row
+    // (a partial check only, for plans whose groups were not cut at all: every plan must keep its segments under
+    // 65536 cells -- HostPlan refuses longer ones, see seg_pos in illico_b200.h)
     if (plan->max_group_size >= 65536 && plan->n_segments == plan->n_groups) return false;
     return true;
 }

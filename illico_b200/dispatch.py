@@ -19,6 +19,7 @@ import numpy as np
 import torch
 
 from .engine import CSC, CSR, DENSE, DeviceMatrix, Engine, make_flags
+from .groups import seg_max_from_env
 
 CSCMatrix = namedtuple("CSCMatrix", ["data", "indices", "indptr", "shape"])
 CSRMatrix = namedtuple("CSRMatrix", ["data", "indices", "indptr", "shape"])
@@ -55,17 +56,19 @@ def _fingerprint(a) -> int:
 
 
 def engine_for(grpc, device=None) -> Engine:
-    """One engine per (group encoding CONTENT, reference group, device); tiny LRU so that the reference's driver,
-    which calls a dispatcher once per gene batch with the same GroupContainer, reuses the plan.  Keyed on a checksum
-    of the codes (2.4 MB at 300k cells, about a millisecond), not on an address: a relabelled or re-created array
-    never returns a stale plan."""
+    """One engine per (group encoding CONTENT, reference group, plan segment length, device); tiny LRU so that the
+    reference's driver, which calls a dispatcher once per gene batch with the same GroupContainer, reuses the plan.
+    Keyed on a checksum of the codes (2.4 MB at 300k cells, about a millisecond), not on an address: a relabelled or
+    re-created array never returns a stale plan, and a changed ``ILLICO_B200_SEG_MAX`` builds a new one."""
     dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
     enc = np.ascontiguousarray(grpc.encoded_groups, dtype=np.int64)
-    key = (zlib.crc32(enc.view(np.uint8)), zlib.adler32(enc.view(np.uint8)), enc.size, int(grpc.encoded_ref_group), str(dev))
+    seg_max = seg_max_from_env()
+    key = (zlib.crc32(enc.view(np.uint8)), zlib.adler32(enc.view(np.uint8)), enc.size, int(grpc.encoded_ref_group), seg_max,
+           str(dev))
     with _lock:
         eng = _engines.get(key)
         if eng is None:
-            eng = Engine(grpc, dev)
+            eng = Engine(grpc, dev, seg_max=seg_max)
             _engines[key] = eng
             while len(_engines) > _MAX_CACHE:
                 _engines.popitem(last=False)

@@ -15,7 +15,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .groups import GroupContainer, HostPlan, build_plan
+from .groups import GroupContainer, HostPlan, build_plan, check_seg_max
 
 DENSE, CSC, CSR = "dense", "csc", "csr"
 
@@ -82,11 +82,14 @@ def require_cuda(device=None) -> torch.device:
 
 class Engine:
     def __init__(self, grpc: GroupContainer, device=None, seg_max: int | None = None, host_plan: HostPlan | None = None):
+        if seg_max is not None:
+            check_seg_max(seg_max)     # (argument errors before any device work)
         self.lib = _lib.load()
         self.device = require_cuda(device)
         self.grpc = grpc
         # the host-side plan does not depend on the device: one per run, shared by the engines of all GPUs
-        self.host_plan: HostPlan = host_plan or build_plan(grpc, seg_max or _env_int("ILLICO_B200_SEG_MAX", 512))
+        # (seg_max None: ILLICO_B200_SEG_MAX, else 512; build_plan refuses a length outside [1, 65535])
+        self.host_plan: HostPlan = host_plan or build_plan(grpc, seg_max)
         hp = self.host_plan
         with torch.cuda.device(self.device):
             self._tables = {k: torch.from_numpy(getattr(hp, k)).to(self.device) for k in HostPlan.TABLES}

@@ -25,6 +25,10 @@ GroupContainer = namedtuple(
 )
 
 SEG_MAX_DEFAULT = 512
+# Longest segment a plan may have: the kernels count a segment's cells in 16-bit counters (the staging kernels' count
+# tiles, the one-versus-rest table bins, the fused CSR pass's control histogram).
+SEG_MAX_LIMIT = 65535
+SEG_MAX_ENV = "ILLICO_B200_SEG_MAX"
 # Slots start on, and are padded to, a multiple of this many floats (a multiple of 8 = one 32-byte sector).  32 floats
 # = one 128-byte line: a typical slot (~15 non-zeros of a ~150-cell group) then lies in ONE line / 64-byte fetch
 # granule instead of straddling two (measured: staging 2.10 -> 2.01 ms at the K562 shape).
@@ -97,10 +101,34 @@ def _is_stable_group_order(enc, perm) -> bool:
     return bool(np.all(np.diff(perm)[same] > 0))
 
 
-class HostPlan:
-    """numpy form of ``illico_plan_t``."""
+def check_seg_max(seg_max) -> int:
+    """``seg_max`` as an int, or a ``ValueError`` naming ``ILLICO_B200_SEG_MAX`` unless it is an integer in
+    ``[1, SEG_MAX_LIMIT]``."""
+    if isinstance(seg_max, (bool, np.bool_)) or not isinstance(seg_max, (int, np.integer)):
+        raise ValueError(f"{SEG_MAX_ENV} (plan segment length) must be an integer, got {seg_max!r}")
+    if not 1 <= seg_max <= SEG_MAX_LIMIT:
+        raise ValueError(f"{SEG_MAX_ENV} (plan segment length) must be in [1, {SEG_MAX_LIMIT}], got {seg_max}")
+    return int(seg_max)
 
-    def __init__(self, grpc: GroupContainer, seg_max: int = SEG_MAX_DEFAULT):
+
+def seg_max_from_env() -> int:
+    """The plan segment length: ``ILLICO_B200_SEG_MAX`` if set, else 512.  An invalid value is an error."""
+    raw = os.environ.get(SEG_MAX_ENV)
+    if raw is None:
+        return SEG_MAX_DEFAULT
+    try:
+        value = int(raw.strip())
+    except ValueError:
+        raise ValueError(f"{SEG_MAX_ENV} (plan segment length) must be an integer, got {raw!r}") from None
+    return check_seg_max(value)
+
+
+class HostPlan:
+    """numpy form of ``illico_plan_t``.  ``seg_max`` (default: :func:`seg_max_from_env`) must lie in
+    ``[1, SEG_MAX_LIMIT]``."""
+
+    def __init__(self, grpc: GroupContainer, seg_max: int | None = None):
+        seg_max = seg_max_from_env() if seg_max is None else check_seg_max(seg_max)
         enc = np.asarray(grpc.encoded_groups, dtype=np.int64)
         counts = np.asarray(grpc.counts, dtype=np.int64)
         n, G = enc.size, counts.size
@@ -149,5 +177,5 @@ class HostPlan:
     TABLES = ("perm", "cell_seg", "seg_pos", "seg_base", "seg_group", "group_seg", "group_size")
 
 
-def build_plan(grpc: GroupContainer, seg_max: int = SEG_MAX_DEFAULT) -> HostPlan:
+def build_plan(grpc: GroupContainer, seg_max: int | None = None) -> HostPlan:
     return HostPlan(grpc, seg_max)

@@ -90,7 +90,10 @@ typedef struct illico_plan {
     int32_t max_target_group_size; /* largest group other than the reference group (= max_group_size without one) */
     const int32_t* perm;        /* [n_cells]     perm[pos] = cell (row) index, groups contiguous, stable */
     const int32_t* cell_seg;    /* [n_cells]     segment of each cell (row -> segment) */
-    const int32_t* seg_pos;     /* [n_segments+1] positions (into perm) covered by each segment */
+    const int32_t* seg_pos;     /* [n_segments+1] positions (into perm) covered by each segment.  Every segment must
+                                   have fewer than 65536 cells (seg_pos[s+1] - seg_pos[s] <= 65535): the staging kernels'
+                                   count tiles, the one-versus-rest table bins and the fused CSR pass's control
+                                   histogram count a segment's cells in 16 bits.  Not checked here. */
     const int32_t* seg_base;    /* [n_segments+1] slot offset of each segment inside a gene's slot space */
     const int32_t* seg_group;   /* [n_segments]  owning group */
     const int32_t* group_seg;   /* [n_groups+1]  segments of each group */
