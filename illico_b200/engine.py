@@ -238,6 +238,8 @@ class Engine:
             M._codes = torch.empty(raw.shape, dtype=torch.float32, device=dev)     # parallel to the stored values
         # dense / CSR key lists have one slot per cell and gene: a sub-batch holds at most 2^26 of them (1 GB of keys)
         step = (ub - lb) if M.fmt == CSC else max(1, min(ub - lb, (1 << 26) // max(n, 1)))
+        if M.fmt == DENSE and 4 <= step < ub - lb:
+            step -= step % 4     # every sub-batch but the last starts on a 16-byte boundary of the input's rows
         for a in range(lb, ub, step):
             z = min(ub, a + step)
             b = z - a
@@ -245,7 +247,7 @@ class Engine:
                 sums = torch.empty((G, b), dtype=torch.float64, device=dev)
                 if M.fmt == DENSE:
                     keys = n * b
-                    codes = torch.empty((n, b), dtype=torch.float32, device=dev)
+                    codes = torch.empty((n, b), dtype=torch.float32, device=dev)   # (the recode kernel writes [n, b] rows)
                 elif M.fmt == CSC:
                     keys = int(M.indptr[z]) - int(M.indptr[a])
                     codes = M._codes
@@ -269,6 +271,8 @@ class Engine:
                                                     ws.data_ptr(), ws.numel(), st)
                     sub, sub_lb = DeviceMatrix(CSR, M.shape, codes, M.indices, M.indptr), a
                 _lib.check(rc, f"illico_recode_{M.fmt}")
+                if M.fmt == DENSE:
+                    sub.data = _padded_rows(codes, st)
             f2 = flags.replace(group_sums=sums.data_ptr())
             dbg = {} if debug is not None else None
             self.run_batch(sub, sub_lb, sub_lb + b, f2, results, result_gene0 + (a - lb), dbg, scores)
@@ -279,6 +283,20 @@ class Engine:
         if debug is not None and "_parts" in debug:
             for k, parts in debug.pop("_parts").items():
                 debug[k] = torch.cat(parts, dim=-1)
+
+
+def _padded_rows(codes: torch.Tensor, stream: int) -> torch.Tensor:
+    """A ``[n, b]`` view of ``codes`` whose rows are 16-byte aligned (stride rounded up to 4 floats, padding zeroed): the
+    TMA staging kernel and the dense fused path take only such rows, so recoded batches of any width reach them."""
+    n, b = codes.shape
+    ld = (b + 3) & ~3
+    if ld == b:
+        return codes
+    out = torch.empty((n, ld), dtype=torch.float32, device=codes.device)
+    out[:, b:].zero_()
+    _lib.check(_lib.load().illico_memcpy2d_async(out.data_ptr(), ld * 4, codes.data_ptr(), b * 4, b * 4, n, 3, stream),
+               "illico_memcpy2d_async")
+    return out[:, :b]
 
 
 _TORCH_OK = (np.float32, np.float64, np.float16, np.int8, np.uint8, np.int16, np.int32, np.int64)
