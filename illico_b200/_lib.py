@@ -97,6 +97,12 @@ SIGNATURES = {
     "illico_bh_adjust": (C.c_int, [_vp, _i64, _i64, _i32, _i32, _vp, _vp, _sz, _vp]),
     "illico_top_genes_workspace_bytes": (_sz, [_i32, _i32]),
     "illico_top_genes": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _sz, _vp]),
+    "illico_top_genes_filtered": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _vp, _vp, _i32, _i32, _i32, _i32, C.c_double, C.c_double,
+                                            C.c_double, C.c_double, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "illico_count_nonzero_dense": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _PP, _vp, _i64, _vp]),
+    "illico_count_nonzero_csr": (C.c_int, [_vp, _i32, _vp, _vp, _i32, _i32, _PP, _vp, _i64, _vp]),
+    "illico_count_nonzero_csc": (C.c_int, [_vp, _i32, _vp, _vp, _i32, _i32, _PP, _vp, _i64, _vp]),
+    "illico_nonzero_fractions": (C.c_int, [_vp, _i64, _vp, _i32, _i32, _i32, _i64, _vp, _vp, _vp]),
     "illico_compute_pval_batch": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
 }
 

@@ -114,6 +114,7 @@ def asymptotic_wilcoxon(
     p_adjust: bool = False,
     log2_fold_change: bool = False,
     score: bool = False,
+    pts: bool = False,
 ):
     """Asymptotic Mann-Whitney / Wilcoxon rank-sum tests for every (group, gene) on B200 GPUs.
 
@@ -133,12 +134,17 @@ def asymptotic_wilcoxon(
       ``score``    add the column ``score``: the signed z of the normal approximation, ``(n_r n_t / 2 - U) / sigma`` with
                    the p-value's (tie-corrected) sigma and no continuity correction -- positive when the group ranks above
                    the reference / rest, 0 on the reference row and where p = 1 (scanpy's wilcoxon ``scores``).  Written
-                   by the kernels next to the p-value.
+                   by the kernels next to the p-value;
+      ``pts``      add the columns ``pct_nz_group`` (fraction of the group's cells whose value is non-zero) and
+                   ``pct_nz_reference`` (the same fraction in the reference group, or in all other cells for one-versus-rest;
+                   NaN when there are no other cells) -- scanpy's ``rank_genes_groups(pts=True)``.  Counted on the GPU in a
+                   pass of its own; p-values, U and fold changes are those of the same call without it.
     With ``return_array`` and an optional column, the result is ``(groups, var_names, results, {name: [G, N] array})``.
     """
     del precompile  # kernels are compiled ahead of time
+    check_flag("pts", pts)
     run = _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, alternative, use_continuity,
-                     tie_correct, layer, device, devices, score=score, on_device=False)
+                     tie_correct, layer, device, devices, score=score, on_device=False, pts=pts)
     out = run.results
     extra = {}
     if p_adjust:
@@ -148,6 +154,8 @@ def asymptotic_wilcoxon(
             extra["log2_fold_change"] = np.log2(out[:, :, 2])
     if score:
         extra["score"] = run.scores
+    if pts:
+        extra["pct_nz_group"], extra["pct_nz_reference"] = _host_fractions(run)
     if return_array:
         if extra:
             return run.groups, np.asarray(adata.var_names), out, extra
@@ -157,18 +165,57 @@ def asymptotic_wilcoxon(
 
 class _Run:
     """What ``_run_tests`` delivers: the groups (``np.unique`` order), the group container, the first GPU, and the results
-    ``[G, N, 3]`` / score plane ``[G, N]`` (None unless asked for) -- pinned host arrays, or tensors on that GPU."""
+    ``[G, N, 3]`` / score plane ``[G, N]`` / int32 count plane ``[G, N]`` of cells with a non-zero value (the planes None
+    unless asked for) -- pinned host arrays, or tensors on that GPU."""
 
-    def __init__(self, groups, grpc, device, results, scores):
-        self.groups, self.grpc, self.device, self.results, self.scores = groups, grpc, device, results, scores
+    def __init__(self, groups, grpc, device, results, scores, nnz=None):
+        self.groups, self.grpc, self.device, self.results, self.scores, self.nnz = groups, grpc, device, results, scores, nnz
+
+
+def check_flag(name: str, value) -> None:
+    if not isinstance(value, (bool, np.bool_)):
+        raise ValueError(f"{name} must be True or False, got {value!r}")
+
+
+def nonzero_fractions(nnz: torch.Tensor, grpc):
+    """``(pct_group, pct_ref)``, ``[G, N]`` float64 tensors on the device of the count plane ``nnz`` ``[G, N]`` int32
+    (``illico_nonzero_fractions``: the one definition of the two fractions)."""
+    from . import _lib
+
+    G, N = int(nnz.shape[0]), int(nnz.shape[1])
+    dev = nnz.device
+    counts = np.asarray(grpc.counts, dtype=np.int64)
+    with torch.cuda.device(dev):
+        sizes = torch.from_numpy(counts.astype(np.int32)).to(dev)
+        pg = torch.empty((G, N), dtype=torch.float64, device=dev)
+        pr = torch.empty((G, N), dtype=torch.float64, device=dev)
+        st = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(_lib.load().illico_nonzero_fractions(nnz.data_ptr(), N, sizes.data_ptr(), G, N, int(grpc.encoded_ref_group),
+                                                        int(counts.sum()), pg.data_ptr(), pr.data_ptr(), st),
+                   "illico_nonzero_fractions")
+    return pg, pr
+
+
+def _host_fractions(run: _Run):
+    """The fractions of a run whose count plane came back to the host: computed on the run's first GPU and copied back."""
+    G, N = run.nnz.shape
+    with torch.cuda.device(run.device):
+        pg, pr = nonzero_fractions(torch.from_numpy(run.nnz).to(run.device, non_blocking=True), run.grpc)
+        out = []
+        for plane in (pg, pr):
+            host = torch.empty((G, N), dtype=torch.float64, pin_memory=True)
+            host.copy_(plane, non_blocking=True)
+            out.append(host)
+        torch.cuda.current_stream(run.device).synchronize()
+    return out[0].numpy(), out[1].numpy()
 
 
 def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, alternative, use_continuity, tie_correct,
-               layer, device, devices, score: bool, on_device: bool) -> _Run:
+               layer, device, devices, score: bool, on_device: bool, pts: bool = False) -> _Run:
     """Every (group, gene) test of ``adata``: validation, upload, group plan, one gene shard per GPU, batches, backed
     streaming.  ``on_device=False``: each shard's slabs are copied into pinned host arrays (``asymptotic_wilcoxon``).
     ``on_device=True``: they stay on the GPUs and meet in ``[G, N, 3]`` / ``[G, N]`` tensors on the first one
-    (device-to-device copies; with one shard its own tensors are the result)."""
+    (device-to-device copies; with one shard its own tensors are the result).  ``pts``: the count plane too."""
     X = adata.layers[layer] if layer is not None else adata.X
     if isinstance(X, (sparse.csr_array, sparse.csc_array)):
         X = sparse.csr_matrix(X) if isinstance(X, sparse.csr_array) else sparse.csc_matrix(X)
@@ -231,6 +278,7 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
                 flags = flags_for()
                 res = torch.empty((engine.n_groups, sh.ub - sh.lb, 3), dtype=torch.float64, device=sh.device)
                 sc = torch.empty((engine.n_groups, sh.ub - sh.lb), dtype=torch.float64, device=sh.device) if score else None
+                nz = torch.empty((engine.n_groups, sh.ub - sh.lb), dtype=torch.int32, device=sh.device) if pts else None
                 if data_handler.in_ram:
                     M.ready()
                     if fmt == CSR and not engine.check_csr_sorted(M):
@@ -242,17 +290,19 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
                         )
                     off = bounds[0] - sh.lb      # gene g of the run is column g + off of the device matrix
                     for lb, ub in _batches(sh.lb, sh.ub, batch_size, engine, True):
-                        engine.run_batch(M, lb + off, ub + off, flags, res, lb - sh.lb, scores=sc)
+                        engine.run_batch(M, lb + off, ub + off, flags, res, lb - sh.lb, scores=sc, nnz=nz)
                 else:
                     _run_backed(data_handler, _batches(sh.lb, sh.ub, batch_size, engine, False), engine, flags, res,
-                                max(1, int(n_threads)), gene0=sh.lb, scores=sc)
+                                max(1, int(n_threads)), gene0=sh.lb, scores=sc, nnz=nz)
                 if on_device and len(shards) == 1:
-                    shared["out"], shared["out_scores"] = res, sc
+                    shared["out"], shared["out_scores"], shared["out_nnz"] = res, sc, nz
                 else:
                     kind = "d2d" if on_device else "d2h"
                     hostio.d2h_slab(shared["out"], res, sh.lb, kind)
                     if sc is not None:
                         hostio.d2h_slab(shared["out_scores"], sc, sh.lb, kind)
+                    if nz is not None:
+                        hostio.d2h_slab(shared["out_nnz"], nz, sh.lb, kind)
                 torch.cuda.current_stream(sh.device).synchronize()
         except BaseException as e:  # re-raised on the calling thread
             sh.error = e
@@ -280,9 +330,11 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
         if not on_device:
             shared["out"] = torch.empty((G, n_genes, 3), dtype=torch.float64, pin_memory=True)
             shared["out_scores"] = torch.empty((G, n_genes), dtype=torch.float64, pin_memory=True) if score else None
+            shared["out_nnz"] = torch.empty((G, n_genes), dtype=torch.int32, pin_memory=True) if pts else None
         elif len(shards) > 1:
             shared["out"] = torch.empty((G, n_genes, 3), dtype=torch.float64, device=devs[0])
             shared["out_scores"] = torch.empty((G, n_genes), dtype=torch.float64, device=devs[0]) if score else None
+            shared["out_nnz"] = torch.empty((G, n_genes), dtype=torch.int32, device=devs[0]) if pts else None
     except BaseException:
         shared["error"] = True
         plan_ready.set()
@@ -298,10 +350,11 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
     for sh in shards:
         if sh.error is not None:
             raise sh.error
-    out, scores = shared["out"], shared["out_scores"]
+    out, scores, nnz = shared["out"], shared["out_scores"], shared.get("out_nnz")
     if not on_device:
         out, scores = out.numpy(), (scores.numpy() if scores is not None else None)
-    return _Run(unique_raw_groups, grpc, shards[0].device, out, scores)
+        nnz = nnz.numpy() if nnz is not None else None
+    return _Run(unique_raw_groups, grpc, shards[0].device, out, scores, nnz)
 
 
 def _bh_adjust(out: np.ndarray, device) -> np.ndarray:
@@ -369,7 +422,7 @@ class _PinnedSlot:
 
 
 def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, results, n_readers: int, gene0: int = 0,
-                scores=None) -> None:
+                scores=None, nnz=None) -> None:
     """Out-of-core input (BASELINE config 4): gene batches stream disk -> pinned ring -> HBM -> kernels.
 
     Reader threads slice the next batches from the backed container straight into pinned staging buffers (a ring of
@@ -455,7 +508,7 @@ def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, resu
             if data.dtype != torch.float32:
                 data, raw = _to_f32_or_wide(data)
             M = DeviceMatrix(fmt, tuple(shape), data, dv["indices"], dv["indptr"], raw=raw)
-        engine.run_batch(M, bounds[0], bounds[1], flags, results, lb - gene0, scores=scores)
+        engine.run_batch(M, bounds[0], bounds[1], flags, results, lb - gene0, scores=scores, nnz=nnz)
 
     try:
         while done < n_readers:

@@ -7,6 +7,8 @@
 //                              clipped at 1.
 //   illico_top_genes           ranks the genes of each group by score (stable radix sort of order-preserving keys carrying
 //                              the gene index) and gathers the first k genes' records: scanpy's rank_genes_groups order.
+//   illico_top_genes_filtered  the same ranking with scanpy's filter_rank_genes_groups criteria applied first (dropped genes
+//                              sort after every kept one) and the expressing-cell fractions in the record.
 //   illico_compute_pval_batch  evaluates the epilogue's compute_pval (epilogue.cuh; reference illico/utils/math.py:64-118)
 //                              on arrays of arguments, so the known-answer vectors of tests/golden/primitives.npz can be
 //                              checked against the device code itself.
@@ -78,12 +80,13 @@ __global__ void __launch_bounds__(BH_THREADS) bh_adjust_kernel(const double* __r
     }
 }
 
-// Per-group ranking (illico_top_genes): one CTA per group (grid-strided), like bh_adjust_kernel.  The key of gene j is the
-// order-preserving u64 image of its score, complemented so that an ascending sort puts the largest score first; NaN keys
-// are all-ones (after every number).  The gene indices ride along as the payload: they go in ascending, and the sort is
-// stable, so equal scores stay in index order.
+// Per-group ranking (illico_top_genes, illico_top_genes_filtered): one CTA per group (grid-strided), like bh_adjust_kernel.
+// The key of gene j is the order-preserving u64 image of its score, complemented so that an ascending sort puts the largest
+// score first.  NaN keys come after every number (~0 - 1: no number's key is above -inf's 0xFFF0...0) and the keys of
+// genes the filter drops after those (~0).  The gene indices ride along as the payload: they go in ascending, and the sort
+// is stable, so equal scores stay in index order.
 __device__ __forceinline__ unsigned long long score_key_desc(double x, int by_abs) {
-    if (x != x) return ~0ull;
+    if (x != x) return ~0ull - 1;
     if (by_abs) x = fabs(x);
     if (x == 0.0) x = 0.0;                                              // -0.0 sorts as +0.0
     const unsigned long long u = (unsigned long long)__double_as_longlong(x);
@@ -91,39 +94,75 @@ __device__ __forceinline__ unsigned long long score_key_desc(double x, int by_ab
     return ~asc;
 }
 
+// The marker filter and the optional fraction planes of illico_top_genes_filtered.  A NaN bound is a criterion not given;
+// illico_top_genes passes no planes, NaN bounds and rec_w = 5.
+struct TopFilter {
+    const double* pct_group;
+    const double* pct_ref;
+    double min_in, max_out, fc_lo, fc_hi;
+    int* kept;
+    int rec_w;
+};
+
 __global__ void __launch_bounds__(BH_THREADS) top_genes_kernel(const double* __restrict__ score, long long score_stride,
                                                                const double* __restrict__ res, long long res_stride,
                                                                const double* __restrict__ padj, int G, int N, int k, int by_abs,
-                                                               int* __restrict__ out_gene, double* __restrict__ out_rec,
+                                                               TopFilter F, int* __restrict__ out_gene, double* __restrict__ out_rec,
                                                                unsigned long long* __restrict__ slab) {
     __shared__ uint32_t hist[BH_NW * 256];
     __shared__ uint32_t aux[RADIX_AUX_WORDS];
+    __shared__ int n_kept;
     const int tid = threadIdx.x;
     unsigned long long* A = slab + (long long)blockIdx.x * 3 * N;
     unsigned long long* B = A + N;
     uint32_t* IA = reinterpret_cast<uint32_t*>(B + N);
     uint32_t* IB = IA + N;
+    const bool by_in = F.min_in == F.min_in, by_out = F.max_out == F.max_out, by_fc = F.fc_lo == F.fc_lo || F.fc_hi == F.fc_hi;
     for (int g = blockIdx.x; g < G; g += gridDim.x) {
         const double* sg = score + (long long)g * score_stride;
+        const double* rg = res + (long long)g * res_stride;
+        const long long plane = (long long)g * N;
+        if (tid == 0) n_kept = 0;
+        __syncthreads();
+        int mine = 0;
         for (int j = tid; j < N; j += BH_THREADS) {
-            A[j] = score_key_desc(sg[j], by_abs);
+            bool keep = true;                                           // a NaN fails every criterion it meets
+            if (by_in) keep = F.pct_group[plane + j] >= F.min_in;
+            if (by_out) keep = keep && F.pct_ref[plane + j] <= F.max_out;
+            if (by_fc) {
+                const double fc = rg[3 * (long long)j + 2];
+                keep = keep && (fc >= F.fc_lo || fc <= F.fc_hi);
+            }
+            A[j] = keep ? score_key_desc(sg[j], by_abs) : ~0ull;
             IA[j] = (uint32_t)j;
+            mine += keep;
         }
+        if (mine) atomicAdd(&n_kept, mine);
         __syncthreads();
         const unsigned long long* S = block_radix_sort_t<unsigned long long, uint32_t>(A, B, N, hist, aux, IA, IB);
         const uint32_t* idx = (S == A) ? IA : IB;
-        const double* rg = res + (long long)g * res_stride;
+        const int m = min(k, n_kept);
         for (int r = tid; r < k; r += BH_THREADS) {
-            const int j = (int)idx[r];
             const long long o = (long long)g * k + r;
+            double* rec = out_rec + o * F.rec_w;
+            if (r >= m) {                                               // fewer than k genes kept
+                out_gene[o] = -1;
+                for (int f = 0; f < F.rec_w; ++f) rec[f] = NAN;
+                continue;
+            }
+            const int j = (int)idx[r];
             out_gene[o] = j;
-            double* rec = out_rec + o * 5;
             rec[0] = sg[j];
             rec[1] = rg[3 * (long long)j];
             rec[2] = rg[3 * (long long)j + 1];
             rec[3] = rg[3 * (long long)j + 2];
-            rec[4] = padj ? padj[(long long)g * N + j] : NAN;
+            rec[4] = padj ? padj[plane + j] : NAN;
+            if (F.rec_w == 7) {
+                rec[5] = F.pct_group ? F.pct_group[plane + j] : NAN;
+                rec[6] = F.pct_ref ? F.pct_ref[plane + j] : NAN;
+            }
         }
+        if (tid == 0 && F.kept) F.kept[g] = n_kept;
         __syncthreads();
     }
 }
@@ -200,14 +239,15 @@ size_t illico_top_genes_workspace_bytes(int32_t n_groups, int32_t n_genes) {
     return (size_t)ctas * 3 * (size_t)(n_genes > 0 ? n_genes : 1) * sizeof(unsigned long long) + 256;
 }
 
-int illico_top_genes(const double* scores, int64_t score_group_stride, const double* results, int64_t result_group_stride,
-                     const double* p_adj, int32_t n_groups, int32_t n_genes, int32_t k, int32_t by_abs, int32_t* out_gene,
-                     double* out_rec, void* workspace, size_t workspace_bytes, void* stream) {
-    if (!scores || !results || !out_gene || !out_rec || !workspace) { set_error("illico_top_genes: NULL argument"); return 1; }
+static int launch_top_genes(const char* who, const double* scores, int64_t score_group_stride, const double* results,
+                            int64_t result_group_stride, const double* p_adj, int32_t n_groups, int32_t n_genes, int32_t k,
+                            int32_t by_abs, const TopFilter& F, int32_t* out_gene, double* out_rec, void* workspace,
+                            size_t workspace_bytes, void* stream) {
+    if (!scores || !results || !out_gene || !out_rec || !workspace) { set_error("%s: NULL argument", who); return 1; }
     if (n_groups <= 0 || n_genes <= 0) return 0;
-    if (k < 1 || k > n_genes) { set_error("illico_top_genes: k = %d outside [1, %d]", k, n_genes); return 1; }
+    if (k < 1 || k > n_genes) { set_error("%s: k = %d outside [1, %d]", who, k, n_genes); return 1; }
     if (workspace_bytes < illico_top_genes_workspace_bytes(n_groups, n_genes)) {
-        set_error("illico_top_genes: workspace too small");
+        set_error("%s: workspace too small", who);
         return 1;
     }
     const int ctas = n_groups < 148 * 2 ? n_groups : 148 * 2;
@@ -216,9 +256,31 @@ int illico_top_genes(const double* scores, int64_t score_group_stride, const dou
     cudaStream_t st = (cudaStream_t)stream;
     ILLICO_LAUNCH("top_genes_kernel", st,
                   top_genes_kernel<<<ctas, BH_THREADS, 0, st>>>(scores, score_group_stride, results, result_group_stride, p_adj,
-                                                                n_groups, n_genes, k, by_abs ? 1 : 0, out_gene, out_rec, slab));
+                                                                n_groups, n_genes, k, by_abs ? 1 : 0, F, out_gene, out_rec, slab));
     ILLICO_CUDA_OK(cudaGetLastError());
     return 0;
+}
+
+int illico_top_genes(const double* scores, int64_t score_group_stride, const double* results, int64_t result_group_stride,
+                     const double* p_adj, int32_t n_groups, int32_t n_genes, int32_t k, int32_t by_abs, int32_t* out_gene,
+                     double* out_rec, void* workspace, size_t workspace_bytes, void* stream) {
+    const TopFilter F{nullptr, nullptr, NAN, NAN, NAN, NAN, nullptr, 5};
+    return launch_top_genes("illico_top_genes", scores, score_group_stride, results, result_group_stride, p_adj, n_groups, n_genes,
+                            k, by_abs, F, out_gene, out_rec, workspace, workspace_bytes, stream);
+}
+
+int illico_top_genes_filtered(const double* scores, int64_t score_group_stride, const double* results, int64_t result_group_stride,
+                              const double* p_adj, const double* pct_group, const double* pct_ref, int32_t n_groups, int32_t n_genes,
+                              int32_t k, int32_t by_abs, double min_in_group, double max_out_group, double fc_min, double fc_max,
+                              int32_t* out_gene, double* out_rec, int32_t* kept, void* workspace, size_t workspace_bytes,
+                              void* stream) {
+    if ((min_in_group == min_in_group && !pct_group) || (max_out_group == max_out_group && !pct_ref)) {
+        set_error("illico_top_genes_filtered: a fraction bound is given without its plane");
+        return 1;
+    }
+    const TopFilter F{pct_group, pct_ref, min_in_group, max_out_group, fc_min, fc_max, kept, 7};
+    return launch_top_genes("illico_top_genes_filtered", scores, score_group_stride, results, result_group_stride, p_adj, n_groups,
+                            n_genes, k, by_abs, F, out_gene, out_rec, workspace, workspace_bytes, stream);
 }
 
 int illico_compute_pval_batch(const int64_t* n_ref, const int64_t* n_tgt, const int64_t* n, const double* tie_sum,

@@ -169,11 +169,14 @@ class Engine:
 
     # ---- one gene batch ----------------------------------------------------------------------------------
     def run_batch(self, M: DeviceMatrix, lb: int, ub: int, flags: _lib.Flags, results: torch.Tensor,
-                  result_gene0: int, debug: dict | None = None, scores: torch.Tensor | None = None) -> None:
+                  result_gene0: int, debug: dict | None = None, scores: torch.Tensor | None = None,
+                  nnz: torch.Tensor | None = None) -> None:
         """Enqueues stage + rank for genes ``[lb, ub)`` of ``M``; writes ``results[:, result_gene0 + k, :]``.
 
         ``results`` is a device tensor ``[G, N_total, 3]`` float64 (contiguous).  ``scores``, a device tensor ``[G, N_total]``
-        float64 (contiguous), also receives the signed score of every test at ``scores[:, result_gene0 + k]``.
+        float64 (contiguous), also receives the signed score of every test at ``scores[:, result_gene0 + k]``.  ``nnz``, a
+        device tensor ``[G, N_total]`` int32 (contiguous), receives at ``nnz[:, result_gene0 + k]`` how many cells of each
+        group have a non-zero value (``illico_count_nonzero_*``, enqueued before the tests on the same stream).
         """
         b = ub - lb
         if b <= 0:
@@ -184,6 +187,8 @@ class Engine:
             raise ValueError(f"Invalid chunk bounds: {(lb, ub)} for data with {M.shape[1]} columns.")
         with torch.cuda.device(self.device):
             M.ready()
+        if nnz is not None:
+            self.count_nonzero(M, lb, ub, nnz, result_gene0)
         if M.raw is not None:
             return self._run_batch_wide(M, lb, ub, flags, results, result_gene0, debug, scores)
         t = self._ensure_buffers(b)
@@ -218,6 +223,24 @@ class Engine:
                 rc = fn(M.data.data_ptr(), M.indices.data_ptr(), M.indptr.data_ptr(), lb, b, C.byref(self.plan),
                         C.byref(flags), C.byref(buf), out_ptr, gstride, dbg_ref, st)
         _lib.check(rc, f"illico_{test}_{M.fmt}_f32")
+
+    def count_nonzero(self, M: DeviceMatrix, lb: int, ub: int, nnz: torch.Tensor, result_gene0: int) -> None:
+        """``nnz[:, result_gene0 + k]`` = cells of each group whose value in gene ``lb + k`` of ``M`` is non-zero, on the
+        current stream.  A matrix kept as float64 (``M.raw``) is counted on those values, not on its recoded batches."""
+        G, Ntot = nnz.shape
+        assert nnz.dtype == torch.int32 and nnz.is_contiguous() and G == self.n_groups and nnz.device == self.device
+        vals, dtype = (M.raw, _lib.DTYPE_F64) if M.raw is not None else (M.data, _lib.DTYPE_F32)
+        out = nnz.data_ptr() + result_gene0 * 4
+        with torch.cuda.device(self.device):
+            st = torch.cuda.current_stream(self.device).cuda_stream
+            if M.fmt == DENSE:
+                rc = self.lib.illico_count_nonzero_dense(vals.data_ptr(), dtype, int(vals.stride(0)), lb, ub - lb,
+                                                         C.byref(self.plan), out, Ntot, st)
+            else:
+                fn = getattr(self.lib, f"illico_count_nonzero_{M.fmt}")
+                rc = fn(vals.data_ptr(), dtype, M.indices.data_ptr(), M.indptr.data_ptr(), lb, ub - lb, C.byref(self.plan), out,
+                        Ntot, st)
+        _lib.check(rc, f"illico_count_nonzero_{M.fmt}")
 
     def _run_batch_wide(self, M: DeviceMatrix, lb: int, ub: int, flags: _lib.Flags, results, result_gene0, debug, scores=None):
         """float64 input (values float32 cannot hold): every sub-batch is recoded on the device to order-preserving

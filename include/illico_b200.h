@@ -311,6 +311,45 @@ int illico_top_genes(const double* scores, int64_t score_group_stride, const dou
                      const double* p_adj, int32_t n_groups, int32_t n_genes, int32_t k, int32_t by_abs, int32_t* out_gene,
                      double* out_rec, void* workspace, size_t workspace_bytes, void* stream);
 
+/* illico_top_genes with scanpy's marker filter (filter_rank_genes_groups) applied before the selection.  A gene is kept
+ * when every GIVEN criterion holds: pct_group >= min_in_group, pct_ref <= max_out_group, fold_change >= fc_min or
+ * fold_change <= fc_max (pass NaN for a criterion that is not given; fc_max is the host's 1 / fc_min for a by-|fold change|
+ * filter, NaN otherwise).  A NaN meeting a given criterion fails it.  Kept genes come first in illico_top_genes' order,
+ * dropped genes after all of them; the first min(k, kept[g]) are written, the rest of the row gets gene -1 and an all-NaN
+ * record.  Records are [n_groups, k, 7] = (score, p_value, statistic, fold_change, p_adj, pct_group, pct_ref), each NaN where
+ * its plane is NULL; pct_group / pct_ref are [n_groups, n_genes] like p_adj (illico_nonzero_fractions) and must be given
+ * with their bound.  kept [n_groups] (NULL: not written) = genes of the group that pass.  The BH p_adj is the caller's:
+ * over all genes, as scanpy adjusts before it filters.  Workspace: illico_top_genes_workspace_bytes. */
+int illico_top_genes_filtered(const double* scores, int64_t score_group_stride, const double* results, int64_t result_group_stride,
+                              const double* p_adj, const double* pct_group, const double* pct_ref, int32_t n_groups, int32_t n_genes,
+                              int32_t k, int32_t by_abs, double min_in_group, double max_out_group, double fc_min, double fc_max,
+                              int32_t* out_gene, double* out_rec, int32_t* kept, void* workspace, size_t workspace_bytes,
+                              void* stream);
+
+/* ---- cells that express a gene (scanpy rank_genes_groups(pts=True): pct_nz_group / pct_nz_reference) -------------------
+ * counts[g * count_group_stride + j] (int32) = cells of group g whose value in gene gene_lb + j satisfies x != 0: -0.0 and
+ * explicitly stored zeros do not count, NaN does.  Every element of the batch's [n_groups, n_genes_batch] plane is written
+ * (the caller zeroes nothing).  `dtype` is ILLICO_DTYPE_F32 or ILLICO_DTYPE_F64 (a recoded batch is counted on its original
+ * float64 values, not on the codes); any other dtype is an error.  The inputs are those of the staging calls: dense rows of
+ * any `ld` (no alignment needed), CSR rows with sorted indices, CSC columns gene_lb.. .  Rows are walked through the plan
+ * (perm / segments; CSC: group of a row = seg_group[cell_seg[row]]).  A read-only pass of its own over the batch, run only
+ * when asked for (csrc/counts.cu). */
+int illico_count_nonzero_dense(const void* X, int32_t dtype, int64_t ld, int32_t gene_lb, int32_t n_genes_batch,
+                               const illico_plan_t* plan, int32_t* counts, int64_t count_group_stride, void* stream);
+int illico_count_nonzero_csr(const void* data, int32_t dtype, const int32_t* indices, const int64_t* indptr, int32_t gene_lb,
+                             int32_t n_genes_batch, const illico_plan_t* plan, int32_t* counts, int64_t count_group_stride,
+                             void* stream);
+int illico_count_nonzero_csc(const void* data, int32_t dtype, const int32_t* indices, const int64_t* indptr, int32_t gene_lb,
+                             int32_t n_genes_batch, const illico_plan_t* plan, int32_t* counts, int64_t count_group_stride,
+                             void* stream);
+/* The gathered count plane counts [n_groups, >= n_genes] -> pct_group / pct_ref [n_groups, n_genes] float64, one IEEE
+ * division each:  pct_group[g, j] = count[g, j] / n_g;  one-versus-reference (ref_group >= 0): pct_ref[g, j] =
+ * count[ref, j] / n_ref on every row, the reference's own included;  one-versus-rest (ref_group < 0): pct_ref[g, j] =
+ * (total_j - count[g, j]) / (n_cells - n_g), total_j the exact sum over the groups (0 / 0 = NaN with a single group).
+ * group_size: device [n_groups]; n_cells = their sum. */
+int illico_nonzero_fractions(const int32_t* counts, int64_t count_group_stride, const int32_t* group_size, int32_t n_groups,
+                             int32_t n_genes, int32_t ref_group, int64_t n_cells, double* pct_group, double* pct_ref, void* stream);
+
 /* The device epilogue's compute_pval (illico/utils/math.py:64-118) on arrays of arguments (device pointers): lets the
  * known-answer vectors of the reference's primitive be checked against the GPU code itself. */
 int illico_compute_pval_batch(const int64_t* n_ref, const int64_t* n_tgt, const int64_t* n, const double* tie_sum,
