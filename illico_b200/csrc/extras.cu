@@ -24,23 +24,34 @@ constexpr int BH_THREADS = 512;
 constexpr int BH_NW = BH_THREADS / 32;
 
 // One CTA per group (grid-strided).  keys: the group's p-values as u64 (non-negative doubles order like their bits).
+// A group with a NaN p-value (one-versus-rest with a single group: sigma = 0) gets NaN for every gene, as in statsmodels,
+// where the NaN sorts last and the reverse running minimum carries it to every rank.
 __global__ void __launch_bounds__(BH_THREADS) bh_adjust_kernel(const double* __restrict__ p, long long group_stride,
                                                                long long gene_stride, int G, int N, double* __restrict__ padj,
                                                                unsigned long long* __restrict__ slab) {
     __shared__ uint32_t hist[BH_NW * 256];
     __shared__ uint32_t aux[RADIX_AUX_WORDS];
     __shared__ double wmin[BH_NW];
+    __shared__ int has_nan;
     const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
     unsigned long long* A = slab + (long long)blockIdx.x * 2 * N;
     unsigned long long* B = A + N;
     for (int g = blockIdx.x; g < G; g += gridDim.x) {
         const double* pg = p + (long long)g * group_stride;
+        if (tid == 0) has_nan = 0;
+        __syncthreads();
         for (int j = tid; j < N; j += BH_THREADS) {
             double v = pg[(long long)j * gene_stride];
-            if (!(v >= 0.0)) v = 0.0;                                   // (-0.0 / NaN never come out of compute_pval)
+            if (v != v) has_nan = 1;
+            if (!(v >= 0.0)) v = 0.0;                                   // (negative p-values never come out of compute_pval)
             A[j] = (unsigned long long)__double_as_longlong(v);
         }
         __syncthreads();
+        if (has_nan) {
+            for (int j = tid; j < N; j += BH_THREADS) padj[(long long)g * N + j] = NAN;
+            __syncthreads();                                             // (every thread has read has_nan before it is reset)
+            continue;
+        }
         unsigned long long* S = block_radix_sort_t<unsigned long long>(A, B, N, hist, aux);
         double* M = reinterpret_cast<double*>(S == A ? B : A);          // suffix minima of p_(k) / (k / N)
         // reverse running minimum: thread t owns the contiguous ranks [lo, hi) counted from the END of the order
@@ -70,7 +81,7 @@ __global__ void __launch_bounds__(BH_THREADS) bh_adjust_kernel(const double* __r
         // every gene takes the value at the rank of the LAST element tied with it
         for (int j = tid; j < N; j += BH_THREADS) {
             double v = pg[(long long)j * gene_stride];
-            if (!(v >= 0.0)) v = 0.0;
+            if (!(v >= 0.0)) v = 0.0;                                   // (the group holds no NaN: see has_nan)
             const unsigned long long key = (unsigned long long)__double_as_longlong(v);
             int a = 0, b = N;
             while (a < b) { const int mid = (a + b) >> 1; if (S[mid] <= key) a = mid + 1; else b = mid; }

@@ -649,8 +649,9 @@ __global__ void __launch_bounds__(T_THREADS, 8) ovr_table_kernel(const OvrParams
             if (SCORE)
                 P.flags.scores[(long long)g * P.flags.score_group_stride + jo] = compute_score(n_r, n_t, n, P.flags.tie_correct ? tie : 0.0, U, mu);
             const double mu_t = sum * (1.0 / (double)n_t);   // (the fused epilogue's form: every path gives the same bits)
-            // exactly zero when the group holds every non-zero of the gene (see fused_epilogue_kernel)
-            const double mu_r = (nnz_g == nnz) ? 0.0 : (total - sum) / (double)(n - n_t);
+            // exactly zero when the group holds every non-zero of the gene (see fused_epilogue_kernel); 0 / 0 = NaN, as in
+            // ovr_kernel and the oracle, when it holds every cell (a single group: there is no rest)
+            const double mu_r = (n_t == n) ? NAN : (nnz_g == nnz) ? 0.0 : (total - sum) / (double)(n - n_t);
             double* o = P.results + (long long)g * P.gstride + (long long)jo * 3;
             o[0] = p; o[1] = U; o[2] = (mu_r == 0.0) ? INFINITY : mu_t / mu_r;
             if (P.dbg_u2) P.dbg_u2[(long long)g * P.n_cols + jo] = u2;

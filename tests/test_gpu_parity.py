@@ -848,7 +848,7 @@ def test_optional_columns_p_adj_and_log2fc():
         adj = np.minimum.accumulate(raw[::-1])[::-1]
         adj[adj > 1] = 1
         want[g, order] = adj
-    np.testing.assert_allclose(df["p_adj"].to_numpy().reshape(G, N), want, rtol=1e-15, atol=0)
+    np.testing.assert_array_equal(df["p_adj"].to_numpy().reshape(G, N), want)
     with np.errstate(divide="ignore", invalid="ignore"):
         np.testing.assert_array_equal(df["log2_fold_change"].to_numpy(), np.log2(df["fold_change"].to_numpy()))
 

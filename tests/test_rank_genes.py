@@ -268,7 +268,7 @@ def check_ranking(df, X, labels, reference, n_genes, by_abs=False, **kw):
     assert list(df.index.get_level_values("pert")) == list(np.repeat(np.asarray(groups)[kept], k))
     assert list(df.index.get_level_values("rank")) == list(np.tile(np.arange(k), len(kept)))
     padj = bh_reference(out[:, :, 0])
-    np.testing.assert_allclose(extra["p_adj"], padj, rtol=1e-15, atol=0)
+    np.testing.assert_array_equal(extra["p_adj"], padj)
     got = df.to_numpy()
     for i, g in enumerate(kept):
         sel = rank_order(extra["score"][g], by_abs)[:k]
