@@ -103,6 +103,11 @@ SIGNATURES = {
     "illico_count_nonzero_csr": (C.c_int, [_vp, _i32, _vp, _vp, _i32, _i32, _PP, _vp, _i64, _vp]),
     "illico_count_nonzero_csc": (C.c_int, [_vp, _i32, _vp, _vp, _i32, _i32, _PP, _vp, _i64, _vp]),
     "illico_nonzero_fractions": (C.c_int, [_vp, _i64, _vp, _i32, _i32, _i32, _i64, _vp, _vp, _vp]),
+    "illico_group_moments_dense": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _PP, _i32, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
+    "illico_group_moments_csr": (C.c_int, [_vp, _i32, _vp, _vp, _i32, _i32, _PP, _i32, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
+    "illico_group_moments_csc": (C.c_int, [_vp, _i32, _vp, _vp, _i32, _i32, _PP, _i32, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
+    "illico_welch_ttest": (C.c_int, [_vp, _vp, _vp, _i64, _vp, _i32, _i32, _i32, _i64, _i32, _i32, _vp, _i64, _vp, _i64, _vp]),
+    "illico_student_t_batch": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _vp]),
     "illico_compute_pval_batch": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
 }
 

@@ -24,22 +24,22 @@ import torch
 from scipy import sparse
 
 from . import hostio
-from .engine import CSR, DeviceMatrix, Engine, make_flags, require_cuda
+from .engine import CSR, WILCOXON, DeviceMatrix, Engine, check_method, make_flags, require_cuda
 from .groups import encode_and_count_groups, seg_max_from_env
 from .registry import DataHandler, data_handler_registry
 
 __all__ = ["asymptotic_wilcoxon"]
 
 
-def _batches(lb: int, ub: int, batch_size, engine: Engine, in_ram: bool):
+def _batches(lb: int, ub: int, batch_size, engine: Engine, in_ram: bool, method: str = WILCOXON):
     """Gene batches of the shard ``[lb, ub)`` (global gene indices)."""
     n_genes = ub - lb
     if isinstance(batch_size, (int, np.integer)) and not isinstance(batch_size, bool):
         if batch_size <= 0:
             raise ValueError(f"Invalid batch_size value: {batch_size}. Must be 'auto' or an integer.")
-        step = min(int(batch_size), engine.max_batch_genes(n_genes))
+        step = min(int(batch_size), engine.max_batch_genes(n_genes, method))
     elif batch_size == "auto":
-        step = engine.max_batch_genes(n_genes)
+        step = engine.max_batch_genes(n_genes, method)
         if not in_ram:
             step = min(step, 256)  # backed data: stream ~256 genes at a time like the reference aims for
     else:
@@ -211,11 +211,13 @@ def _host_fractions(run: _Run):
 
 
 def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, alternative, use_continuity, tie_correct,
-               layer, device, devices, score: bool, on_device: bool, pts: bool = False) -> _Run:
+               layer, device, devices, score: bool, on_device: bool, pts: bool = False, method: str = WILCOXON) -> _Run:
     """Every (group, gene) test of ``adata``: validation, upload, group plan, one gene shard per GPU, batches, backed
     streaming.  ``on_device=False``: each shard's slabs are copied into pinned host arrays (``asymptotic_wilcoxon``).
     ``on_device=True``: they stay on the GPUs and meet in ``[G, N, 3]`` / ``[G, N]`` tensors on the first one
-    (device-to-device copies; with one shard its own tensors are the result).  ``pts``: the count plane too."""
+    (device-to-device copies; with one shard its own tensors are the result).  ``pts``: the count plane too.  ``method``:
+    the Wilcoxon test or one of the t-tests (``Engine.run_batch``)."""
+    check_method(method)
     X = adata.layers[layer] if layer is not None else adata.X
     if isinstance(X, (sparse.csr_array, sparse.csc_array)):
         X = sparse.csr_matrix(X) if isinstance(X, sparse.csr_array) else sparse.csc_matrix(X)
@@ -289,11 +291,11 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
                             "prior to computing DE genes."
                         )
                     off = bounds[0] - sh.lb      # gene g of the run is column g + off of the device matrix
-                    for lb, ub in _batches(sh.lb, sh.ub, batch_size, engine, True):
-                        engine.run_batch(M, lb + off, ub + off, flags, res, lb - sh.lb, scores=sc, nnz=nz)
+                    for lb, ub in _batches(sh.lb, sh.ub, batch_size, engine, True, method):
+                        engine.run_batch(M, lb + off, ub + off, flags, res, lb - sh.lb, scores=sc, nnz=nz, method=method)
                 else:
-                    _run_backed(data_handler, _batches(sh.lb, sh.ub, batch_size, engine, False), engine, flags, res,
-                                max(1, int(n_threads)), gene0=sh.lb, scores=sc, nnz=nz)
+                    _run_backed(data_handler, _batches(sh.lb, sh.ub, batch_size, engine, False, method), engine, flags, res,
+                                max(1, int(n_threads)), gene0=sh.lb, scores=sc, nnz=nz, method=method)
                 if on_device and len(shards) == 1:
                     shared["out"], shared["out_scores"], shared["out_nnz"] = res, sc, nz
                 else:
@@ -422,7 +424,7 @@ class _PinnedSlot:
 
 
 def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, results, n_readers: int, gene0: int = 0,
-                scores=None, nnz=None) -> None:
+                scores=None, nnz=None, method: str = WILCOXON) -> None:
     """Out-of-core input (BASELINE config 4): gene batches stream disk -> pinned ring -> HBM -> kernels.
 
     Reader threads slice the next batches from the backed container straight into pinned staging buffers (a ring of
@@ -508,7 +510,7 @@ def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, resu
             if data.dtype != torch.float32:
                 data, raw = _to_f32_or_wide(data)
             M = DeviceMatrix(fmt, tuple(shape), data, dv["indices"], dv["indptr"], raw=raw)
-        engine.run_batch(M, bounds[0], bounds[1], flags, results, lb - gene0, scores=scores, nnz=nnz)
+        engine.run_batch(M, bounds[0], bounds[1], flags, results, lb - gene0, scores=scores, nnz=nnz, method=method)
 
     try:
         while done < n_readers:

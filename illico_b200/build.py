@@ -8,7 +8,7 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libillico_b200.so")
-SOURCES = ["api.cu", "stage.cu", "stage_dense_tma.cu", "fused.cu", "rank_ovr.cu", "rank_ovo.cu", "extras.cu", "counts.cu", "repart.cu", "recode.cu", "hostpack.c"]
+SOURCES = ["api.cu", "stage.cu", "stage_dense_tma.cu", "fused.cu", "rank_ovr.cu", "rank_ovo.cu", "extras.cu", "counts.cu", "ttest.cu", "repart.cu", "recode.cu", "hostpack.c"]
 HEADERS = ["common.cuh", "sort.cuh", "epilogue.cuh", "tma.cuh", os.path.join("..", "..", "include", "illico_b200.h")]
 
 NVCC_FLAGS = [

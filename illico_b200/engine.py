@@ -18,6 +18,14 @@ from . import _lib
 from .groups import GroupContainer, HostPlan, build_plan, check_seg_max
 
 DENSE, CSC, CSR = "dense", "csc", "csr"
+WILCOXON = "wilcoxon"
+METHODS = (WILCOXON, "t-test", "t-test_overestim_var")   # scanpy rank_genes_groups' names
+
+
+def check_method(method) -> str:
+    if not isinstance(method, str) or method not in METHODS:
+        raise ValueError(f"method must be one of {', '.join(repr(m) for m in METHODS)}, got {method!r}")
+    return method
 
 
 def _env_int(name: str, default: int) -> int:
@@ -113,11 +121,16 @@ class Engine:
     def is_ovo(self) -> bool:
         return self.host_plan.ref_group >= 0
 
-    def max_batch_genes(self, n_genes: int) -> int:
-        """Genes per device batch so that the staged lists stay within the memory budget."""
+    def max_batch_genes(self, n_genes: int, method: str = WILCOXON) -> int:
+        """Genes per device batch so that the staged lists (Wilcoxon) or the three float64 moment planes (t-test) stay
+        within the memory budget."""
         free, _total = torch.cuda.mem_get_info(self.device)
-        budget = min(_env_int("ILLICO_B200_IR_BYTES", 16 << 30), int(free * 0.35))
-        per_gene = self.host_plan.slot_cap * 4 + self.host_plan.n_segments * 4
+        if method == WILCOXON:
+            budget = min(_env_int("ILLICO_B200_IR_BYTES", 16 << 30), int(free * 0.35))
+            per_gene = self.host_plan.slot_cap * 4 + self.host_plan.n_segments * 4
+        else:
+            budget = int(free * 0.35)
+            per_gene = self.host_plan.n_groups * 3 * 8
         b = max(1, budget // max(per_gene, 1))
         b = int(min(n_genes, b, _env_int("ILLICO_B200_BATCH_GENES", 1 << 30)))
         return b if b < 8 or b == n_genes else (b // 4) * 4  # multiples of 4 keep the 128-bit staging path
@@ -170,13 +183,14 @@ class Engine:
     # ---- one gene batch ----------------------------------------------------------------------------------
     def run_batch(self, M: DeviceMatrix, lb: int, ub: int, flags: _lib.Flags, results: torch.Tensor,
                   result_gene0: int, debug: dict | None = None, scores: torch.Tensor | None = None,
-                  nnz: torch.Tensor | None = None) -> None:
+                  nnz: torch.Tensor | None = None, method: str = WILCOXON) -> None:
         """Enqueues stage + rank for genes ``[lb, ub)`` of ``M``; writes ``results[:, result_gene0 + k, :]``.
 
         ``results`` is a device tensor ``[G, N_total, 3]`` float64 (contiguous).  ``scores``, a device tensor ``[G, N_total]``
         float64 (contiguous), also receives the signed score of every test at ``scores[:, result_gene0 + k]``.  ``nnz``, a
         device tensor ``[G, N_total]`` int32 (contiguous), receives at ``nnz[:, result_gene0 + k]`` how many cells of each
         group have a non-zero value (``illico_count_nonzero_*``, enqueued before the tests on the same stream).
+        ``method`` "t-test" / "t-test_overestim_var": Welch's t-test instead (``_run_batch_ttest``), same outputs.
         """
         b = ub - lb
         if b <= 0:
@@ -187,6 +201,8 @@ class Engine:
             raise ValueError(f"Invalid chunk bounds: {(lb, ub)} for data with {M.shape[1]} columns.")
         with torch.cuda.device(self.device):
             M.ready()
+        if method != WILCOXON:
+            return self._run_batch_ttest(M, lb, ub, flags, results, result_gene0, scores, nnz, check_method(method))
         if nnz is not None:
             self.count_nonzero(M, lb, ub, nnz, result_gene0)
         if M.raw is not None:
@@ -241,6 +257,50 @@ class Engine:
                 rc = fn(vals.data_ptr(), dtype, M.indices.data_ptr(), M.indptr.data_ptr(), lb, ub - lb, C.byref(self.plan), out,
                         Ntot, st)
         _lib.check(rc, f"illico_count_nonzero_{M.fmt}")
+
+    def _run_batch_ttest(self, M: DeviceMatrix, lb: int, ub: int, flags: _lib.Flags, results, result_gene0, scores, nnz, method):
+        """Welch's t-test of genes ``[lb, ub)``: one pass over the batch for the per-(group, gene) moments (and the count
+        plane when ``nnz`` is given) -- ``illico_group_moments_*`` -- then ``illico_welch_ttest`` into the same result and
+        score slabs.  float64 values (``M.raw``) are read as they are: no recoding, no staged lists."""
+        b = ub - lb
+        G, Ntot = results.shape[0], results.shape[1]
+        assert results.dtype == torch.float64 and results.is_contiguous() and G == self.n_groups
+        dev = self.device
+        log1p = int(bool(flags.is_log1p))
+        t = self._tls
+        if getattr(t, "mom_genes", 0) < b:
+            t.mom = None
+            with torch.cuda.device(dev):
+                t.mom = torch.empty((3, G, b), dtype=torch.float64, device=dev)
+            t.mom_genes = b
+        mom = t.mom
+        stream = torch.cuda.current_stream(dev)
+        mom.record_stream(stream)
+        ms = mom.shape[2]
+        s1, s2, sf = (mom[k].data_ptr() for k in range(3))
+        vals, dtype = (M.raw, _lib.DTYPE_F64) if M.raw is not None else (M.data, _lib.DTYPE_F32)
+        cnt, cstride = (None, 0)
+        if nnz is not None:
+            assert nnz.dtype == torch.int32 and nnz.is_contiguous() and tuple(nnz.shape) == (G, Ntot)
+            cnt, cstride = nnz.data_ptr() + result_gene0 * 4, Ntot
+        if scores is not None:
+            assert scores.dtype == torch.float64 and scores.is_contiguous() and tuple(scores.shape) == (G, Ntot)
+        hp = self.host_plan
+        with torch.cuda.device(dev):
+            st = stream.cuda_stream
+            if M.fmt == DENSE:
+                rc = self.lib.illico_group_moments_dense(vals.data_ptr(), dtype, int(vals.stride(0)), lb, b, C.byref(self.plan), log1p,
+                                                         s1, s2, sf, cnt, cstride, ms, st)
+            else:
+                fn = getattr(self.lib, f"illico_group_moments_{M.fmt}")
+                rc = fn(vals.data_ptr(), dtype, M.indices.data_ptr(), M.indptr.data_ptr(), lb, b, C.byref(self.plan), log1p, s1, s2,
+                        sf, cnt, cstride, ms, st)
+            _lib.check(rc, f"illico_group_moments_{M.fmt}")
+            rc = self.lib.illico_welch_ttest(s1, s2, sf if log1p else None, ms, self._tables["group_size"].data_ptr(), G, b,
+                                             hp.ref_group, hp.n_cells, int(method == "t-test_overestim_var"), flags.alternative,
+                                             results.data_ptr() + result_gene0 * 3 * 8, Ntot * 3,
+                                             scores.data_ptr() + result_gene0 * 8 if scores is not None else None, Ntot, st)
+            _lib.check(rc, "illico_welch_ttest")
 
     def _run_batch_wide(self, M: DeviceMatrix, lb: int, ub: int, flags: _lib.Flags, results, result_gene0, debug, scores=None):
         """float64 input (values float32 cannot hold): every sub-batch is recoded on the device to order-preserving

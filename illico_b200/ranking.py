@@ -19,6 +19,7 @@ import torch
 
 from . import _lib
 from .asymptotic_wilcoxon import _run_tests, check_flag, nonzero_fractions
+from .engine import check_method
 
 __all__ = ["rank_genes"]
 
@@ -55,8 +56,9 @@ def rank_genes(
     min_in_group_fraction: float | None = None,
     max_out_group_fraction: float | None = None,
     min_fold_change: float | None = None,
+    method: str = "wilcoxon",
 ) -> pd.DataFrame:
-    """The ``n_genes`` strongest genes of every group, by Wilcoxon score.
+    """The ``n_genes`` strongest genes of every group, by Wilcoxon score (or Welch's t with ``method="t-test"``).
 
     The tests are those of ``asymptotic_wilcoxon`` (same arguments, same checks and errors).  Each group's genes are
     sorted by ``score`` descending -- the signed z of the normal approximation, ``(n_r n_t / 2 - U) / sigma``, positive
@@ -77,7 +79,12 @@ def rank_genes(
     only when given, a NaN failing it (scanpy's ``filter_rank_genes_groups`` defaults are 0.25, 0.5 and 1).  The filter
     runs before the selection: a group has ``min(n_genes, genes kept)`` rows (none when nothing is kept) and ``p_adj``
     stays over all of its genes.  A filter implies ``pts``.
+
+    ``method`` is scanpy's: ``"wilcoxon"`` (the default), ``"t-test"`` or ``"t-test_overestim_var"`` (Welch's t-test, as
+    ``illico_b200.ttest``).  For a t-test ``score`` and ``statistic`` are t (``score`` with NaN replaced by 0, the p-value
+    NaN replaced by 1), the fold change is the Wilcoxon call's, and ``use_continuity`` / ``tie_correct`` are ignored.
     """
+    check_method(method)
     if n_genes is not None:
         if isinstance(n_genes, bool) or not isinstance(n_genes, (int, np.integer)):
             raise ValueError(f"n_genes must be a positive integer or None, got {n_genes!r}")
@@ -89,7 +96,7 @@ def rank_genes(
     fc_min = _bound("min_fold_change", min_fold_change, None)
     with_pts = bool(pts) or any(v is not None for v in (min_in, max_out, fc_min))
     run = _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, alternative, use_continuity,
-                     tie_correct, layer, device, devices, score=True, on_device=True, pts=with_pts)
+                     tie_correct, layer, device, devices, score=True, on_device=True, pts=with_pts, method=method)
     res, scores = run.results, run.scores
     G, N = int(res.shape[0]), int(res.shape[1])
     k = N if n_genes is None else min(int(n_genes), N)

@@ -350,6 +350,47 @@ int illico_count_nonzero_csc(const void* data, int32_t dtype, const int32_t* ind
 int illico_nonzero_fractions(const int32_t* counts, int64_t count_group_stride, const int32_t* group_size, int32_t n_groups,
                              int32_t n_genes, int32_t ref_group, int64_t n_cells, double* pct_group, double* pct_ref, void* stream);
 
+/* ---- Welch's t-test (scanpy rank_genes_groups(method="t-test" | "t-test_overestim_var")) -----------------------------------
+ * illico_group_moments_*: the count kernels' walks with float64 accumulators.  For group g and gene gene_lb + j:
+ * sums[g * group_stride + j] = sum of x, sumsq[..] = sum of x * x (x widened to float64 first, then squared), and with
+ * is_log1p fsums[..] = sum of expm1(x) (the fold change's values; fsums is not touched otherwise and may be NULL).  counts
+ * (may be NULL) receives illico_count_nonzero_*'s plane in the same launch, counts[g * count_group_stride + j].  Every element of the
+ * [n_groups, n_genes_batch] planes is written.  A group with one plan segment stores its sums; one with several adds its
+ * segments' sums (exact for integer data, any order).  dtype ILLICO_DTYPE_F32 or ILLICO_DTYPE_F64: float64 input is read as
+ * it is, no recoding.  Inputs as for illico_count_nonzero_* (csrc/counts.cu). */
+int illico_group_moments_dense(const void* X, int32_t dtype, int64_t ld, int32_t gene_lb, int32_t n_genes_batch,
+                               const illico_plan_t* plan, int32_t is_log1p, double* sums, double* sumsq, double* fsums,
+                               int32_t* counts, int64_t count_group_stride, int64_t group_stride, void* stream);
+int illico_group_moments_csr(const void* data, int32_t dtype, const int32_t* indices, const int64_t* indptr, int32_t gene_lb,
+                             int32_t n_genes_batch, const illico_plan_t* plan, int32_t is_log1p, double* sums, double* sumsq,
+                             double* fsums, int32_t* counts, int64_t count_group_stride, int64_t group_stride,
+                             void* stream);
+int illico_group_moments_csc(const void* data, int32_t dtype, const int32_t* indices, const int64_t* indptr, int32_t gene_lb,
+                             int32_t n_genes_batch, const illico_plan_t* plan, int32_t is_log1p, double* sums, double* sumsq,
+                             double* fsums, int32_t* counts, int64_t count_group_stride, int64_t group_stride,
+                             void* stream);
+/* The moment planes of a batch of n_genes genes -> results[g * result_group_stride + 3 j ..] = (p, t, fold_change) and, when
+ * scores is not NULL, scores[g * score_group_stride + j] = t with NaN -> 0.  One thread per gene (csrc/ttest.cu):
+ *   mean = S1 / n;  var = S2 / n - mean * mean;  if n != 1: var *= n / (n - 1)        (scanpy 1.10 _get_mean_var, dense)
+ *   comparison sample: group ref_group (>= 0), or all other cells (< 0: the gene's sums over the groups in a fixed order,
+ *   minus the group's; n_cells - n_g cells)
+ *   vn = sqrt(var)**2 / n;  df = (vn1 + vn2)**2 / (vn1**2 / (n1 - 1) + vn2**2 / (n2 - 1)), NaN -> 1;
+ *   t = (mean1 - mean2) / sqrt(vn1 + vn2)                   (scipy 1.18 _unequal_var_ttest_denom, _ttest_ind_from_stats)
+ *   p = 2 stdtr(df, -|t|) | stdtr(df, -t) (greater) | stdtr(df, t) (less), NaN -> 1          (scipy _get_pvalue; scanpy)
+ * with n2 = the group's own size for overestim_var != 0 ("t-test_overestim_var"; the comparison variance still comes from
+ * its own cells).  The fold change is the Wilcoxon kernels' expression on fsums (sums when fsums is NULL): OVO
+ * (sum_g * (1 / n_g)) * (1 / (sum_r / n_r)), OVR (sum_g * (1 / n_g)) / ((total - sum_g) / (n_cells - n_g)), inf where the
+ * comparison mean is 0.  The reference group's row is (1, 0, fold change of the control with itself), score 0.
+ * group_size: device [n_groups].  Two launches: t, df and the fold change (CTA = 32 genes x 16 group lanes), then p. */
+int illico_welch_ttest(const double* sums, const double* sumsq, const double* fsums, int64_t group_stride, const int32_t* group_size,
+                       int32_t n_groups, int32_t n_genes, int32_t ref_group, int64_t n_cells, int32_t overestim_var,
+                       int32_t alternative, double* results, int64_t result_group_stride, double* scores, int64_t score_group_stride,
+                       void* stream);
+/* The t-test's p-value on arrays (device pointers): out[i] = 2 stdtr(df[i], -|t[i]|) (ILLICO_TWO_SIDED), stdtr(df[i], -t[i])
+ * (ILLICO_GREATER) or stdtr(df[i], t[i]) (ILLICO_LESS), stdtr the Student t CDF (scipy.special.stdtr), without the NaN -> 1
+ * replacement: the known-answer hook of the device code. */
+int illico_student_t_batch(const double* df, const double* t, int64_t n, int32_t alternative, double* out, void* stream);
+
 /* The device epilogue's compute_pval (illico/utils/math.py:64-118) on arrays of arguments (device pointers): lets the
  * known-answer vectors of the reference's primitive be checked against the GPU code itself. */
 int illico_compute_pval_batch(const int64_t* n_ref, const int64_t* n_tgt, const int64_t* n, const double* tie_sum,
