@@ -91,7 +91,13 @@ SIGNATURES = {
     "illico_csr_shard_count": (C.c_int, [_vp, _vp, _i64, _vp, _i32, _vp, _vp, _vp]),
     "illico_csr_shard_scatter": (C.c_int, [_vp, _vp, _vp, _i64, _i64, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "illico_host_pack_rows_f32": (C.c_long, [_vp, C.c_long, C.c_long, C.c_long, _vp, _vp, _vp, C.c_long]),
+    "illico_host_pack_row_list_f32": (C.c_long, [_vp, C.c_long, _vp, C.c_long, C.c_long, _vp, _vp, _vp, C.c_long]),
     "illico_host_pack_isa": (C.c_int, []),
+    "illico_select_rows_dense": (C.c_int, [_vp, _i32, _i64, _i64, _vp, _i64, _vp, _i64, _vp]),
+    "illico_select_rows_csr_indptr": (C.c_int, [_vp, _vp, _i64, _vp, _vp]),
+    "illico_select_rows_csr": (C.c_int, [_vp, _i32, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp]),
+    "illico_select_rows_csc_indptr": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _vp]),
+    "illico_select_rows_csc": (C.c_int, [_vp, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp]),
     "illico_unpack_rows_f32": (C.c_int, [_vp, _vp, _vp, _i64, _i32, _vp, _i64, _vp]),
     "illico_bh_workspace_bytes": (_sz, [_i32, _i32]),
     "illico_bh_adjust": (C.c_int, [_vp, _i64, _i64, _i32, _i32, _vp, _vp, _sz, _vp]),

@@ -25,7 +25,7 @@ from scipy import sparse
 
 from . import hostio
 from .engine import CSR, WILCOXON, DeviceMatrix, Engine, check_method, make_flags, require_cuda
-from .groups import encode_and_count_groups, seg_max_from_env
+from .groups import collapse_unselected, encode_and_count_groups, seg_max_from_env, select_groups, subset_for_reference
 from .registry import DataHandler, data_handler_registry
 
 __all__ = ["asymptotic_wilcoxon"]
@@ -115,6 +115,7 @@ def asymptotic_wilcoxon(
     log2_fold_change: bool = False,
     score: bool = False,
     pts: bool = False,
+    groups=None,
 ):
     """Asymptotic Mann-Whitney / Wilcoxon rank-sum tests for every (group, gene) on B200 GPUs.
 
@@ -138,13 +139,19 @@ def asymptotic_wilcoxon(
       ``pts``      add the columns ``pct_nz_group`` (fraction of the group's cells whose value is non-zero) and
                    ``pct_nz_reference`` (the same fraction in the reference group, or in all other cells for one-versus-rest;
                    NaN when there are no other cells) -- scanpy's ``rank_genes_groups(pts=True)``.  Counted on the GPU in a
-                   pass of its own; p-values, U and fold changes are those of the same call without it.
+                   pass of its own; p-values, U and fold changes are those of the same call without it;
+      ``groups``   scanpy's ``groups``: ``None`` / ``"all"`` (every group), one label or an iterable of labels -- only those
+                   groups are tested and reported (in ``np.unique`` order, the reference group added when missing; an unknown
+                   label or an empty selection is a ``ValueError``).  One-versus-reference reads only the cells of the
+                   selected groups (the others never reach the GPU where the input allows); one-versus-rest still compares
+                   each selected group with every other cell, those of the unselected groups included.  Each selected group's
+                   rows are those of the same call without ``groups``.
     With ``return_array`` and an optional column, the result is ``(groups, var_names, results, {name: [G, N] array})``.
     """
     del precompile  # kernels are compiled ahead of time
     check_flag("pts", pts)
     run = _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, alternative, use_continuity,
-                     tie_correct, layer, device, devices, score=score, on_device=False, pts=pts)
+                     tie_correct, layer, device, devices, score=score, on_device=False, pts=pts, groups=groups)
     out = run.results
     extra = {}
     if p_adjust:
@@ -165,8 +172,10 @@ def asymptotic_wilcoxon(
 
 class _Run:
     """What ``_run_tests`` delivers: the groups (``np.unique`` order), the group container, the first GPU, and the results
-    ``[G, N, 3]`` / score plane ``[G, N]`` / int32 count plane ``[G, N]`` of cells with a non-zero value (the planes None
-    unless asked for) -- pinned host arrays, or tensors on that GPU."""
+    ``[G, N, 3]`` / score plane ``[G, N]`` / int32 count plane ``[G', N]`` of cells with a non-zero value (the planes None
+    unless asked for) -- pinned host arrays, or tensors on that GPU.  With ``groups=`` one-versus-rest, the container and
+    the count plane also hold the pseudo-groups of the cells of the other groups (``G' > G``: rows ``G ..``), which the
+    fractions of the rest need; the results and scores hold the selected groups only."""
 
     def __init__(self, groups, grpc, device, results, scores, nnz=None):
         self.groups, self.grpc, self.device, self.results, self.scores, self.nnz = groups, grpc, device, results, scores, nnz
@@ -198,9 +207,9 @@ def nonzero_fractions(nnz: torch.Tensor, grpc):
 
 def _host_fractions(run: _Run):
     """The fractions of a run whose count plane came back to the host: computed on the run's first GPU and copied back."""
-    G, N = run.nnz.shape
+    G, N = len(run.groups), run.nnz.shape[1]
     with torch.cuda.device(run.device):
-        pg, pr = nonzero_fractions(torch.from_numpy(run.nnz).to(run.device, non_blocking=True), run.grpc)
+        pg, pr = (p[:G] for p in nonzero_fractions(torch.from_numpy(run.nnz).to(run.device, non_blocking=True), run.grpc))
         out = []
         for plane in (pg, pr):
             host = torch.empty((G, N), dtype=torch.float64, pin_memory=True)
@@ -211,16 +220,37 @@ def _host_fractions(run: _Run):
 
 
 def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, alternative, use_continuity, tie_correct,
-               layer, device, devices, score: bool, on_device: bool, pts: bool = False, method: str = WILCOXON) -> _Run:
+               layer, device, devices, score: bool, on_device: bool, pts: bool = False, method: str = WILCOXON,
+               groups=None) -> _Run:
     """Every (group, gene) test of ``adata``: validation, upload, group plan, one gene shard per GPU, batches, backed
     streaming.  ``on_device=False``: each shard's slabs are copied into pinned host arrays (``asymptotic_wilcoxon``).
     ``on_device=True``: they stay on the GPUs and meet in ``[G, N, 3]`` / ``[G, N]`` tensors on the first one
     (device-to-device copies; with one shard its own tensors are the result).  ``pts``: the count plane too.  ``method``:
-    the Wilcoxon test or one of the t-tests (``Engine.run_batch``)."""
+    the Wilcoxon test or one of the t-tests (``Engine.run_batch``).  ``groups``: the groups to test (``asymptotic_wilcoxon``);
+    one-versus-reference then runs on the rows of their cells (``rows``, with their own group container), one-versus-rest
+    on every cell with the other groups collapsed into pseudo-groups whose rows are dropped."""
     check_method(method)
     X = adata.layers[layer] if layer is not None else adata.X
     if isinstance(X, (sparse.csr_array, sparse.csc_array)):
         X = sparse.csr_matrix(X) if isinstance(X, sparse.csr_array) else sparse.csc_matrix(X)
+    unique_raw_groups = grpc = rows = None
+    if not (groups is None or (isinstance(groups, str) and groups == "all")):
+        # the labels decide which rows go to the GPU: encode them first (and refuse a bad selection before any device work)
+        unique_raw_groups, grpc = _encode_groups(adata, group_keys, reference, X.shape[0])
+        sel = select_groups(unique_raw_groups, groups, grpc.encoded_ref_group)
+        if sel is not None:
+            unique_raw_groups = unique_raw_groups[sel]
+            if grpc.encoded_ref_group >= 0:
+                rows, grpc = subset_for_reference(grpc, sel)
+                if isinstance(X, sparse.csr_matrix):
+                    X, rows = X[rows], None     # host CSR: its rows are cut here (scipy keeps the indices sorted)
+            else:
+                grpc = collapse_unselected(grpc, sel)
+    selection = None
+    if rows is not None:
+        from .select import RowSelection
+
+        selection = RowSelection(rows, X.shape[0])
     data_handler = data_handler_registry.get(X)  # KeyError for unsupported containers, like the reference
     if devices is None and device is None and isinstance(X, torch.Tensor) and X.is_cuda:
         device = X.device          # a device-resident matrix is ranked where it lives
@@ -259,6 +289,11 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
             prep = threading.Thread(target=_prep, daemon=True)
             prep.start()
 
+    def upload(sh: _Shard):
+        if selection is None:
+            return data_handler.upload_shard(sh.lb, sh.ub, sh.device)
+        return data_handler.upload_shard(sh.lb, sh.ub, sh.device, rows=selection.rows)
+
     def run_shard(sh: _Shard):
         """Everything one GPU does, on its own host thread: upload its gene shard (started before the groups are
         encoded), rank it batch by batch, deliver its slab."""
@@ -272,7 +307,7 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
             with torch.cuda.device(sh.device):
                 M = bounds = None
                 if data_handler.in_ram:
-                    M, bounds = sh.started or data_handler.upload_shard(sh.lb, sh.ub, sh.device)
+                    M, bounds = sh.started or upload(sh)
                 plan_ready.wait()
                 if "error" in shared:
                     return
@@ -283,6 +318,10 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
                 nz = torch.empty((engine.n_groups, sh.ub - sh.lb), dtype=torch.int32, device=sh.device) if pts else None
                 if data_handler.in_ram:
                     M.ready()
+                    if selection is not None:
+                        from .select import select_rows
+
+                        M, bounds = select_rows(M, bounds, selection)
                     if fmt == CSR and not engine.check_csr_sorted(M):
                         raise ValueError(
                             "Input data matrix indices are not sorted. This is very unusual and may lead to incorrect results. "
@@ -295,7 +334,7 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
                         engine.run_batch(M, lb + off, ub + off, flags, res, lb - sh.lb, scores=sc, nnz=nz, method=method)
                 else:
                     _run_backed(data_handler, _batches(sh.lb, sh.ub, batch_size, engine, False, method), engine, flags, res,
-                                max(1, int(n_threads)), gene0=sh.lb, scores=sc, nnz=nz, method=method)
+                                max(1, int(n_threads)), gene0=sh.lb, scores=sc, nnz=nz, method=method, selection=selection)
                 if on_device and len(shards) == 1:
                     shared["out"], shared["out_scores"], shared["out_nnz"] = res, sc, nz
                 else:
@@ -321,10 +360,9 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
         if len(shards) == 1 and data_handler.in_ram:
             # single GPU: start the upload from this thread, then encode while it is in flight
             with torch.cuda.device(shards[0].device):
-                shards[0].started = data_handler.upload_shard(shards[0].lb, shards[0].ub, shards[0].device)
-        unique_raw_groups, grpc = encode_and_count_groups(groups=adata.obs[group_keys], ref_group=reference)
-        if grpc.encoded_groups.size != n_cells:
-            raise ValueError(f"{grpc.encoded_groups.size} group labels for {n_cells} cells")
+                shards[0].started = upload(shards[0])
+        if grpc is None:
+            unique_raw_groups, grpc = _encode_groups(adata, group_keys, reference, n_cells)
         from .groups import build_plan
 
         shared["grpc"], shared["host_plan"] = grpc, build_plan(grpc, seg_max)
@@ -356,7 +394,15 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
     if not on_device:
         out, scores = out.numpy(), (scores.numpy() if scores is not None else None)
         nnz = nnz.numpy() if nnz is not None else None
-    return _Run(unique_raw_groups, grpc, shards[0].device, out, scores, nnz)
+    S = len(unique_raw_groups)     # (fewer than G when one-versus-rest pseudo-groups follow the selected groups)
+    return _Run(unique_raw_groups, grpc, shards[0].device, out[:S], scores[:S] if scores is not None else None, nnz)
+
+
+def _encode_groups(adata, group_keys, reference, n_cells: int):
+    unique_raw_groups, grpc = encode_and_count_groups(groups=adata.obs[group_keys], ref_group=reference)
+    if grpc.encoded_groups.size != n_cells:
+        raise ValueError(f"{grpc.encoded_groups.size} group labels for {n_cells} cells")
+    return unique_raw_groups, grpc
 
 
 def _bh_adjust(out: np.ndarray, device) -> np.ndarray:
@@ -424,14 +470,15 @@ class _PinnedSlot:
 
 
 def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, results, n_readers: int, gene0: int = 0,
-                scores=None, nnz=None, method: str = WILCOXON) -> None:
+                scores=None, nnz=None, method: str = WILCOXON, selection=None) -> None:
     """Out-of-core input (BASELINE config 4): gene batches stream disk -> pinned ring -> HBM -> kernels.
 
     Reader threads slice the next batches from the backed container straight into pinned staging buffers (a ring of
     ``n_readers + 2`` slots); the main thread enqueues each batch's ``cudaMemcpyAsync`` on a copy stream and the
     kernels on the compute stream, ordered by events, so the disk read and H2D copy of batch ``i + 1`` overlap the
     ranking of batch ``i`` (the reference's joblib threads overlap I/O and numba kernels the same way,
-    ``asymptotic_wilcoxon.py:212-249``)."""
+    ``asymptotic_wilcoxon.py:212-249``).  ``selection`` (``select.RowSelection``): only those rows are ranked -- the readers
+    gather them out of dense batches, CSC batches are compacted on the device (``illico_select_rows_csc``)."""
     from .engine import DENSE, DeviceMatrix, _to_f32_or_wide
 
     dev = engine.device
@@ -467,6 +514,8 @@ def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, resu
                     slot.copied.synchronize()   # the device is done reading this slot's previous batch
                 data, bounds = data_handler.fetch(lb, ub)
                 if fmt == DENSE:
+                    if selection is not None:
+                        data = np.take(data, selection.rows, axis=0)
                     staged = {"shape": data.shape, "x": slot.stage("x", data)}
                 else:
                     staged = {"shape": data.shape, "data": slot.stage("data", data.data),
@@ -510,6 +559,10 @@ def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, resu
             if data.dtype != torch.float32:
                 data, raw = _to_f32_or_wide(data)
             M = DeviceMatrix(fmt, tuple(shape), data, dv["indices"], dv["indptr"], raw=raw)
+            if selection is not None:
+                from .select import select_rows
+
+                M, bounds = select_rows(M, bounds, selection)
         engine.run_batch(M, bounds[0], bounds[1], flags, results, lb - gene0, scores=scores, nnz=nnz, method=method)
 
     try:

@@ -11,6 +11,7 @@
  */
 #include <immintrin.h>
 #include <stdint.h>
+#include <stddef.h>
 #include <string.h>
 
 #define PREFETCH_AHEAD 4096
@@ -95,13 +96,8 @@ int illico_host_pack_isa(void) {
     return 0;
 }
 
-/* Packs rows [0, n_rows) of a row-major float32 matrix (row stride in elements, n_cols columns read per row):
- *   mask    [n_rows][W] uint32, W = (n_cols + 31) / 32: bit k of word w = element 32 w + k is non-zero
- *   row_off [n_rows + 1] uint32: position of each row's first value in vals
- *   vals    the non-zero values, row by row, in column order; capacity vals_cap floats (16 floats of slack included)
- * Returns the number of values, or -1 when they do not fit (the caller then sends the chunk as it is). */
-long illico_host_pack_rows_f32(const float* src, long row_stride, long n_rows, long n_cols, uint32_t* mask, uint32_t* row_off,
-                               float* vals, long vals_cap) {
+static long pack_rows(const float* src, long row_stride, const int64_t* rows, long n_rows, long n_cols, uint32_t* mask,
+                      uint32_t* row_off, float* vals, long vals_cap) {
     const int isa = illico_host_pack_isa();
     if (isa == 1 && !g_perm_ready) build_perm();
     const long W = (n_cols + 31) / 32;
@@ -109,11 +105,28 @@ long illico_host_pack_rows_f32(const float* src, long row_stride, long n_rows, l
     for (long r = 0; r < n_rows; ++r) {
         if ((o - vals) + n_cols + 16 > vals_cap) return -1;
         row_off[r] = (uint32_t)(o - vals);
-        const float* row = src + r * row_stride;
+        const float* row = src + (rows ? rows[r] : r) * row_stride;
         if (isa == 2) row_avx512(row, n_cols, mask + r * W, &o);
         else if (isa == 1) row_avx2(row, n_cols, mask + r * W, &o);
         else scalar_words(row, 0, n_cols, mask + r * W, &o);
     }
     row_off[n_rows] = (uint32_t)(o - vals);
     return (long)(o - vals);
+}
+
+/* Packs rows [0, n_rows) of a row-major float32 matrix (row stride in elements, n_cols columns read per row):
+ *   mask    [n_rows][W] uint32, W = (n_cols + 31) / 32: bit k of word w = element 32 w + k is non-zero
+ *   row_off [n_rows + 1] uint32: position of each row's first value in vals
+ *   vals    the non-zero values, row by row, in column order; capacity vals_cap floats (16 floats of slack included)
+ * Returns the number of values, or -1 when they do not fit (the caller then sends the chunk as it is). */
+long illico_host_pack_rows_f32(const float* src, long row_stride, long n_rows, long n_cols, uint32_t* mask, uint32_t* row_off,
+                               float* vals, long vals_cap) {
+    return pack_rows(src, row_stride, NULL, n_rows, n_cols, mask, row_off, vals, vals_cap);
+}
+
+/* The same for the rows rows[0 .. n_rows) of the matrix (any order; packed row r is source row rows[r]): the upload of the
+ * cells of the groups a call tests gathers them while it squeezes them. */
+long illico_host_pack_row_list_f32(const float* src, long row_stride, const int64_t* rows, long n_rows, long n_cols, uint32_t* mask,
+                                   uint32_t* row_off, float* vals, long vals_cap) {
+    return pack_rows(src, row_stride, rows, n_rows, n_cols, mask, row_off, vals, vals_cap);
 }

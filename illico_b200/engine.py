@@ -398,22 +398,24 @@ def _torch_dtype(a: np.ndarray):
     return torch.from_numpy(np.empty(0, dtype=a.dtype)).dtype
 
 
-def upload_dense(X, device, gene_lb: int = 0, gene_ub: int | None = None) -> DeviceMatrix:
+def upload_dense(X, device, gene_lb: int = 0, gene_ub: int | None = None, rows=None) -> DeviceMatrix:
     """Starts the copy of ``X[:, gene_lb:gene_ub]`` (any real dtype) into a device matrix and returns at once: pinned
     sources go out as one strided asynchronous copy, pageable ones through the pinned staging ring of
-    :mod:`illico_b200.hostio` (worker threads), so the caller keeps working on the host meanwhile.
-    ``DeviceMatrix.ready()`` joins."""
+    :mod:`illico_b200.hostio` (worker threads), so the caller keeps working on the host meanwhile.  ``rows`` (ascending
+    int64, optional): only those rows go up, gathered by the staging threads.  ``DeviceMatrix.ready()`` joins."""
     from . import hostio
 
     device = require_cuda(device)
     n, N = X.shape
+    if rows is not None:
+        n = len(rows)
     gene_ub = N if gene_ub is None else gene_ub
     if isinstance(X, torch.Tensor):
         X = X.numpy()
     view = _uploadable(np.asarray(X[:, gene_lb:gene_ub]))
     with torch.cuda.device(device):
         d = torch.empty((n, gene_ub - gene_lb), dtype=_torch_dtype(view), device=device)
-        pend = hostio.h2d_2d(d, view)
+        pend = hostio.h2d_2d(d, view, rows=rows)
     if d.dtype == torch.float32:
         return DeviceMatrix(DENSE, (n, gene_ub - gene_lb), d, gene_offset=gene_lb, pending=[pend])
     return DeviceMatrix(DENSE, (n, gene_ub - gene_lb), None, gene_offset=gene_lb, pending=[pend], unconverted=d)

@@ -84,13 +84,67 @@ def encode_and_count_groups(groups, ref_group: Any):
         encoded_ref = int(hit[0])
     else:
         encoded_ref = -1
-    G = len(unique_groups)
-    encoded = np.ascontiguousarray(inverse, dtype=np.int64)
+    return unique_groups, _container(inverse, len(unique_groups), encoded_ref)
+
+
+def _container(codes, G: int, encoded_ref: int) -> GroupContainer:
+    encoded = np.ascontiguousarray(codes, dtype=np.int64)
     counts = np.bincount(encoded, minlength=G).astype(np.int64)
     small = encoded.astype(np.int16) if G < 2**15 else encoded  # 16-bit keys take numpy's radix sort
     indices = np.argsort(small, kind="stable").astype(np.int64)
     indptr = np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
-    return unique_groups, GroupContainer(encoded, counts, indices, indptr, encoded_ref)
+    return GroupContainer(encoded, counts, indices, indptr, encoded_ref)
+
+
+# ---- groups= : the groups a call tests ----------------------------------------------------------------------------------
+# Cells of a one-versus-rest pseudo-group (the cells of the groups not tested, collapsed): below the fused path's 65 536-cell
+# group limit (DESIGN.md section 2.2), so that collapsing them never moves a batch off that path.
+PSEUDO_GROUP_MAX = 65535
+
+
+def select_groups(unique_groups, groups, encoded_ref: int):
+    """Indices into ``unique_groups`` (ascending: ``np.unique`` order) of the groups ``groups`` asks for, the reference group
+    added when it is missing; None when that is every group.  ``groups``: None or ``"all"`` (every group), one label
+    (a ``str``) or an iterable of labels, duplicates collapsed.  An unknown label or an empty selection is a ``ValueError``."""
+    import pandas as pd
+
+    if groups is None or (isinstance(groups, str) and groups == "all"):
+        return None
+    labels = [groups] if isinstance(groups, str) else list(groups)
+    if not labels:
+        raise ValueError("groups selects no group: pass None or 'all' for every group, or at least one label")
+    hit = pd.Index(unique_groups).get_indexer(pd.Index(labels, dtype=object))
+    if (hit < 0).any():
+        missing = [lab for lab, h in zip(labels, hit) if h < 0]
+        raise ValueError(f"groups: {missing} not found in the group labels")
+    sel = np.unique(np.concatenate([hit, [encoded_ref]]) if encoded_ref >= 0 else hit)
+    return None if sel.size == len(unique_groups) else sel.astype(np.int64)
+
+
+def subset_for_reference(grpc: GroupContainer, sel: np.ndarray):
+    """One-versus-reference on the selected groups ``sel``: ``(rows, GroupContainer)`` -- the rows of their cells, ascending,
+    and the container of the matrix made of those rows (groups renumbered ``0 .. sel.size - 1`` in the same order, the
+    reference among them).  Every selected group keeps its cells in their order, so the plan gives it the segments of the
+    full call."""
+    remap = np.full(grpc.counts.size, -1, dtype=np.int64)
+    remap[sel] = np.arange(sel.size)
+    codes = remap[grpc.encoded_groups]
+    rows = np.flatnonzero(codes >= 0)
+    return rows, _container(codes[rows], sel.size, int(remap[grpc.encoded_ref_group]))
+
+
+def collapse_unselected(grpc: GroupContainer, sel: np.ndarray) -> GroupContainer:
+    """One-versus-rest on the selected groups ``sel``: every cell stays (the rest of a group is every other cell).  The
+    selected groups become groups ``0 .. sel.size - 1``; the other cells, in ascending row order, are cut into
+    ``ceil(n / PSEUDO_GROUP_MAX)`` runs of near-equal size, the pseudo-groups ``sel.size ..``, whose rows of every output are
+    dropped."""
+    remap = np.full(grpc.counts.size, -1, dtype=np.int64)
+    remap[sel] = np.arange(sel.size)
+    codes = remap[grpc.encoded_groups]
+    rest = np.flatnonzero(codes < 0)
+    P = -(-rest.size // PSEUDO_GROUP_MAX)
+    codes[rest] = sel.size + np.arange(rest.size, dtype=np.int64) * P // rest.size
+    return _container(codes, sel.size + P, -1)
 
 
 def _is_stable_group_order(enc, perm) -> bool:

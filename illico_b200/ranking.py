@@ -57,6 +57,7 @@ def rank_genes(
     max_out_group_fraction: float | None = None,
     min_fold_change: float | None = None,
     method: str = "wilcoxon",
+    groups=None,
 ) -> pd.DataFrame:
     """The ``n_genes`` strongest genes of every group, by Wilcoxon score (or Welch's t with ``method="t-test"``).
 
@@ -83,6 +84,9 @@ def rank_genes(
     ``method`` is scanpy's: ``"wilcoxon"`` (the default), ``"t-test"`` or ``"t-test_overestim_var"`` (Welch's t-test, as
     ``illico_b200.ttest``).  For a t-test ``score`` and ``statistic`` are t (``score`` with NaN replaced by 0, the p-value
     NaN replaced by 1), the fold change is the Wilcoxon call's, and ``use_continuity`` / ``tie_correct`` are ignored.
+
+    ``groups`` is scanpy's (see ``asymptotic_wilcoxon``): only the selected groups are tested and shown, each with the rows
+    it has in the same call without ``groups``.
     """
     check_method(method)
     if n_genes is not None:
@@ -96,7 +100,7 @@ def rank_genes(
     fc_min = _bound("min_fold_change", min_fold_change, None)
     with_pts = bool(pts) or any(v is not None for v in (min_in, max_out, fc_min))
     run = _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, alternative, use_continuity,
-                     tie_correct, layer, device, devices, score=True, on_device=True, pts=with_pts, method=method)
+                     tie_correct, layer, device, devices, score=True, on_device=True, pts=with_pts, method=method, groups=groups)
     res, scores = run.results, run.scores
     G, N = int(res.shape[0]), int(res.shape[1])
     k = N if n_genes is None else min(int(n_genes), N)
@@ -110,7 +114,7 @@ def rank_genes(
         gene, rec = np.zeros((G, 0), np.int32), np.zeros((G, 0, width))
         k, rows[:] = 0, 0
     elif with_pts:
-        pct = nonzero_fractions(run.nnz, run.grpc)
+        pct = tuple(p[:G] for p in nonzero_fractions(run.nnz, run.grpc))     # (one-versus-rest pseudo-groups dropped)
         fc_max = (1.0 / fc_min if fc_min > 0 else math.inf) if rankby_abs and fc_min is not None else None
         gene, rec, kept = top_genes_filtered(res, scores, pct, k, rankby_abs, min_in, max_out, fc_min, fc_max)
         rows = np.minimum(rows, kept)

@@ -112,16 +112,18 @@ class InRAMDataHandler(DataHandler):
             self._resident = self.upload_shard(0, self.data.shape[1], getattr(engine, "device", engine))[0]
         return self._resident
 
-    def upload_shard(self, lb: int, ub: int, device) -> tuple:
+    def upload_shard(self, lb: int, ub: int, device, rows=None) -> tuple:
         """``(DeviceMatrix, (lb', ub'))``: genes ``[lb, ub)`` on ``device`` and their bounds inside that matrix.
-        Returns as soon as the copies are started (``DeviceMatrix.ready()`` joins them)."""
+        Returns as soon as the copies are started (``DeviceMatrix.ready()`` joins them).  ``rows`` (ascending int64): the
+        cells a call needs; a handler that can gather them on the way up does, the others upload every row and the caller
+        selects them on the device (``select.select_rows``)."""
         raise NotImplementedError
 
 
 @data_handler_registry.register(np.ndarray)
 class DenseDataHandler(InRAMDataHandler):
-    def upload_shard(self, lb, ub, device):
-        return upload_dense(self.data, device, lb, ub), (0, ub - lb)
+    def upload_shard(self, lb, ub, device, rows=None):
+        return upload_dense(self.data, device, lb, ub, rows), (0, ub - lb)
 
     def kernel_data_format(self):
         return KernelDataFormat.DENSE
@@ -132,7 +134,7 @@ class DenseDataHandler(InRAMDataHandler):
 
 @data_handler_registry.register(py_sparse.csr_matrix)
 class CSRDataHandler(InRAMDataHandler):
-    def upload_shard(self, lb, ub, device):
+    def upload_shard(self, lb, ub, device, rows=None):
         # every CSR row holds all genes: the whole matrix goes to each GPU over its own link (1.9 GB at the K562 shape)
         # and the kernels select the gene range
         return upload_sparse(self.data, CSR, device), (lb, ub)
@@ -146,7 +148,7 @@ class CSRDataHandler(InRAMDataHandler):
 
 @data_handler_registry.register(py_sparse.csc_matrix)
 class CSCDataHandler(InRAMDataHandler):
-    def upload_shard(self, lb, ub, device):
+    def upload_shard(self, lb, ub, device, rows=None):
         return upload_sparse(self.data, CSC, device, lb, ub), (0, ub - lb)
 
     def kernel_data_format(self):
@@ -198,7 +200,7 @@ class TorchDenseDataHandler(InRAMDataHandler):
     """A 2-D ``torch.Tensor``: CUDA tensors are used where they are (no host round trip -- SURVEY section 8f.3), CPU
     tensors go through the ndarray path."""
 
-    def upload_shard(self, lb, ub, device):
+    def upload_shard(self, lb, ub, device, rows=None):
         import torch
 
         from .engine import _to_f32_or_wide
@@ -207,7 +209,7 @@ class TorchDenseDataHandler(InRAMDataHandler):
         if X.ndim != 2:
             raise ValueError("expression matrix must be two-dimensional")
         if not X.is_cuda:
-            return upload_dense(X.numpy(), device, lb, ub), (0, ub - lb)
+            return upload_dense(X.numpy(), device, lb, ub, rows), (0, ub - lb)
         want = torch.device(device)
         if want.type == "cuda" and want.index is None:
             want = torch.device("cuda", torch.cuda.current_device())

@@ -37,6 +37,7 @@ def ttest(
     log2_fold_change: bool = False,
     score: bool = False,
     pts: bool = False,
+    groups=None,
 ):
     """Welch's t-test of every group against ``reference`` (or, when it is None, against all other cells) in every gene.
 
@@ -51,14 +52,14 @@ def ttest(
     of ``expm1(x)`` when ``is_log1p``; ``inf`` where the comparison mean is 0).  The reference group's rows are
     ``(1, 0, fold change of the control with itself)``.  ``is_log1p`` affects only the fold change.
     ``score`` adds t with NaN replaced by 0 (scanpy's ``scores``); ``p_adjust``, ``log2_fold_change``, ``pts``,
-    ``return_array``, ``device``, ``devices``, ``n_threads``, ``batch_size`` and ``layer`` are those of
+    ``return_array``, ``device``, ``devices``, ``n_threads``, ``batch_size``, ``layer`` and ``groups`` are those of
     ``asymptotic_wilcoxon``.
     """
     if check_method(method) == WILCOXON:
         raise ValueError("ttest runs the t-tests; method='wilcoxon' is asymptotic_wilcoxon")
     check_flag("pts", pts)
     run = _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, alternative, True, True, layer, device,
-                     devices, score=score, on_device=False, pts=pts, method=method)
+                     devices, score=score, on_device=False, pts=pts, method=method, groups=groups)
     out = run.results
     extra = {}
     if p_adjust:

@@ -287,9 +287,37 @@ int illico_csr_shard_scatter(const float* data, const int32_t* indices, const in
  * (the caller then sends the chunk as it is).  The isa call returns 2 / 1 / 0 = AVX-512 / AVX2 / scalar. */
 long illico_host_pack_rows_f32(const float* src, long row_stride, long n_rows, long n_cols, uint32_t* mask, uint32_t* row_off,
                                float* vals, long vals_cap);
+/* The same for source rows rows[0 .. n_rows) (host int64 array): packed row r is row rows[r] of src. */
+long illico_host_pack_row_list_f32(const float* src, long row_stride, const int64_t* rows, long n_rows, long n_cols, uint32_t* mask,
+                                   uint32_t* row_off, float* vals, long vals_cap);
 int illico_host_pack_isa(void);
 int illico_unpack_rows_f32(const uint32_t* mask, const uint32_t* row_off, const float* vals, int64_t n_rows, int32_t n_cols,
                            float* dst, int64_t dst_ld, void* stream);
+
+/* ---- the cells of the groups a call tests (groups=, one-versus-reference) -----------------------------------------------
+ * Row selection of a device-resident matrix, rows kept in the order given (the caller passes them ascending, so that every
+ * group keeps the order of its cells).  `dtype` is ILLICO_DTYPE_F32 or ILLICO_DTYPE_F64; values are copied bit for bit.
+ *   illico_select_rows_dense       out[i, c] = X[rows[i], c] for c < n_cols, 0 for n_cols <= c < out_ld (row padding); X of
+ *                                  any ld >= n_cols.
+ *   illico_select_rows_csr_indptr  out_indptr [n_rows + 1] = the exclusive scan of the lengths of rows rows[i] (out_indptr[n_rows]
+ *                                  = the entries of the selection: read it back to size out_data / out_indices).
+ *   illico_select_rows_csr         the pieces of those rows at out_indptr[i] (column indices stay sorted).
+ *   illico_select_rows_csc_indptr  columns [0, n_cols) of `indptr` (pass indptr + gene_lb for a batch; the values index
+ *                                  data / indices as they are): out_indptr [n_cols + 1] = the exclusive scan of the entries
+ *                                  whose row r has new_row[r] >= 0 (new_row [n_cells]: the row's number in the selection,
+ *                                  -1 = dropped).
+ *   illico_select_rows_csc         those entries at out_indptr[c], rows renumbered through new_row, in their order (a stable
+ *                                  compaction: each column's rows still ascend).
+ * No workspace; the scans run in place on out_indptr. */
+int illico_select_rows_dense(const void* X, int32_t dtype, int64_t ld, int64_t n_cols, const int32_t* rows, int64_t n_rows,
+                             void* out, int64_t out_ld, void* stream);
+int illico_select_rows_csr_indptr(const int64_t* indptr, const int32_t* rows, int64_t n_rows, int64_t* out_indptr, void* stream);
+int illico_select_rows_csr(const void* data, int32_t dtype, const int32_t* indices, const int64_t* indptr, const int32_t* rows,
+                           int64_t n_rows, const int64_t* out_indptr, void* out_data, int32_t* out_indices, void* stream);
+int illico_select_rows_csc_indptr(const int32_t* indices, const int64_t* indptr, int32_t n_cols, const int32_t* new_row,
+                                  int64_t* out_indptr, void* stream);
+int illico_select_rows_csc(const void* data, int32_t dtype, const int32_t* indices, const int64_t* indptr, int32_t n_cols,
+                           const int32_t* new_row, const int64_t* out_indptr, void* out_data, int32_t* out_indices, void* stream);
 
 /* ---- next to the path (SURVEY.md section 8f.4) and a test hook ------------------------------------------- */
 
