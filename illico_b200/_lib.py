@@ -92,8 +92,10 @@ SIGNATURES = {
     "illico_csr_shard_scatter": (C.c_int, [_vp, _vp, _vp, _i64, _i64, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "illico_host_pack_rows_f32": (C.c_long, [_vp, C.c_long, C.c_long, C.c_long, _vp, _vp, _vp, C.c_long]),
     "illico_host_pack_row_list_f32": (C.c_long, [_vp, C.c_long, _vp, C.c_long, C.c_long, _vp, _vp, _vp, C.c_long]),
+    "illico_host_pack_cols_f32": (C.c_long, [_vp, C.c_long, _vp, C.c_long, _vp, C.c_long, _vp, _vp, _vp, C.c_long]),
     "illico_host_pack_isa": (C.c_int, []),
     "illico_select_rows_dense": (C.c_int, [_vp, _i32, _i64, _i64, _vp, _i64, _vp, _i64, _vp]),
+    "illico_select_cols_dense": (C.c_int, [_vp, _i32, _i64, _vp, _i64, _vp, _i64, _vp, _i64, _vp]),
     "illico_select_rows_csr_indptr": (C.c_int, [_vp, _vp, _i64, _vp, _vp]),
     "illico_select_rows_csr": (C.c_int, [_vp, _i32, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp]),
     "illico_select_rows_csc_indptr": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _vp]),

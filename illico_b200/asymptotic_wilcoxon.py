@@ -116,6 +116,7 @@ def asymptotic_wilcoxon(
     score: bool = False,
     pts: bool = False,
     groups=None,
+    mask_var=None,
 ):
     """Asymptotic Mann-Whitney / Wilcoxon rank-sum tests for every (group, gene) on B200 GPUs.
 
@@ -145,13 +146,22 @@ def asymptotic_wilcoxon(
                    label or an empty selection is a ``ValueError``).  One-versus-reference reads only the cells of the
                    selected groups (the others never reach the GPU where the input allows); one-versus-rest still compares
                    each selected group with every other cell, those of the unselected groups included.  Each selected group's
-                   rows are those of the same call without ``groups``.
+                   rows are those of the same call without ``groups``;
+      ``mask_var`` scanpy's ``mask_var``: ``None`` (every gene), the name of a boolean column of ``adata.var`` (such as
+                   ``"highly_variable"``) or a boolean mask of length ``n_vars`` (numpy array, list or pandas Series; integer
+                   positions, a wrong length, a missing or non-boolean column and a mask with no ``True`` are a ``ValueError``,
+                   raised before any device work) -- only those genes are tested and reported, in ``var_names`` order.  Each
+                   one's p-value, U, fold change, score and fractions are those of the same call without ``mask_var``;
+                   ``p_adj`` is Benjamini-Hochberg over the selected genes of each group, as in scanpy.  Dense host matrices,
+                   CSC input (in RAM or backed) and CUDA tensors move only the selected columns to the GPU; a host CSR matrix
+                   goes up whole and is compacted there.
     With ``return_array`` and an optional column, the result is ``(groups, var_names, results, {name: [G, N] array})``.
     """
     del precompile  # kernels are compiled ahead of time
     check_flag("pts", pts)
     run = _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, alternative, use_continuity,
-                     tie_correct, layer, device, devices, score=score, on_device=False, pts=pts, groups=groups)
+                     tie_correct, layer, device, devices, score=score, on_device=False, pts=pts, groups=groups,
+                     mask_var=mask_var)
     out = run.results
     extra = {}
     if p_adjust:
@@ -165,9 +175,9 @@ def asymptotic_wilcoxon(
         extra["pct_nz_group"], extra["pct_nz_reference"] = _host_fractions(run)
     if return_array:
         if extra:
-            return run.groups, np.asarray(adata.var_names), out, extra
-        return run.groups, np.asarray(adata.var_names), out
-    return _result_frame(run.groups, adata.var_names, out, extra)
+            return run.groups, np.asarray(run.var_names), out, extra
+        return run.groups, np.asarray(run.var_names), out
+    return _result_frame(run.groups, run.var_names, out, extra)
 
 
 class _Run:
@@ -175,10 +185,12 @@ class _Run:
     ``[G, N, 3]`` / score plane ``[G, N]`` / int32 count plane ``[G', N]`` of cells with a non-zero value (the planes None
     unless asked for) -- pinned host arrays, or tensors on that GPU.  With ``groups=`` one-versus-rest, the container and
     the count plane also hold the pseudo-groups of the cells of the other groups (``G' > G``: rows ``G ..``), which the
-    fractions of the rest need; the results and scores hold the selected groups only."""
+    fractions of the rest need; the results and scores hold the selected groups only.  ``var_names``: the names of the
+    ``N`` genes tested (``adata.var_names``, or its selected entries with ``mask_var=``)."""
 
-    def __init__(self, groups, grpc, device, results, scores, nnz=None):
+    def __init__(self, groups, grpc, device, results, scores, nnz=None, var_names=None):
         self.groups, self.grpc, self.device, self.results, self.scores, self.nnz = groups, grpc, device, results, scores, nnz
+        self.var_names = var_names
 
 
 def check_flag(name: str, value) -> None:
@@ -221,18 +233,24 @@ def _host_fractions(run: _Run):
 
 def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, alternative, use_continuity, tie_correct,
                layer, device, devices, score: bool, on_device: bool, pts: bool = False, method: str = WILCOXON,
-               groups=None) -> _Run:
+               groups=None, mask_var=None) -> _Run:
     """Every (group, gene) test of ``adata``: validation, upload, group plan, one gene shard per GPU, batches, backed
     streaming.  ``on_device=False``: each shard's slabs are copied into pinned host arrays (``asymptotic_wilcoxon``).
     ``on_device=True``: they stay on the GPUs and meet in ``[G, N, 3]`` / ``[G, N]`` tensors on the first one
     (device-to-device copies; with one shard its own tensors are the result).  ``pts``: the count plane too.  ``method``:
     the Wilcoxon test or one of the t-tests (``Engine.run_batch``).  ``groups``: the groups to test (``asymptotic_wilcoxon``);
     one-versus-reference then runs on the rows of their cells (``rows``, with their own group container), one-versus-rest
-    on every cell with the other groups collapsed into pseudo-groups whose rows are dropped."""
+    on every cell with the other groups collapsed into pseudo-groups whose rows are dropped.  ``mask_var``: the genes to
+    test (``asymptotic_wilcoxon``); shards, batches and result planes then span the ``n_sel`` selected genes, and every
+    batch runs on a matrix that holds only their columns (``select.ColumnSelection``)."""
+    from .select import ColumnSelection, resolve_mask_var
+
     check_method(method)
     X = adata.layers[layer] if layer is not None else adata.X
     if isinstance(X, (sparse.csr_array, sparse.csc_array)):
         X = sparse.csr_matrix(X) if isinstance(X, sparse.csr_array) else sparse.csc_matrix(X)
+    cols = resolve_mask_var(adata, mask_var, X.shape[1])     # (a bad mask is refused before any device work)
+    colsel = ColumnSelection(cols, X.shape[1]) if cols is not None else None
     unique_raw_groups = grpc = rows = None
     if not (groups is None or (isinstance(groups, str) and groups == "all")):
         # the labels decide which rows go to the GPU: encode them first (and refuse a bad selection before any device work)
@@ -256,7 +274,7 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
         device = X.device          # a device-resident matrix is ranked where it lives
     seg_max = seg_max_from_env()   # an invalid ILLICO_B200_SEG_MAX fails before any device work
     devs = _device_list(device, devices)
-    n_cells, n_genes = X.shape
+    n_cells, n_genes = X.shape[0], (X.shape[1] if colsel is None else colsel.size)     # (genes of the run)
     fmt = data_handler.kernel_data_format().value
     flags_for = lambda: make_flags(is_log1p, use_continuity, tie_correct, alternative, fmt)  # noqa: E731
     flags_for()  # validates `alternative` before any work starts
@@ -280,7 +298,8 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
         if repartition.peer_access_ok([sh.device for sh in shards]):
             def _prep():
                 try:
-                    Ms = repartition.repartition_csr(X, [sh.device for sh in shards], [sh.lb for sh in shards] + [shards[-1].ub])
+                    Ms = repartition.repartition_csr(X, [sh.device for sh in shards], [sh.lb for sh in shards] + [shards[-1].ub],
+                                                     cols=colsel)
                     for sh, M in zip(shards, Ms):
                         sh.started = (M, (0, sh.ub - sh.lb))
                 except BaseException as e:
@@ -290,9 +309,12 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
             prep.start()
 
     def upload(sh: _Shard):
-        if selection is None:
-            return data_handler.upload_shard(sh.lb, sh.ub, sh.device)
-        return data_handler.upload_shard(sh.lb, sh.ub, sh.device, rows=selection.rows)
+        kw = {}
+        if selection is not None:
+            kw["rows"] = selection.rows
+        if colsel is not None:
+            kw["cols"] = colsel.cols[sh.lb:sh.ub]
+        return data_handler.upload_shard(sh.lb, sh.ub, sh.device, **kw)
 
     def run_shard(sh: _Shard):
         """Everything one GPU does, on its own host thread: upload its gene shard (started before the groups are
@@ -318,6 +340,10 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
                 nz = torch.empty((engine.n_groups, sh.ub - sh.lb), dtype=torch.int32, device=sh.device) if pts else None
                 if data_handler.in_ram:
                     M.ready()
+                    if colsel is not None:      # (a dense matrix: its row selection in the same pass)
+                        from .select import select_cols
+
+                        M, bounds = select_cols(M, bounds, colsel, sh.lb, sh.ub, selection)
                     if selection is not None:
                         from .select import select_rows
 
@@ -334,7 +360,8 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
                         engine.run_batch(M, lb + off, ub + off, flags, res, lb - sh.lb, scores=sc, nnz=nz, method=method)
                 else:
                     _run_backed(data_handler, _batches(sh.lb, sh.ub, batch_size, engine, False, method), engine, flags, res,
-                                max(1, int(n_threads)), gene0=sh.lb, scores=sc, nnz=nz, method=method, selection=selection)
+                                max(1, int(n_threads)), gene0=sh.lb, scores=sc, nnz=nz, method=method, selection=selection,
+                                columns=colsel)
                 if on_device and len(shards) == 1:
                     shared["out"], shared["out_scores"], shared["out_nnz"] = res, sc, nz
                 else:
@@ -395,7 +422,8 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
         out, scores = out.numpy(), (scores.numpy() if scores is not None else None)
         nnz = nnz.numpy() if nnz is not None else None
     S = len(unique_raw_groups)     # (fewer than G when one-versus-rest pseudo-groups follow the selected groups)
-    return _Run(unique_raw_groups, grpc, shards[0].device, out[:S], scores[:S] if scores is not None else None, nnz)
+    var_names = adata.var_names if colsel is None else adata.var_names[colsel.cols]
+    return _Run(unique_raw_groups, grpc, shards[0].device, out[:S], scores[:S] if scores is not None else None, nnz, var_names)
 
 
 def _encode_groups(adata, group_keys, reference, n_cells: int):
@@ -470,7 +498,7 @@ class _PinnedSlot:
 
 
 def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, results, n_readers: int, gene0: int = 0,
-                scores=None, nnz=None, method: str = WILCOXON, selection=None) -> None:
+                scores=None, nnz=None, method: str = WILCOXON, selection=None, columns=None) -> None:
     """Out-of-core input (BASELINE config 4): gene batches stream disk -> pinned ring -> HBM -> kernels.
 
     Reader threads slice the next batches from the backed container straight into pinned staging buffers (a ring of
@@ -478,7 +506,9 @@ def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, resu
     kernels on the compute stream, ordered by events, so the disk read and H2D copy of batch ``i + 1`` overlap the
     ranking of batch ``i`` (the reference's joblib threads overlap I/O and numba kernels the same way,
     ``asymptotic_wilcoxon.py:212-249``).  ``selection`` (``select.RowSelection``): only those rows are ranked -- the readers
-    gather them out of dense batches, CSC batches are compacted on the device (``illico_select_rows_csc``)."""
+    gather them out of dense batches, CSC batches are compacted on the device (``illico_select_rows_csc``).  ``columns``
+    (``select.ColumnSelection``): the batches are ranges of the selected genes, and the readers fetch each one's runs of
+    consecutive columns as slices (``ColumnSelection.fetch``)."""
     from .engine import DENSE, DeviceMatrix, _to_f32_or_wide
 
     dev = engine.device
@@ -512,7 +542,7 @@ def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, resu
             try:
                 if slot.copied is not None:
                     slot.copied.synchronize()   # the device is done reading this slot's previous batch
-                data, bounds = data_handler.fetch(lb, ub)
+                data, bounds = data_handler.fetch(lb, ub) if columns is None else columns.fetch(data_handler, lb, ub)
                 if fmt == DENSE:
                     if selection is not None:
                         data = np.take(data, selection.rows, axis=0)

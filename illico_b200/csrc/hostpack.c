@@ -16,14 +16,14 @@
 
 #define PREFETCH_AHEAD 4096
 
-static void scalar_words(const float* row, long c0, long c1, uint32_t* mask, float** out) {
-    /* columns [c0, c1) of one row, c0 a multiple of 32 */
+static void scalar_words(const float* row, const int32_t* cols, long c0, long c1, uint32_t* mask, float** out) {
+    /* columns [c0, c1) of one row (element k is row[cols[k]] with a column list), c0 a multiple of 32 */
     float* o = *out;
     for (long c = c0; c < c1; c += 32) {
         uint32_t m = 0;
         const long e = c + 32 < c1 ? c + 32 : c1;
         for (long k = c; k < e; ++k) {
-            const float v = row[k];
+            const float v = cols ? row[cols[k]] : row[k];
             if (v != 0.0f) { m |= 1u << (k - c); *o++ = v; }
         }
         mask[c >> 5] = m;
@@ -51,7 +51,28 @@ __attribute__((target("avx512f"))) static void row_avx512(const float* row, long
         mask[c >> 5] = (uint32_t)ma | ((uint32_t)mb << 16);
     }
     *out = o;
-    if (full < n_cols) scalar_words(row, full, n_cols, mask, out);
+    if (full < n_cols) scalar_words(row, NULL, full, n_cols, mask, out);
+}
+
+/* row_avx512 over the elements row[cols[k]]: the hardware gather loads them (cols ascend, so a gather's 16 lanes touch few
+ * cache lines), the squeeze is the same */
+__attribute__((target("avx512f"))) static void gather_avx512(const float* row, const int32_t* cols, long n_cols, uint32_t* mask,
+                                                            float** out) {
+    float* o = *out;
+    const __m512 zero = _mm512_setzero_ps();
+    const long full = n_cols & ~31L;
+    for (long c = 0; c < full; c += 32) {
+        const __m512 a = _mm512_i32gather_ps(_mm512_loadu_si512((const void*)(cols + c)), row, 4);
+        const __m512 b = _mm512_i32gather_ps(_mm512_loadu_si512((const void*)(cols + c + 16)), row, 4);
+        const __mmask16 ma = _mm512_cmp_ps_mask(a, zero, _CMP_NEQ_UQ), mb = _mm512_cmp_ps_mask(b, zero, _CMP_NEQ_UQ);
+        _mm512_storeu_ps(o, _mm512_maskz_compress_ps(ma, a));
+        o += __builtin_popcount((unsigned)ma);
+        _mm512_storeu_ps(o, _mm512_maskz_compress_ps(mb, b));
+        o += __builtin_popcount((unsigned)mb);
+        mask[c >> 5] = (uint32_t)ma | ((uint32_t)mb << 16);
+    }
+    *out = o;
+    if (full < n_cols) scalar_words(row, cols, full, n_cols, mask, out);
 }
 
 static int32_t g_perm[256][8];
@@ -85,7 +106,27 @@ __attribute__((target("avx2"))) static void row_avx2(const float* row, long n_co
         mask[c >> 5] = m;
     }
     *out = o;
-    if (full < n_cols) scalar_words(row, full, n_cols, mask, out);
+    if (full < n_cols) scalar_words(row, NULL, full, n_cols, mask, out);
+}
+
+__attribute__((target("avx2"))) static void gather_avx2(const float* row, const int32_t* cols, long n_cols, uint32_t* mask, float** out) {
+    float* o = *out;
+    const __m256 zero = _mm256_setzero_ps();
+    const long full = n_cols & ~31L;
+    for (long c = 0; c < full; c += 32) {
+        uint32_t m = 0;
+        for (int q = 0; q < 4; ++q) {
+            const __m256 v = _mm256_i32gather_ps(row, _mm256_loadu_si256((const __m256i*)(cols + c + 8 * q)), 4);
+            const int mm = _mm256_movemask_ps(_mm256_cmp_ps(v, zero, _CMP_NEQ_UQ));
+            const __m256i idx = _mm256_loadu_si256((const __m256i*)g_perm[mm]);
+            _mm256_storeu_ps(o, _mm256_permutevar8x32_ps(v, idx));
+            o += __builtin_popcount((unsigned)mm);
+            m |= (uint32_t)mm << (8 * q);
+        }
+        mask[c >> 5] = m;
+    }
+    *out = o;
+    if (full < n_cols) scalar_words(row, cols, full, n_cols, mask, out);
 }
 
 /* which code path this CPU takes: 2 = AVX-512, 1 = AVX2, 0 = scalar */
@@ -96,8 +137,8 @@ int illico_host_pack_isa(void) {
     return 0;
 }
 
-static long pack_rows(const float* src, long row_stride, const int64_t* rows, long n_rows, long n_cols, uint32_t* mask,
-                      uint32_t* row_off, float* vals, long vals_cap) {
+static long pack_rows(const float* src, long row_stride, const int64_t* rows, long n_rows, const int32_t* cols, long n_cols,
+                      uint32_t* mask, uint32_t* row_off, float* vals, long vals_cap) {
     const int isa = illico_host_pack_isa();
     if (isa == 1 && !g_perm_ready) build_perm();
     const long W = (n_cols + 31) / 32;
@@ -106,9 +147,13 @@ static long pack_rows(const float* src, long row_stride, const int64_t* rows, lo
         if ((o - vals) + n_cols + 16 > vals_cap) return -1;
         row_off[r] = (uint32_t)(o - vals);
         const float* row = src + (rows ? rows[r] : r) * row_stride;
-        if (isa == 2) row_avx512(row, n_cols, mask + r * W, &o);
+        if (cols) {
+            if (isa == 2) gather_avx512(row, cols, n_cols, mask + r * W, &o);
+            else if (isa == 1) gather_avx2(row, cols, n_cols, mask + r * W, &o);
+            else scalar_words(row, cols, 0, n_cols, mask + r * W, &o);
+        } else if (isa == 2) row_avx512(row, n_cols, mask + r * W, &o);
         else if (isa == 1) row_avx2(row, n_cols, mask + r * W, &o);
-        else scalar_words(row, 0, n_cols, mask + r * W, &o);
+        else scalar_words(row, NULL, 0, n_cols, mask + r * W, &o);
     }
     row_off[n_rows] = (uint32_t)(o - vals);
     return (long)(o - vals);
@@ -121,12 +166,20 @@ static long pack_rows(const float* src, long row_stride, const int64_t* rows, lo
  * Returns the number of values, or -1 when they do not fit (the caller then sends the chunk as it is). */
 long illico_host_pack_rows_f32(const float* src, long row_stride, long n_rows, long n_cols, uint32_t* mask, uint32_t* row_off,
                                float* vals, long vals_cap) {
-    return pack_rows(src, row_stride, NULL, n_rows, n_cols, mask, row_off, vals, vals_cap);
+    return pack_rows(src, row_stride, NULL, n_rows, NULL, n_cols, mask, row_off, vals, vals_cap);
 }
 
 /* The same for the rows rows[0 .. n_rows) of the matrix (any order; packed row r is source row rows[r]): the upload of the
  * cells of the groups a call tests gathers them while it squeezes them. */
 long illico_host_pack_row_list_f32(const float* src, long row_stride, const int64_t* rows, long n_rows, long n_cols, uint32_t* mask,
                                    uint32_t* row_off, float* vals, long vals_cap) {
-    return pack_rows(src, row_stride, rows, n_rows, n_cols, mask, row_off, vals, vals_cap);
+    return pack_rows(src, row_stride, rows, n_rows, NULL, n_cols, mask, row_off, vals, vals_cap);
+}
+
+/* The same for the columns cols[0 .. n_cols) of rows rows[0 .. n_rows) (rows [0, n_rows) when rows is NULL): packed row r
+ * holds src[rows[r], cols[k]] as its element k.  The upload of the genes a call tests (mask_var=) gathers them while it
+ * squeezes them, so that only their bytes cross PCIe. */
+long illico_host_pack_cols_f32(const float* src, long row_stride, const int64_t* rows, long n_rows, const int32_t* cols, long n_cols,
+                               uint32_t* mask, uint32_t* row_off, float* vals, long vals_cap) {
+    return pack_rows(src, row_stride, rows, n_rows, cols, n_cols, mask, row_off, vals, vals_cap);
 }

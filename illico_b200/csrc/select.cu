@@ -1,10 +1,13 @@
-// select.cu -- the cells of the groups a call tests (scanpy's rank_genes_groups(groups=...)), one-versus-reference (sm_100a).
+// select.cu -- the cells of the groups a call tests (scanpy's rank_genes_groups(groups=...)), one-versus-reference, and the
+// genes it tests (mask_var=) (sm_100a).
 //
 // A one-versus-reference test of a few groups needs only their cells and the reference's.  These kernels cut those rows
 // out of a device-resident matrix, keeping their ascending order, so that the group plan built from the same rows gives
 // every selected group the segments and summation order of the full call and the six dispatchers run unchanged on the
-// result.  Values are moved as bit patterns: float32 or float64 (a float64 matrix stays float64 and keeps going through the
-// recode path).  Every call only enqueues work on `stream`.
+// result.  A call that tests a subset of the genes needs only their columns: the dense gather takes a column list (and an
+// optional row list, in the same pass), and a CSR row is compacted through a new_col table by the CSC kernels with the
+// roles of rows and columns swapped.  Values are moved as bit patterns: float32 or float64 (a float64 matrix stays float64
+// and keeps going through the recode path).  Every call only enqueues work on `stream`.
 #include "common.cuh"
 
 namespace illico {
@@ -15,20 +18,22 @@ constexpr int SEL_THREADS = 256;
 constexpr int SEL_SCAN_THREADS = 1024;
 
 // One CTA per (output row, tile of 4 * 256 columns): the four loads of a thread are issued before its stores.  Columns
-// [n_cols, out_ld) of the output row are written as zeros (the padding that keeps rows 16-byte aligned).
-template <typename T>
-__global__ void __launch_bounds__(SEL_THREADS) select_rows_dense_kernel(const T* __restrict__ X, long long ld, long long n_cols,
-                                                                        const int32_t* __restrict__ rows, T* __restrict__ out,
-                                                                        long long out_ld) {
+// [n_cols, out_ld) of the output row are written as zeros (the padding that keeps rows 16-byte aligned).  ROWS: output row r
+// is source row rows[r] (else r).  COLS: output column c is source column cols[c] (else c); lane t of a warp reads the
+// t-th of 32 consecutive entries of the ascending list, so a warp's loads fall into as few sectors as the list allows.
+template <typename T, bool ROWS, bool COLS>
+__global__ void __launch_bounds__(SEL_THREADS) select_dense_kernel(const T* __restrict__ X, long long ld, long long n_cols,
+                                                                   const int32_t* __restrict__ rows, const int32_t* __restrict__ cols,
+                                                                   T* __restrict__ out, long long out_ld) {
     const long long r = blockIdx.x;
-    const T* src = X + (long long)rows[r] * ld;
+    const T* src = X + (ROWS ? (long long)rows[r] : r) * ld;
     T* dst = out + r * out_ld;
     const long long c0 = (long long)blockIdx.y * (4 * SEL_THREADS) + threadIdx.x;
     T v[4];
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
         const long long c = c0 + k * SEL_THREADS;
-        v[k] = c < n_cols ? src[c] : T(0);
+        v[k] = c < n_cols ? src[COLS ? (long long)__ldg(cols + c) : c] : T(0);
     }
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
@@ -162,6 +167,31 @@ int scan_lengths(long long* out_indptr, long long n, cudaStream_t st) {
     return 0;
 }
 
+template <typename T, bool ROWS, bool COLS>
+int launch_select_dense(const void* X, long long ld, long long n_cols, const int32_t* rows, const int32_t* cols, dim3 grid, void* out,
+                        long long out_ld, cudaStream_t st) {
+    ILLICO_LAUNCH("select_dense_kernel", st,
+                  (select_dense_kernel<T, ROWS, COLS><<<grid, SEL_THREADS, 0, st>>>((const T*)X, ld, n_cols, rows, cols, (T*)out, out_ld)));
+    ILLICO_CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
+// out[i, c] = X[rows ? rows[i] : i, cols ? cols[c] : c] for c < n_cols, zeros up to out_ld
+int select_dense(const void* X, int vb, long long ld, long long n_cols, const int32_t* rows, const int32_t* cols, long long n_rows,
+                 void* out, long long out_ld, cudaStream_t st, const char* who) {
+    const long long tiles = (out_ld + 4 * SEL_THREADS - 1) / (4 * SEL_THREADS);
+    if (tiles > 65535) { set_error("%s: rows wider than %d elements", who, 65535 * 4 * SEL_THREADS); return 1; }
+    const dim3 grid((unsigned)n_rows, (unsigned)tiles);
+    if (vb == 4) {
+        if (!cols) return launch_select_dense<float, true, false>(X, ld, n_cols, rows, cols, grid, out, out_ld, st);
+        if (rows) return launch_select_dense<float, true, true>(X, ld, n_cols, rows, cols, grid, out, out_ld, st);
+        return launch_select_dense<float, false, true>(X, ld, n_cols, rows, cols, grid, out, out_ld, st);
+    }
+    if (!cols) return launch_select_dense<double, true, false>(X, ld, n_cols, rows, cols, grid, out, out_ld, st);
+    if (rows) return launch_select_dense<double, true, true>(X, ld, n_cols, rows, cols, grid, out, out_ld, st);
+    return launch_select_dense<double, false, true>(X, ld, n_cols, rows, cols, grid, out, out_ld, st);
+}
+
 }  // namespace
 
 }  // namespace illico
@@ -178,18 +208,20 @@ extern "C" int illico_select_rows_dense(const void* X, int32_t dtype, int64_t ld
         return 1;
     }
     if (n_rows > 0x7fffffffLL) { set_error("illico_select_rows_dense: more than 2^31 - 1 rows"); return 1; }
-    const long long tiles = (out_ld + 4 * SEL_THREADS - 1) / (4 * SEL_THREADS);
-    if (tiles > 65535) { set_error("illico_select_rows_dense: rows wider than %d elements", 65535 * 4 * SEL_THREADS); return 1; }
-    cudaStream_t st = (cudaStream_t)stream;
-    const dim3 grid((unsigned)n_rows, (unsigned)tiles);
-    if (vb == 4)
-        ILLICO_LAUNCH("select_rows_dense_kernel", st,
-                      select_rows_dense_kernel<float><<<grid, SEL_THREADS, 0, st>>>((const float*)X, ld, n_cols, rows, (float*)out, out_ld));
-    else
-        ILLICO_LAUNCH("select_rows_dense_kernel", st,
-                      select_rows_dense_kernel<double><<<grid, SEL_THREADS, 0, st>>>((const double*)X, ld, n_cols, rows, (double*)out, out_ld));
-    ILLICO_CUDA_OK(cudaGetLastError());
-    return 0;
+    return select_dense(X, vb, ld, n_cols, rows, nullptr, n_rows, out, out_ld, (cudaStream_t)stream, "illico_select_rows_dense");
+}
+
+extern "C" int illico_select_cols_dense(const void* X, int32_t dtype, int64_t ld, const int32_t* rows, int64_t n_rows, const int32_t* cols,
+                                        int64_t n_cols, void* out, int64_t out_ld, void* stream) {
+    const int vb = value_bytes(dtype, "illico_select_cols_dense");
+    if (!vb) return 1;
+    if (n_rows <= 0 || out_ld <= 0) return 0;
+    if (!X || !out || n_cols < 0 || out_ld < n_cols || ld <= 0 || (n_cols > 0 && !cols)) {
+        set_error("illico_select_cols_dense: bad argument");
+        return 1;
+    }
+    if (n_rows > 0x7fffffffLL) { set_error("illico_select_cols_dense: more than 2^31 - 1 rows"); return 1; }
+    return select_dense(X, vb, ld, n_cols, rows, cols, n_rows, out, out_ld, (cudaStream_t)stream, "illico_select_cols_dense");
 }
 
 extern "C" int illico_select_rows_csr_indptr(const int64_t* indptr, const int32_t* rows, int64_t n_rows, int64_t* out_indptr,

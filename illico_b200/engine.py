@@ -398,11 +398,13 @@ def _torch_dtype(a: np.ndarray):
     return torch.from_numpy(np.empty(0, dtype=a.dtype)).dtype
 
 
-def upload_dense(X, device, gene_lb: int = 0, gene_ub: int | None = None, rows=None) -> DeviceMatrix:
+def upload_dense(X, device, gene_lb: int = 0, gene_ub: int | None = None, rows=None, cols=None) -> DeviceMatrix:
     """Starts the copy of ``X[:, gene_lb:gene_ub]`` (any real dtype) into a device matrix and returns at once: pinned
     sources go out as one strided asynchronous copy, pageable ones through the pinned staging ring of
     :mod:`illico_b200.hostio` (worker threads), so the caller keeps working on the host meanwhile.  ``rows`` (ascending
-    int64, optional): only those rows go up, gathered by the staging threads.  ``DeviceMatrix.ready()`` joins."""
+    int64, optional): only those rows go up, gathered by the staging threads.  ``cols`` (ascending int64, optional): the
+    columns of ``X`` that go up, gathered the same way, in place of ``[gene_lb, gene_ub)`` (genes ``[gene_lb, gene_ub)``
+    of a run over a column selection, ``gene_ub - gene_lb == len(cols)``).  ``DeviceMatrix.ready()`` joins."""
     from . import hostio
 
     device = require_cuda(device)
@@ -412,10 +414,16 @@ def upload_dense(X, device, gene_lb: int = 0, gene_ub: int | None = None, rows=N
     gene_ub = N if gene_ub is None else gene_ub
     if isinstance(X, torch.Tensor):
         X = X.numpy()
-    view = _uploadable(np.asarray(X[:, gene_lb:gene_ub]))
+    rel = None
+    if cols is not None:
+        c0 = int(cols[0])
+        view = _uploadable(np.asarray(X[:, c0:int(cols[-1]) + 1]))
+        rel = np.asarray(cols, dtype=np.int64) - c0
+    else:
+        view = _uploadable(np.asarray(X[:, gene_lb:gene_ub]))
     with torch.cuda.device(device):
         d = torch.empty((n, gene_ub - gene_lb), dtype=_torch_dtype(view), device=device)
-        pend = hostio.h2d_2d(d, view, rows=rows)
+        pend = hostio.h2d_2d(d, view, rows=rows, cols=rel)
     if d.dtype == torch.float32:
         return DeviceMatrix(DENSE, (n, gene_ub - gene_lb), d, gene_offset=gene_lb, pending=[pend])
     return DeviceMatrix(DENSE, (n, gene_ub - gene_lb), None, gene_offset=gene_lb, pending=[pend], unconverted=d)

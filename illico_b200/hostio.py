@@ -183,24 +183,33 @@ class Pending:
                 cur.wait_event(ev)
 
 
-def _gather(out: np.ndarray, src: np.ndarray, rows, r0: int, r1: int) -> None:
-    """``out[:] = src[r0:r1]``, or ``src[rows[r0:r1]]`` with a row list (numpy releases the GIL in both copy loops)."""
-    if rows is None:
+def _gather(out: np.ndarray, src: np.ndarray, rows, r0: int, r1: int, cols=None) -> None:
+    """``out[:] = src[r0:r1]``, or ``src[rows[r0:r1]]`` with a row list, then only the columns ``cols`` with a column list
+    (numpy releases the GIL in these copy loops)."""
+    if cols is not None:
+        block = src[r0:r1] if rows is None else np.take(src, rows[r0:r1], axis=0)
+        np.take(block, cols, axis=1, out=out, mode="clip")
+    elif rows is None:
         np.copyto(out, src[r0:r1])
     else:
         np.take(src, rows[r0:r1], axis=0, out=out, mode="clip")     # ("clip": the rows are valid; no buffered copy)
 
 
-def h2d_2d(dst: torch.Tensor, src: np.ndarray, n_threads: int | None = None, allow_pack: bool = True, rows=None) -> Pending:
+def h2d_2d(dst: torch.Tensor, src: np.ndarray, n_threads: int | None = None, allow_pack: bool = True, rows=None,
+           cols=None) -> Pending:
     """Starts the copy of the 2-D host array ``src`` (any row stride, unit column stride) into the contiguous device
     tensor ``dst`` of the same shape and dtype.  ``rows`` (int64, optional): only those rows of ``src``, in that order, go
     up -- the staging threads gather them, so the other rows never cross PCIe (``dst`` then has ``len(rows)`` rows).
-    Returns at once; see :class:`Pending`."""
+    ``cols`` (int64, optional): the same for columns (``dst`` then has ``len(cols)`` columns).  Returns at once; see
+    :class:`Pending`."""
     device = dst.device
     n, b = src.shape
     if rows is not None:
         rows = np.ascontiguousarray(rows, dtype=np.int64)
         n = rows.size
+    if cols is not None:
+        cols = np.ascontiguousarray(cols, dtype=np.int64)
+        b = cols.size
     item = src.dtype.itemsize
     assert dst.is_contiguous() and tuple(dst.shape) == (n, b) and dst.element_size() == item
     if n == 0 or b == 0:
@@ -209,14 +218,14 @@ def h2d_2d(dst: torch.Tensor, src: np.ndarray, n_threads: int | None = None, all
         src = np.ascontiguousarray(src)
     cur = torch.cuda.current_stream(device)
     row_bytes = b * item
-    pinned_src = is_pinned(src) and rows is None     # (a row list is gathered by the staging threads, never DMA'd as it is)
+    pinned_src = is_pinned(src) and rows is None and cols is None     # (a row or column list is gathered by the staging threads)
     # A pinned source is squeezed while this host feeds at most FOUR GPUs: plain DMA needs no CPU at all, but the links
     # of 2 / 4 GPUs together carry 111 / 115 GB/s on the measured box and its cores scan ~135 GB/s of raw matrix into an
     # eighth of the bytes (two ranks, each its own K562 matrix: 0.201 -> 0.140 s; one matrix split over two: 0.093 ->
     # 0.075 s); eight links carry 186 GB/s and win.  A pageable source has to be touched by the CPU anyway.
     feeding = int(os.environ.get("LOCAL_WORLD_SIZE", "1") or 1) * max(1, CONCURRENT_UPLOADS)
-    if allow_pack and (not pinned_src or feeding <= 4 or os.environ.get("ILLICO_PACK_UPLOAD") == "1") and _pack_wanted(src, n, b, rows):
-        return _h2d_2d_packed(dst, src, n_threads, rows)
+    if allow_pack and (not pinned_src or feeding <= 4 or os.environ.get("ILLICO_PACK_UPLOAD") == "1") and _pack_wanted(src, n, b, rows, cols):
+        return _h2d_2d_packed(dst, src, n_threads, rows, cols)
     if pinned_src:
         if src.strides[0] == b * item:      # contiguous: one linear asynchronous copy
             with warnings.catch_warnings():
@@ -226,7 +235,8 @@ def h2d_2d(dst: torch.Tensor, src: np.ndarray, n_threads: int | None = None, all
             copy2d_async(dst.data_ptr(), b * item, src.__array_interface__["data"][0], src.strides[0], b * item, n, "h2d", cur)
         return Pending(device)
     if n * row_bytes <= (4 << 20) or row_bytes > CHUNK_BYTES:   # small (or absurdly wide rows): the driver's own staged copy
-        dst.copy_(torch.from_numpy(np.ascontiguousarray(src if rows is None else src[rows])), non_blocking=True)
+        part = src if rows is None else src[rows]
+        dst.copy_(torch.from_numpy(np.ascontiguousarray(part if cols is None else part[:, cols])), non_blocking=True)
         return Pending(device)
     T = n_threads or stage_threads()
     rows_per_chunk = max(1, CHUNK_BYTES // row_bytes)
@@ -262,7 +272,7 @@ def h2d_2d(dst: torch.Tensor, src: np.ndarray, n_threads: int | None = None, all
                     buf = ring.slot(t, k)
                     view = buf[: (r1 - r0) * row_bytes]
                     hv = view.numpy().view(src.dtype).reshape(r1 - r0, b)
-                    _gather(hv, src, rows, r0, r1)     # GIL released inside; strided sources are gathered row by row
+                    _gather(hv, src, rows, r0, r1, cols)     # GIL released inside; strided sources are gathered row by row
                     with torch.cuda.stream(st):
                         dst_bytes[r0:r1].copy_(view.view(r1 - r0, row_bytes), non_blocking=True)
                         ev = torch.cuda.Event()
@@ -281,29 +291,34 @@ def h2d_2d(dst: torch.Tensor, src: np.ndarray, n_threads: int | None = None, all
 
 
 # ---- packed upload (float32, mostly zeros) -----------------------------------------------------------------------------
-def _pack_wanted(src: np.ndarray, n: int, b: int, rows=None) -> bool:
-    """A large float32 matrix (``n`` rows of ``src``, or ``src[rows]``) whose sampled rows are mostly zeros goes up packed
-    (``ILLICO_PACK_UPLOAD``: 0 never, 1 whenever the layout allows, default: when the sampled density is at most 0.3)."""
+def _pack_wanted(src: np.ndarray, n: int, b: int, rows=None, cols=None) -> bool:
+    """A large float32 matrix (``n`` rows of ``src``, or ``src[rows]``; its ``b`` columns, or ``cols``) whose sampled rows are
+    mostly zeros goes up packed (``ILLICO_PACK_UPLOAD``: 0 never, 1 whenever the layout allows, default: when the sampled
+    density is at most 0.3)."""
     mode = os.environ.get("ILLICO_PACK_UPLOAD", "auto")
     if mode == "0" or src.dtype != np.float32 or b < 64 or n * b * 4 < (64 << 20) or b * 4 > CHUNK_BYTES // 2:
         return False
     if mode == "1":
         return True
     picked = np.linspace(0, n - 1, num=min(n, 48), dtype=np.int64)
-    sample = src[picked if rows is None else rows[picked]][:, :: max(1, b // 2048)]                 # at most ~100k elements, spread over the matrix
+    step = max(1, b // 2048)                   # at most ~100k elements, spread over the matrix
+    sample = src[picked if rows is None else rows[picked]][:, slice(None, None, step) if cols is None else cols[::step]]
     return float(np.count_nonzero(sample)) <= 0.3 * sample.size
 
 
-def _h2d_2d_packed(dst: torch.Tensor, src: np.ndarray, n_threads: int | None, rows=None) -> Pending:
+def _h2d_2d_packed(dst: torch.Tensor, src: np.ndarray, n_threads: int | None, rows=None, cols=None) -> Pending:
     """The upload of a mostly-zero float32 matrix with the host threads squeezing the row chunks (bit mask + non-zero
     values, ``illico_host_pack_rows_f32``) instead of copying them: the packed chunk crosses PCIe (about 1/8 of the bytes
     at 10 % density) and ``illico_unpack_rows_f32`` rebuilds the rows in the destination.  The threads share one queue
-    of chunks.  With a row list (``rows``), chunk rows are ``src[rows[r0:r1]]`` (``illico_host_pack_row_list_f32``).  (A worker sending chunks of a pinned source as they are, beside the squeeze threads, measured slower on
-    the K562 matrix: the squeeze threads slow down ten-fold while plain DMA out of the same pinned pages is running;
+    of chunks.  With a row list (``rows``), chunk rows are ``src[rows[r0:r1]]`` (``illico_host_pack_row_list_f32``); with a
+    column list (``cols``), only those columns are squeezed (``illico_host_pack_cols_f32``).  (A worker sending chunks of a
+    pinned source as they are, beside the squeeze threads, measured slower on the K562 matrix: the squeeze threads slow
+    down ten-fold while plain DMA out of the same pinned pages is running;
     0.17 s against 0.10 s with the threads alone.)"""
     lib = _lib.load()
     device = dst.device
-    n, b = (src.shape[0] if rows is None else rows.size), src.shape[1]
+    n, b = (src.shape[0] if rows is None else rows.size), (src.shape[1] if cols is None else cols.size)
+    cols32 = None if cols is None else np.ascontiguousarray(cols, dtype=np.int32)
     W = (b + 31) // 32
     row_bytes = b * 4
     rows_per_chunk = max(1, CHUNK_BYTES // row_bytes)          # a chunk that does not squeeze still fits its buffer
@@ -349,7 +364,11 @@ def _h2d_2d_packed(dst: torch.Tensor, src: np.ndarray, n_threads: int | None, ro
                     buf = ring.slot(t, k)
                     base = buf.data_ptr()
                     off_bytes = nr * W * 4
-                    if rows is None:                # (ctypes releases the GIL)
+                    if cols32 is not None:          # (ctypes releases the GIL)
+                        nnz = lib.illico_host_pack_cols_f32(src_ptr if rows is not None else src_ptr + r0 * src_stride, src_stride // 4,
+                                                            rows[r0:r1].ctypes.data if rows is not None else None, nr,
+                                                            cols32.ctypes.data, b, base, base + off_bytes, base + hdr_bytes, vals_cap)
+                    elif rows is None:
                         nnz = lib.illico_host_pack_rows_f32(src_ptr + r0 * src_stride, src_stride // 4, nr, b, base, base + off_bytes,
                                                             base + hdr_bytes, vals_cap)
                     else:
@@ -367,7 +386,7 @@ def _h2d_2d_packed(dst: torch.Tensor, src: np.ndarray, n_threads: int | None, ro
                             stats["bytes"] += used
                         else:                     # a dense chunk: as it is
                             hv = buf[: nr * row_bytes].numpy().view(np.float32).reshape(nr, b)
-                            _gather(hv, src, rows, r0, r1)
+                            _gather(hv, src, rows, r0, r1, cols)
                             dst.view(torch.uint8).view(n, row_bytes)[r0:r1].copy_(buf[: nr * row_bytes].view(nr, row_bytes), non_blocking=True)
                             stats["raw"] += 1
                             stats["bytes"] += nr * row_bytes

@@ -58,6 +58,7 @@ def rank_genes(
     min_fold_change: float | None = None,
     method: str = "wilcoxon",
     groups=None,
+    mask_var=None,
 ) -> pd.DataFrame:
     """The ``n_genes`` strongest genes of every group, by Wilcoxon score (or Welch's t with ``method="t-test"``).
 
@@ -87,6 +88,10 @@ def rank_genes(
 
     ``groups`` is scanpy's (see ``asymptotic_wilcoxon``): only the selected groups are tested and shown, each with the rows
     it has in the same call without ``groups``.
+
+    ``mask_var`` is scanpy's (see ``asymptotic_wilcoxon``): only the selected genes are tested and ranked -- ``n_genes`` is
+    clipped to their number, ``feature`` is categorical over their names, and ``p_adj`` is over the selected genes of each
+    group.
     """
     check_method(method)
     if n_genes is not None:
@@ -100,11 +105,12 @@ def rank_genes(
     fc_min = _bound("min_fold_change", min_fold_change, None)
     with_pts = bool(pts) or any(v is not None for v in (min_in, max_out, fc_min))
     run = _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, alternative, use_continuity,
-                     tie_correct, layer, device, devices, score=True, on_device=True, pts=with_pts, method=method, groups=groups)
+                     tie_correct, layer, device, devices, score=True, on_device=True, pts=with_pts, method=method, groups=groups,
+                     mask_var=mask_var)
     res, scores = run.results, run.scores
     G, N = int(res.shape[0]), int(res.shape[1])
     k = N if n_genes is None else min(int(n_genes), N)
-    var_names = np.asarray(adata.var_names)
+    var_names = np.asarray(run.var_names)
     keep = np.arange(G)
     if reference is not None:
         keep = keep[keep != run.grpc.encoded_ref_group]

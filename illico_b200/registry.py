@@ -112,18 +112,21 @@ class InRAMDataHandler(DataHandler):
             self._resident = self.upload_shard(0, self.data.shape[1], getattr(engine, "device", engine))[0]
         return self._resident
 
-    def upload_shard(self, lb: int, ub: int, device, rows=None) -> tuple:
+    def upload_shard(self, lb: int, ub: int, device, rows=None, cols=None) -> tuple:
         """``(DeviceMatrix, (lb', ub'))``: genes ``[lb, ub)`` on ``device`` and their bounds inside that matrix.
         Returns as soon as the copies are started (``DeviceMatrix.ready()`` joins them).  ``rows`` (ascending int64): the
         cells a call needs; a handler that can gather them on the way up does, the others upload every row and the caller
-        selects them on the device (``select.select_rows``)."""
+        selects them on the device (``select.select_rows``).  ``cols`` (ascending int64, ``ub - lb`` of them): the columns
+        of genes ``[lb, ub)`` of a run over a column selection; a handler that can gather them on the way up returns a
+        matrix of exactly those columns, the others one holding a column range that contains them, which the caller cuts
+        on the device (``select.select_cols``)."""
         raise NotImplementedError
 
 
 @data_handler_registry.register(np.ndarray)
 class DenseDataHandler(InRAMDataHandler):
-    def upload_shard(self, lb, ub, device, rows=None):
-        return upload_dense(self.data, device, lb, ub, rows), (0, ub - lb)
+    def upload_shard(self, lb, ub, device, rows=None, cols=None):
+        return upload_dense(self.data, device, lb, ub, rows, cols), (0, ub - lb)
 
     def kernel_data_format(self):
         return KernelDataFormat.DENSE
@@ -134,9 +137,9 @@ class DenseDataHandler(InRAMDataHandler):
 
 @data_handler_registry.register(py_sparse.csr_matrix)
 class CSRDataHandler(InRAMDataHandler):
-    def upload_shard(self, lb, ub, device, rows=None):
+    def upload_shard(self, lb, ub, device, rows=None, cols=None):
         # every CSR row holds all genes: the whole matrix goes to each GPU over its own link (1.9 GB at the K562 shape)
-        # and the kernels select the gene range
+        # and the kernels select the gene range (with a column selection, the GPU compacts the rows first)
         return upload_sparse(self.data, CSR, device), (lb, ub)
 
     def kernel_data_format(self):
@@ -148,7 +151,9 @@ class CSRDataHandler(InRAMDataHandler):
 
 @data_handler_registry.register(py_sparse.csc_matrix)
 class CSCDataHandler(InRAMDataHandler):
-    def upload_shard(self, lb, ub, device, rows=None):
+    def upload_shard(self, lb, ub, device, rows=None, cols=None):
+        if cols is not None:        # the selected columns only (scipy's CSC column index copies them, indices unchanged)
+            return upload_sparse(self.data[:, cols], CSC, device), (0, ub - lb)
         return upload_sparse(self.data, CSC, device, lb, ub), (0, ub - lb)
 
     def kernel_data_format(self):
@@ -200,7 +205,7 @@ class TorchDenseDataHandler(InRAMDataHandler):
     """A 2-D ``torch.Tensor``: CUDA tensors are used where they are (no host round trip -- SURVEY section 8f.3), CPU
     tensors go through the ndarray path."""
 
-    def upload_shard(self, lb, ub, device, rows=None):
+    def upload_shard(self, lb, ub, device, rows=None, cols=None):
         import torch
 
         from .engine import _to_f32_or_wide
@@ -209,7 +214,7 @@ class TorchDenseDataHandler(InRAMDataHandler):
         if X.ndim != 2:
             raise ValueError("expression matrix must be two-dimensional")
         if not X.is_cuda:
-            return upload_dense(X.numpy(), device, lb, ub, rows), (0, ub - lb)
+            return upload_dense(X.numpy(), device, lb, ub, rows, cols), (0, ub - lb)
         want = torch.device(device)
         if want.type == "cuda" and want.index is None:
             want = torch.device("cuda", torch.cuda.current_device())
@@ -219,6 +224,9 @@ class TorchDenseDataHandler(InRAMDataHandler):
                 d = d.contiguous()
             return DeviceMatrix(DENSE, tuple(X.shape), d, raw=raw), (lb, ub)
         # another GPU's shard of a device-resident matrix: peer copy of the columns (NVLink), never a remote read by a kernel
+        # (with a column selection, the range that spans the shard's columns; the caller cuts them)
+        if cols is not None:
+            lb, ub = int(cols[0]), int(cols[-1]) + 1
         with torch.cuda.device(want):
             shard = X[:, lb:ub].to(want, non_blocking=True).contiguous()
         d, raw = (shard, None) if shard.dtype == torch.float32 else _to_f32_or_wide(shard)

@@ -39,9 +39,11 @@ def row_blocks(indptr: np.ndarray, k: int) -> list:
     return [(int(edges[i]), int(edges[i + 1])) for i in range(k)]
 
 
-def repartition_csr(X, devices, gene_bounds) -> list:
+def repartition_csr(X, devices, gene_bounds, cols=None) -> list:
     """``X``: scipy CSR (float32-exact values); ``devices[j]`` gets genes ``[gene_bounds[j], gene_bounds[j + 1])`` of every
-    row as a :class:`DeviceMatrix` (columns rebased to the shard).  Raises ``ValueError`` for unsorted row indices."""
+    row as a :class:`DeviceMatrix` (columns rebased to the shard).  Raises ``ValueError`` for unsorted row indices.
+    ``cols`` (``select.ColumnSelection``): the genes are those of the selection -- each GPU compacts its row block to the
+    selected columns (``select.compact``) before it counts and cuts it, so ``gene_bounds`` are in the selected-gene space."""
     import os
     import time
 
@@ -96,6 +98,11 @@ def repartition_csr(X, devices, gene_bounds) -> list:
                 _lib.check(1, "illico_check_csr_sorted")
             if sorted_ != 1:
                 raise ValueError(UNSORTED)
+            if cols is not None:
+                from .select import compact
+
+                new_col = torch.from_numpy(cols.new_col()).to(s["dev"], non_blocking=True)
+                s["ptr"], s["data"], s["idx"] = compact(s["data"], _lib.DTYPE_F32, s["idx"], s["ptr"].data_ptr(), nr, new_col)
             _lib.check(lib.illico_csr_shard_count(s["idx"].data_ptr(), s["ptr"].data_ptr(), nr, s["bounds"].data_ptr(), S,
                                                   s["cnt"].data_ptr(), s["totals"].data_ptr(), stream), "illico_csr_shard_count")
     lap("uploads started and joined, counts enqueued")

@@ -38,6 +38,7 @@ def ttest(
     score: bool = False,
     pts: bool = False,
     groups=None,
+    mask_var=None,
 ):
     """Welch's t-test of every group against ``reference`` (or, when it is None, against all other cells) in every gene.
 
@@ -52,14 +53,15 @@ def ttest(
     of ``expm1(x)`` when ``is_log1p``; ``inf`` where the comparison mean is 0).  The reference group's rows are
     ``(1, 0, fold change of the control with itself)``.  ``is_log1p`` affects only the fold change.
     ``score`` adds t with NaN replaced by 0 (scanpy's ``scores``); ``p_adjust``, ``log2_fold_change``, ``pts``,
-    ``return_array``, ``device``, ``devices``, ``n_threads``, ``batch_size``, ``layer`` and ``groups`` are those of
-    ``asymptotic_wilcoxon``.
+    ``return_array``, ``device``, ``devices``, ``n_threads``, ``batch_size``, ``layer``, ``groups`` and ``mask_var`` are
+    those of ``asymptotic_wilcoxon``.
     """
     if check_method(method) == WILCOXON:
         raise ValueError("ttest runs the t-tests; method='wilcoxon' is asymptotic_wilcoxon")
     check_flag("pts", pts)
     run = _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, alternative, True, True, layer, device,
-                     devices, score=score, on_device=False, pts=pts, method=method, groups=groups)
+                     devices, score=score, on_device=False, pts=pts, method=method, groups=groups,
+                     mask_var=mask_var)
     out = run.results
     extra = {}
     if p_adjust:
@@ -73,6 +75,6 @@ def ttest(
         extra["pct_nz_group"], extra["pct_nz_reference"] = _host_fractions(run)
     if return_array:
         if extra:
-            return run.groups, np.asarray(adata.var_names), out, extra
-        return run.groups, np.asarray(adata.var_names), out
-    return _result_frame(run.groups, adata.var_names, out, extra)
+            return run.groups, np.asarray(run.var_names), out, extra
+        return run.groups, np.asarray(run.var_names), out
+    return _result_frame(run.groups, run.var_names, out, extra)

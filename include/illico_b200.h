@@ -290,11 +290,15 @@ long illico_host_pack_rows_f32(const float* src, long row_stride, long n_rows, l
 /* The same for source rows rows[0 .. n_rows) (host int64 array): packed row r is row rows[r] of src. */
 long illico_host_pack_row_list_f32(const float* src, long row_stride, const int64_t* rows, long n_rows, long n_cols, uint32_t* mask,
                                    uint32_t* row_off, float* vals, long vals_cap);
+/* The same for the columns cols[0 .. n_cols) (host int32 array, any order) of rows rows[0 .. n_rows), or of rows [0, n_rows) when
+ * rows is NULL: the output is the pack of the contiguous matrix src[rows][:, cols]. */
+long illico_host_pack_cols_f32(const float* src, long row_stride, const int64_t* rows, long n_rows, const int32_t* cols, long n_cols,
+                               uint32_t* mask, uint32_t* row_off, float* vals, long vals_cap);
 int illico_host_pack_isa(void);
 int illico_unpack_rows_f32(const uint32_t* mask, const uint32_t* row_off, const float* vals, int64_t n_rows, int32_t n_cols,
                            float* dst, int64_t dst_ld, void* stream);
 
-/* ---- the cells of the groups a call tests (groups=, one-versus-reference) -----------------------------------------------
+/* ---- the cells of the groups a call tests (groups=, one-versus-reference) and the genes it tests (mask_var=) --------------
  * Row selection of a device-resident matrix, rows kept in the order given (the caller passes them ascending, so that every
  * group keeps the order of its cells).  `dtype` is ILLICO_DTYPE_F32 or ILLICO_DTYPE_F64; values are copied bit for bit.
  *   illico_select_rows_dense       out[i, c] = X[rows[i], c] for c < n_cols, 0 for n_cols <= c < out_ld (row padding); X of
@@ -308,9 +312,15 @@ int illico_unpack_rows_f32(const uint32_t* mask, const uint32_t* row_off, const 
  *                                  -1 = dropped).
  *   illico_select_rows_csc         those entries at out_indptr[c], rows renumbered through new_row, in their order (a stable
  *                                  compaction: each column's rows still ascend).
+ *   illico_select_cols_dense       out[i, c] = X[rows[i], cols[c]] for c < n_cols (X[i, cols[c]] when rows is NULL), 0 for
+ *                                  n_cols <= c < out_ld; X of row stride ld.  One pass for a column list and a row list.
+ * The CSC pair also compacts the columns of a CSR matrix: pass its row pointer as `indptr`, its row count as `n_cols` and a
+ * new_col [n_genes] table as `new_row`; each row keeps the entries of the kept columns, renumbered, still ascending.
  * No workspace; the scans run in place on out_indptr. */
 int illico_select_rows_dense(const void* X, int32_t dtype, int64_t ld, int64_t n_cols, const int32_t* rows, int64_t n_rows,
                              void* out, int64_t out_ld, void* stream);
+int illico_select_cols_dense(const void* X, int32_t dtype, int64_t ld, const int32_t* rows, int64_t n_rows, const int32_t* cols,
+                             int64_t n_cols, void* out, int64_t out_ld, void* stream);
 int illico_select_rows_csr_indptr(const int64_t* indptr, const int32_t* rows, int64_t n_rows, int64_t* out_indptr, void* stream);
 int illico_select_rows_csr(const void* data, int32_t dtype, const int32_t* indices, const int64_t* indptr, const int32_t* rows,
                            int64_t n_rows, const int64_t* out_indptr, void* out_data, int32_t* out_indices, void* stream);
