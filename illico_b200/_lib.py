@@ -114,6 +114,13 @@ SIGNATURES = {
     "illico_group_moments_dense": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _PP, _i32, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
     "illico_group_moments_csr": (C.c_int, [_vp, _i32, _vp, _vp, _i32, _i32, _PP, _i32, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
     "illico_group_moments_csc": (C.c_int, [_vp, _i32, _vp, _vp, _i32, _i32, _PP, _i32, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
+    "illico_group_sums_dense": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _PP, _vp, _vp, _i64, _i64, _vp]),
+    "illico_group_sums_csr": (C.c_int, [_vp, _i32, _vp, _vp, _i32, _i32, _PP, _vp, _vp, _i64, _i64, _vp]),
+    "illico_group_sums_csc": (C.c_int, [_vp, _i32, _vp, _vp, _i32, _i32, _PP, _vp, _vp, _i64, _i64, _vp]),
+    "illico_log_fold_changes": (C.c_int, [_vp, _i64, _vp, _i32, _i32, _i32, _i64, C.c_double, _vp, _i64, _vp]),
+    "illico_bonferroni_adjust": (C.c_int, [_vp, _i64, _i64, _i32, _i32, _vp, _vp]),
+    "illico_top_genes_columns": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _vp, _i64, _i32, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _vp,
+                                           _vp, _vp, _vp, _sz, _vp]),
     "illico_welch_ttest": (C.c_int, [_vp, _vp, _vp, _i64, _vp, _i32, _i32, _i32, _i64, _i32, _i32, _vp, _i64, _vp, _i64, _vp]),
     "illico_student_t_batch": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _vp]),
     "illico_compute_pval_batch": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),

@@ -31,15 +31,16 @@ from .registry import DataHandler, data_handler_registry
 __all__ = ["asymptotic_wilcoxon"]
 
 
-def _batches(lb: int, ub: int, batch_size, engine: Engine, in_ram: bool, method: str = WILCOXON):
+def _batches(lb: int, ub: int, batch_size, engine: Engine, in_ram: bool, method: str = WILCOXON, lfc: bool = False):
     """Gene batches of the shard ``[lb, ub)`` (global gene indices)."""
     n_genes = ub - lb
+    kw = {"lfc": True} if lfc else {}
     if isinstance(batch_size, (int, np.integer)) and not isinstance(batch_size, bool):
         if batch_size <= 0:
             raise ValueError(f"Invalid batch_size value: {batch_size}. Must be 'auto' or an integer.")
-        step = min(int(batch_size), engine.max_batch_genes(n_genes, method))
+        step = min(int(batch_size), engine.max_batch_genes(n_genes, method, **kw))
     elif batch_size == "auto":
-        step = engine.max_batch_genes(n_genes, method)
+        step = engine.max_batch_genes(n_genes, method, **kw)
         if not in_ram:
             step = min(step, 256)  # backed data: stream ~256 genes at a time like the reference aims for
     else:
@@ -186,11 +187,12 @@ class _Run:
     unless asked for) -- pinned host arrays, or tensors on that GPU.  With ``groups=`` one-versus-rest, the container and
     the count plane also hold the pseudo-groups of the cells of the other groups (``G' > G``: rows ``G ..``), which the
     fractions of the rest need; the results and scores hold the selected groups only.  ``var_names``: the names of the
-    ``N`` genes tested (``adata.var_names``, or its selected entries with ``mask_var=``)."""
+    ``N`` genes tested (``adata.var_names``, or its selected entries with ``mask_var=``).  ``lfc``: scanpy's log fold change
+    plane ``[G, N]`` float64 (None unless asked for), laid out like the scores."""
 
-    def __init__(self, groups, grpc, device, results, scores, nnz=None, var_names=None):
+    def __init__(self, groups, grpc, device, results, scores, nnz=None, var_names=None, lfc=None):
         self.groups, self.grpc, self.device, self.results, self.scores, self.nnz = groups, grpc, device, results, scores, nnz
-        self.var_names = var_names
+        self.var_names, self.lfc = var_names, lfc
 
 
 def check_flag(name: str, value) -> None:
@@ -233,7 +235,7 @@ def _host_fractions(run: _Run):
 
 def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, alternative, use_continuity, tie_correct,
                layer, device, devices, score: bool, on_device: bool, pts: bool = False, method: str = WILCOXON,
-               groups=None, mask_var=None) -> _Run:
+               groups=None, mask_var=None, lfc: bool = False, log_scale: float = 1.0) -> _Run:
     """Every (group, gene) test of ``adata``: validation, upload, group plan, one gene shard per GPU, batches, backed
     streaming.  ``on_device=False``: each shard's slabs are copied into pinned host arrays (``asymptotic_wilcoxon``).
     ``on_device=True``: they stay on the GPUs and meet in ``[G, N, 3]`` / ``[G, N]`` tensors on the first one
@@ -242,7 +244,8 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
     one-versus-reference then runs on the rows of their cells (``rows``, with their own group container), one-versus-rest
     on every cell with the other groups collapsed into pseudo-groups whose rows are dropped.  ``mask_var``: the genes to
     test (``asymptotic_wilcoxon``); shards, batches and result planes then span the ``n_sel`` selected genes, and every
-    batch runs on a matrix that holds only their columns (``select.ColumnSelection``)."""
+    batch runs on a matrix that holds only their columns (``select.ColumnSelection``).  ``lfc``: scanpy's log fold change
+    plane too (``Engine.run_batch(lfc=, log_scale=)``), allocated, sharded and gathered like the score plane."""
     from .select import ColumnSelection, resolve_mask_var
 
     check_method(method)
@@ -338,6 +341,7 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
                 res = torch.empty((engine.n_groups, sh.ub - sh.lb, 3), dtype=torch.float64, device=sh.device)
                 sc = torch.empty((engine.n_groups, sh.ub - sh.lb), dtype=torch.float64, device=sh.device) if score else None
                 nz = torch.empty((engine.n_groups, sh.ub - sh.lb), dtype=torch.int32, device=sh.device) if pts else None
+                lf = torch.empty((engine.n_groups, sh.ub - sh.lb), dtype=torch.float64, device=sh.device) if lfc else None
                 if data_handler.in_ram:
                     M.ready()
                     if colsel is not None:      # (a dense matrix: its row selection in the same pass)
@@ -356,14 +360,15 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
                             "prior to computing DE genes."
                         )
                     off = bounds[0] - sh.lb      # gene g of the run is column g + off of the device matrix
-                    for lb, ub in _batches(sh.lb, sh.ub, batch_size, engine, True, method):
-                        engine.run_batch(M, lb + off, ub + off, flags, res, lb - sh.lb, scores=sc, nnz=nz, method=method)
+                    for lb, ub in _batches(sh.lb, sh.ub, batch_size, engine, True, method, lfc):
+                        engine.run_batch(M, lb + off, ub + off, flags, res, lb - sh.lb, scores=sc, nnz=nz, method=method, lfc=lf,
+                                         log_scale=log_scale)
                 else:
-                    _run_backed(data_handler, _batches(sh.lb, sh.ub, batch_size, engine, False, method), engine, flags, res,
+                    _run_backed(data_handler, _batches(sh.lb, sh.ub, batch_size, engine, False, method, lfc), engine, flags, res,
                                 max(1, int(n_threads)), gene0=sh.lb, scores=sc, nnz=nz, method=method, selection=selection,
-                                columns=colsel)
+                                columns=colsel, lfc=lf, log_scale=log_scale)
                 if on_device and len(shards) == 1:
-                    shared["out"], shared["out_scores"], shared["out_nnz"] = res, sc, nz
+                    shared["out"], shared["out_scores"], shared["out_nnz"], shared["out_lfc"] = res, sc, nz, lf
                 else:
                     kind = "d2d" if on_device else "d2h"
                     hostio.d2h_slab(shared["out"], res, sh.lb, kind)
@@ -371,6 +376,8 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
                         hostio.d2h_slab(shared["out_scores"], sc, sh.lb, kind)
                     if nz is not None:
                         hostio.d2h_slab(shared["out_nnz"], nz, sh.lb, kind)
+                    if lf is not None:
+                        hostio.d2h_slab(shared["out_lfc"], lf, sh.lb, kind)
                 torch.cuda.current_stream(sh.device).synchronize()
         except BaseException as e:  # re-raised on the calling thread
             sh.error = e
@@ -398,10 +405,12 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
             shared["out"] = torch.empty((G, n_genes, 3), dtype=torch.float64, pin_memory=True)
             shared["out_scores"] = torch.empty((G, n_genes), dtype=torch.float64, pin_memory=True) if score else None
             shared["out_nnz"] = torch.empty((G, n_genes), dtype=torch.int32, pin_memory=True) if pts else None
+            shared["out_lfc"] = torch.empty((G, n_genes), dtype=torch.float64, pin_memory=True) if lfc else None
         elif len(shards) > 1:
             shared["out"] = torch.empty((G, n_genes, 3), dtype=torch.float64, device=devs[0])
             shared["out_scores"] = torch.empty((G, n_genes), dtype=torch.float64, device=devs[0]) if score else None
             shared["out_nnz"] = torch.empty((G, n_genes), dtype=torch.int32, device=devs[0]) if pts else None
+            shared["out_lfc"] = torch.empty((G, n_genes), dtype=torch.float64, device=devs[0]) if lfc else None
     except BaseException:
         shared["error"] = True
         plan_ready.set()
@@ -417,13 +426,15 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
     for sh in shards:
         if sh.error is not None:
             raise sh.error
-    out, scores, nnz = shared["out"], shared["out_scores"], shared.get("out_nnz")
+    out, scores, nnz, lfcs = shared["out"], shared["out_scores"], shared.get("out_nnz"), shared.get("out_lfc")
     if not on_device:
         out, scores = out.numpy(), (scores.numpy() if scores is not None else None)
         nnz = nnz.numpy() if nnz is not None else None
+        lfcs = lfcs.numpy() if lfcs is not None else None
     S = len(unique_raw_groups)     # (fewer than G when one-versus-rest pseudo-groups follow the selected groups)
     var_names = adata.var_names if colsel is None else adata.var_names[colsel.cols]
-    return _Run(unique_raw_groups, grpc, shards[0].device, out[:S], scores[:S] if scores is not None else None, nnz, var_names)
+    return _Run(unique_raw_groups, grpc, shards[0].device, out[:S], scores[:S] if scores is not None else None, nnz, var_names,
+                lfcs[:S] if lfcs is not None else None)
 
 
 def _encode_groups(adata, group_keys, reference, n_cells: int):
@@ -498,7 +509,7 @@ class _PinnedSlot:
 
 
 def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, results, n_readers: int, gene0: int = 0,
-                scores=None, nnz=None, method: str = WILCOXON, selection=None, columns=None) -> None:
+                scores=None, nnz=None, method: str = WILCOXON, selection=None, columns=None, lfc=None, log_scale: float = 1.0) -> None:
     """Out-of-core input (BASELINE config 4): gene batches stream disk -> pinned ring -> HBM -> kernels.
 
     Reader threads slice the next batches from the backed container straight into pinned staging buffers (a ring of
@@ -593,7 +604,8 @@ def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, resu
                 from .select import select_rows
 
                 M, bounds = select_rows(M, bounds, selection)
-        engine.run_batch(M, bounds[0], bounds[1], flags, results, lb - gene0, scores=scores, nnz=nnz, method=method)
+        engine.run_batch(M, bounds[0], bounds[1], flags, results, lb - gene0, scores=scores, nnz=nnz, method=method, lfc=lfc,
+                         log_scale=log_scale)
 
     try:
         while done < n_readers:

@@ -9,6 +9,9 @@
 //                              the gene index) and gathers the first k genes' records: scanpy's rank_genes_groups order.
 //   illico_top_genes_filtered  the same ranking with scanpy's filter_rank_genes_groups criteria applied first (dropped genes
 //                              sort after every kept one) and the expressing-cell fractions in the record.
+//   illico_bonferroni_adjust   Bonferroni adjusted p-values, min(p * n_genes, 1) (scanpy's corr_method="bonferroni").
+//   illico_top_genes_columns   illico_top_genes' ranking written column-major in scanpy's record layout ([k, groups]
+//                              planes of gene index, float32 score / log fold change, float64 p / p_adj).
 //   illico_compute_pval_batch  evaluates the epilogue's compute_pval (epilogue.cuh; reference illico/utils/math.py:64-118)
 //                              on arrays of arguments, so the known-answer vectors of tests/golden/primitives.npz can be
 //                              checked against the device code itself.
@@ -91,6 +94,16 @@ __global__ void __launch_bounds__(BH_THREADS) bh_adjust_kernel(const double* __r
     }
 }
 
+// A thread per test: p * n_genes clipped at 1, NaN kept (np.minimum(p * n_genes, 1.0))
+__global__ void __launch_bounds__(256) bonferroni_kernel(const double* __restrict__ p, long long group_stride, long long gene_stride,
+                                                         int G, int N, double* __restrict__ padj) {
+    const long long i = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (i >= (long long)G * N) return;
+    const int g = (int)(i / N), j = (int)(i - (long long)g * N);
+    const double v = __dmul_rn(p[(long long)g * group_stride + (long long)j * gene_stride], (double)N);
+    padj[i] = (v > 1.0) ? 1.0 : v;
+}
+
 // Per-group ranking (illico_top_genes, illico_top_genes_filtered): one CTA per group (grid-strided), like bh_adjust_kernel.
 // The key of gene j is the order-preserving u64 image of its score, complemented so that an ascending sort puts the largest
 // score first.  NaN keys come after every number (~0 - 1: no number's key is above -inf's 0xFFF0...0) and the keys of
@@ -115,11 +128,27 @@ struct TopFilter {
     int rec_w;
 };
 
+// The column-major outputs of illico_top_genes_columns: output column c is group rows[c] (rows NULL: group c), rank r of
+// it goes to element r * n_cols + c of each plane; lfc (NULL: NaN) is read at g * lfc_stride + j.
+struct TopColumns {
+    const int32_t* rows;
+    int n_cols;
+    const double* lfc;
+    long long lfc_stride;
+    float* score;
+    float* lfc_out;
+    double* p;
+    double* p_adj;
+};
+
+// COLS = false: records [G, k, rec_w] (illico_top_genes, illico_top_genes_filtered); COLS = true: TopColumns' planes, no
+// filter.  The keys and the sort are the same.
+template <bool COLS>
 __global__ void __launch_bounds__(BH_THREADS) top_genes_kernel(const double* __restrict__ score, long long score_stride,
                                                                const double* __restrict__ res, long long res_stride,
                                                                const double* __restrict__ padj, int G, int N, int k, int by_abs,
                                                                TopFilter F, int* __restrict__ out_gene, double* __restrict__ out_rec,
-                                                               unsigned long long* __restrict__ slab) {
+                                                               unsigned long long* __restrict__ slab, TopColumns O) {
     __shared__ uint32_t hist[BH_NW * 256];
     __shared__ uint32_t aux[RADIX_AUX_WORDS];
     __shared__ int n_kept;
@@ -129,7 +158,9 @@ __global__ void __launch_bounds__(BH_THREADS) top_genes_kernel(const double* __r
     uint32_t* IA = reinterpret_cast<uint32_t*>(B + N);
     uint32_t* IB = IA + N;
     const bool by_in = F.min_in == F.min_in, by_out = F.max_out == F.max_out, by_fc = F.fc_lo == F.fc_lo || F.fc_hi == F.fc_hi;
-    for (int g = blockIdx.x; g < G; g += gridDim.x) {
+    const int n_out = COLS ? O.n_cols : G;
+    for (int oc = blockIdx.x; oc < n_out; oc += gridDim.x) {
+        const int g = (COLS && O.rows) ? O.rows[oc] : oc;
         const double* sg = score + (long long)g * score_stride;
         const double* rg = res + (long long)g * res_stride;
         const long long plane = (long long)g * N;
@@ -153,24 +184,36 @@ __global__ void __launch_bounds__(BH_THREADS) top_genes_kernel(const double* __r
         const unsigned long long* S = block_radix_sort_t<unsigned long long, uint32_t>(A, B, N, hist, aux, IA, IB);
         const uint32_t* idx = (S == A) ? IA : IB;
         const int m = min(k, n_kept);
-        for (int r = tid; r < k; r += BH_THREADS) {
-            const long long o = (long long)g * k + r;
-            double* rec = out_rec + o * F.rec_w;
-            if (r >= m) {                                               // fewer than k genes kept
-                out_gene[o] = -1;
-                for (int f = 0; f < F.rec_w; ++f) rec[f] = NAN;
-                continue;
+        if constexpr (COLS) {
+            for (int r = tid; r < k; r += BH_THREADS) {                // (no filter: every gene is kept, m == k)
+                const long long o = (long long)r * O.n_cols + oc;
+                const int j = (int)idx[r];
+                out_gene[o] = j;
+                O.score[o] = (float)sg[j];
+                O.lfc_out[o] = O.lfc ? (float)O.lfc[(long long)g * O.lfc_stride + j] : NAN;
+                O.p[o] = rg[3 * (long long)j];
+                O.p_adj[o] = padj ? padj[plane + j] : NAN;
             }
-            const int j = (int)idx[r];
-            out_gene[o] = j;
-            rec[0] = sg[j];
-            rec[1] = rg[3 * (long long)j];
-            rec[2] = rg[3 * (long long)j + 1];
-            rec[3] = rg[3 * (long long)j + 2];
-            rec[4] = padj ? padj[plane + j] : NAN;
-            if (F.rec_w == 7) {
-                rec[5] = F.pct_group ? F.pct_group[plane + j] : NAN;
-                rec[6] = F.pct_ref ? F.pct_ref[plane + j] : NAN;
+        } else {
+            for (int r = tid; r < k; r += BH_THREADS) {
+                const long long o = (long long)g * k + r;
+                double* rec = out_rec + o * F.rec_w;
+                if (r >= m) {                                           // fewer than k genes kept
+                    out_gene[o] = -1;
+                    for (int f = 0; f < F.rec_w; ++f) rec[f] = NAN;
+                    continue;
+                }
+                const int j = (int)idx[r];
+                out_gene[o] = j;
+                rec[0] = sg[j];
+                rec[1] = rg[3 * (long long)j];
+                rec[2] = rg[3 * (long long)j + 1];
+                rec[3] = rg[3 * (long long)j + 2];
+                rec[4] = padj ? padj[plane + j] : NAN;
+                if (F.rec_w == 7) {
+                    rec[5] = F.pct_group ? F.pct_group[plane + j] : NAN;
+                    rec[6] = F.pct_ref ? F.pct_ref[plane + j] : NAN;
+                }
             }
         }
         if (tid == 0 && F.kept) F.kept[g] = n_kept;
@@ -266,8 +309,9 @@ static int launch_top_genes(const char* who, const double* scores, int64_t score
         reinterpret_cast<unsigned long long*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
     cudaStream_t st = (cudaStream_t)stream;
     ILLICO_LAUNCH("top_genes_kernel", st,
-                  top_genes_kernel<<<ctas, BH_THREADS, 0, st>>>(scores, score_group_stride, results, result_group_stride, p_adj,
-                                                                n_groups, n_genes, k, by_abs ? 1 : 0, F, out_gene, out_rec, slab));
+                  top_genes_kernel<false><<<ctas, BH_THREADS, 0, st>>>(scores, score_group_stride, results, result_group_stride,
+                                                                       p_adj, n_groups, n_genes, k, by_abs ? 1 : 0, F, out_gene, out_rec,
+                                                                       slab, TopColumns{}));
     ILLICO_CUDA_OK(cudaGetLastError());
     return 0;
 }
@@ -292,6 +336,49 @@ int illico_top_genes_filtered(const double* scores, int64_t score_group_stride, 
     const TopFilter F{pct_group, pct_ref, min_in_group, max_out_group, fc_min, fc_max, kept, 7};
     return launch_top_genes("illico_top_genes_filtered", scores, score_group_stride, results, result_group_stride, p_adj, n_groups,
                             n_genes, k, by_abs, F, out_gene, out_rec, workspace, workspace_bytes, stream);
+}
+
+int illico_bonferroni_adjust(const double* p_values, int64_t group_stride, int64_t gene_stride, int32_t n_groups, int32_t n_genes,
+                             double* p_adj, void* stream) {
+    if (!p_values || !p_adj) { set_error("illico_bonferroni_adjust: NULL argument"); return 1; }
+    if (n_groups <= 0 || n_genes <= 0) return 0;
+    const long long tests = (long long)n_groups * n_genes;
+    cudaStream_t st = (cudaStream_t)stream;
+    ILLICO_LAUNCH("bonferroni_kernel", st,
+                  bonferroni_kernel<<<(unsigned)((tests + 255) / 256), 256, 0, st>>>(p_values, group_stride, gene_stride, n_groups,
+                                                                                   n_genes, p_adj));
+    ILLICO_CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
+int illico_top_genes_columns(const double* scores, int64_t score_group_stride, const double* results, int64_t result_group_stride,
+                             const double* p_adj, const double* lfc, int64_t lfc_group_stride, int32_t n_groups, int32_t n_genes,
+                             const int32_t* group_rows, int32_t n_cols, int32_t k, int32_t by_abs, int32_t* out_gene, float* out_score,
+                             float* out_lfc, double* out_p, double* out_p_adj, void* workspace, size_t workspace_bytes, void* stream) {
+    const char* who = "illico_top_genes_columns";
+    if (!scores || !results || !out_gene || !out_score || !out_lfc || !out_p || !out_p_adj || !workspace) {
+        set_error("%s: NULL argument", who);
+        return 1;
+    }
+    if (n_groups <= 0 || n_genes <= 0 || n_cols <= 0) return 0;
+    if (k < 1 || k > n_genes) { set_error("%s: k = %d outside [1, %d]", who, k, n_genes); return 1; }
+    if ((!group_rows && n_cols > n_groups) || (lfc && lfc_group_stride < n_genes)) {
+        set_error("%s: n_cols > n_groups without group_rows, or lfc_group_stride < n_genes", who);
+        return 1;
+    }
+    if (workspace_bytes < illico_top_genes_workspace_bytes(n_cols, n_genes)) { set_error("%s: workspace too small", who); return 1; }
+    const int ctas = n_cols < 148 * 2 ? n_cols : 148 * 2;
+    unsigned long long* slab =
+        reinterpret_cast<unsigned long long*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
+    const TopFilter F{nullptr, nullptr, NAN, NAN, NAN, NAN, nullptr, 0};
+    const TopColumns O{group_rows, n_cols, lfc, lfc_group_stride, out_score, out_lfc, out_p, out_p_adj};
+    cudaStream_t st = (cudaStream_t)stream;
+    ILLICO_LAUNCH("top_genes_columns_kernel", st,
+                  top_genes_kernel<true><<<ctas, BH_THREADS, 0, st>>>(scores, score_group_stride, results, result_group_stride, p_adj,
+                                                                      n_groups, n_genes, k, by_abs ? 1 : 0, F, out_gene, nullptr,
+                                                                      slab, O));
+    ILLICO_CUDA_OK(cudaGetLastError());
+    return 0;
 }
 
 int illico_compute_pval_batch(const int64_t* n_ref, const int64_t* n_tgt, const int64_t* n, const double* tie_sum,

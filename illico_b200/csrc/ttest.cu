@@ -5,6 +5,9 @@
 //                           -> (p, t, fold_change) records and the score plane: welch_ttest_kernel (CTA = 32 genes x 16
 //                           group lanes) for t, df and the fold change, welch_pvalue_kernel (a thread per test) for p.
 //   illico_student_t_batch  the device Student t CDF on arrays of (df, t): the known-answer hook of the p-value.
+//   illico_log_fold_changes the group sums S1 (illico_group_sums_* or the moments pass) -> scanpy's `logfoldchanges`,
+//                           log2((f(mean_g) + 1e-9) / (f(mean_rest) + 1e-9)), f = expm1(x * ln base), in the CTA layout of
+//                           welch_ttest_kernel and with its means and one-versus-rest totals.
 //
 // Per group and gene, with n cells, S1 = sum x, S2 = sum x*x (scanpy 1.10 _get_mean_var, dense branch, one pass):
 //   mean = S1 / n;  var = S2 / n - mean * mean;  if n != 1: var *= n / (n - 1)
@@ -135,10 +138,15 @@ __device__ __forceinline__ double t_pvalue(double df, double t, int alternative)
     return stdtr(df, alternative == ILLICO_GREATER ? -t : t);
 }
 
+// _get_mean_var's mean: S1 / n (the t-test's and the log fold change's)
+__device__ __forceinline__ double group_mean(double s1, long long n) {
+    return __ddiv_rn(s1, (double)n);
+}
+
 // _get_mean_var, dense branch: mean = S1 / n, var = S2 / n - mean^2, times n / (n - 1) unless n == 1
 __device__ __forceinline__ void mean_var(double s1, double s2, long long n, double& mean, double& var) {
     const double dn = (double)n;
-    mean = __ddiv_rn(s1, dn);
+    mean = group_mean(s1, n);
     var = __dsub_rn(__ddiv_rn(s2, dn), __dmul_rn(mean, mean));
     if (n != 1) var = __dmul_rn(var, __ddiv_rn(dn, (double)(n - 1)));
 }
@@ -239,6 +247,41 @@ __global__ void __launch_bounds__(256) welch_pvalue_kernel(double* __restrict__ 
     rec[0] = (p != p) ? 1.0 : p;
 }
 
+// scanpy's log fold change from the two means: log2((f(m_g) + 1e-9) / (f(m_r) + 1e-9)), f(m) = expm1(m * log_scale)
+__device__ __forceinline__ double log_fold_change(double mg, double mr, double log_scale) {
+    const double fg = __dadd_rn(expm1(__dmul_rn(mg, log_scale)), 1e-9);
+    const double fr = __dadd_rn(expm1(__dmul_rn(mr, log_scale)), 1e-9);
+    return log2(__ddiv_rn(fg, fr));
+}
+
+// CTA = TT_COLS genes x TT_ROWS group lanes, as welch_ttest_kernel: the one-versus-rest totals are added in its order
+__global__ void __launch_bounds__(TT_COLS * TT_ROWS) log_fold_change_kernel(const double* __restrict__ S1, long long ms,
+                                                                            const int32_t* __restrict__ group_size, int G, int N,
+                                                                            int ref, long long n_cells, double log_scale,
+                                                                            double* __restrict__ lfc, long long lstride) {
+    __shared__ double part[TT_ROWS][TT_COLS + 1];
+    const int c = threadIdx.x % TT_COLS, r = threadIdx.x / TT_COLS;
+    const int j = blockIdx.x * TT_COLS + c;
+    const bool in = j < N;
+    double total = 0.0;
+    if (ref < 0) {
+        if (in)
+            for (int g = r; g < G; g += TT_ROWS) total = __dadd_rn(total, S1[(long long)g * ms + j]);
+        part[r][c] = total;
+        __syncthreads();
+        total = 0.0;
+        for (int q = 0; q < TT_ROWS; ++q) total = __dadd_rn(total, part[q][c]);
+    }
+    if (!in) return;
+    const double ref_mean = ref >= 0 ? group_mean(S1[(long long)ref * ms + j], group_size[ref]) : 0.0;
+    for (int g = r; g < G; g += TT_ROWS) {
+        const long long ng = group_size[g];
+        const double s1 = S1[(long long)g * ms + j];
+        const double rest = ref >= 0 ? ref_mean : group_mean(__dsub_rn(total, s1), n_cells - ng);
+        lfc[(long long)g * lstride + j] = log_fold_change(group_mean(s1, ng), rest, log_scale);
+    }
+}
+
 __global__ void student_t_batch_kernel(const double* df, const double* t, long long n, int alternative, double* out) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out[i] = t_pvalue(df[i], t[i], alternative);
@@ -277,6 +320,25 @@ int illico_welch_ttest(const double* sums, const double* sumsq, const double* fs
     ILLICO_LAUNCH("welch_pvalue_kernel", st,
                   welch_pvalue_kernel<<<(unsigned)((tests + 255) / 256), 256, 0, st>>>(results, result_group_stride, n_groups, n_genes,
                                                                                      ref_group < 0 ? -1 : ref_group, alternative));
+    ILLICO_CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
+int illico_log_fold_changes(const double* sums, int64_t group_stride, const int32_t* group_size, int32_t n_groups, int32_t n_genes,
+                            int32_t ref_group, int64_t n_cells, double log_scale, double* lfc, int64_t lfc_group_stride,
+                            void* stream) {
+    if (!sums || !group_size || !lfc) { set_error("illico_log_fold_changes: NULL argument"); return 1; }
+    if (n_groups <= 0 || n_genes <= 0) return 0;
+    if (group_stride < n_genes || lfc_group_stride < n_genes || ref_group >= n_groups) {
+        set_error("illico_log_fold_changes: a stride below the batch width or ref_group out of range");
+        return 1;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const unsigned ctas = (unsigned)(((long long)n_genes + TT_COLS - 1) / TT_COLS);
+    ILLICO_LAUNCH("log_fold_change_kernel", st,
+                  log_fold_change_kernel<<<ctas, TT_COLS * TT_ROWS, 0, st>>>(sums, group_stride, group_size, n_groups, n_genes,
+                                                                             ref_group < 0 ? -1 : ref_group, (long long)n_cells,
+                                                                             log_scale, lfc, lfc_group_stride));
     ILLICO_CUDA_OK(cudaGetLastError());
     return 0;
 }

@@ -121,13 +121,13 @@ class Engine:
     def is_ovo(self) -> bool:
         return self.host_plan.ref_group >= 0
 
-    def max_batch_genes(self, n_genes: int, method: str = WILCOXON) -> int:
-        """Genes per device batch so that the staged lists (Wilcoxon) or the three float64 moment planes (t-test) stay
-        within the memory budget."""
+    def max_batch_genes(self, n_genes: int, method: str = WILCOXON, lfc: bool = False) -> int:
+        """Genes per device batch so that the staged lists (Wilcoxon; with ``lfc``, the float64 group sums too) or the three
+        float64 moment planes (t-test) stay within the memory budget."""
         free, _total = torch.cuda.mem_get_info(self.device)
         if method == WILCOXON:
             budget = min(_env_int("ILLICO_B200_IR_BYTES", 16 << 30), int(free * 0.35))
-            per_gene = self.host_plan.slot_cap * 4 + self.host_plan.n_segments * 4
+            per_gene = self.host_plan.slot_cap * 4 + self.host_plan.n_segments * 4 + (self.host_plan.n_groups * 8 if lfc else 0)
         else:
             budget = int(free * 0.35)
             per_gene = self.host_plan.n_groups * 3 * 8
@@ -183,7 +183,8 @@ class Engine:
     # ---- one gene batch ----------------------------------------------------------------------------------
     def run_batch(self, M: DeviceMatrix, lb: int, ub: int, flags: _lib.Flags, results: torch.Tensor,
                   result_gene0: int, debug: dict | None = None, scores: torch.Tensor | None = None,
-                  nnz: torch.Tensor | None = None, method: str = WILCOXON) -> None:
+                  nnz: torch.Tensor | None = None, method: str = WILCOXON, lfc: torch.Tensor | None = None,
+                  log_scale: float = 1.0) -> None:
         """Enqueues stage + rank for genes ``[lb, ub)`` of ``M``; writes ``results[:, result_gene0 + k, :]``.
 
         ``results`` is a device tensor ``[G, N_total, 3]`` float64 (contiguous).  ``scores``, a device tensor ``[G, N_total]``
@@ -191,6 +192,9 @@ class Engine:
         device tensor ``[G, N_total]`` int32 (contiguous), receives at ``nnz[:, result_gene0 + k]`` how many cells of each
         group have a non-zero value (``illico_count_nonzero_*``, enqueued before the tests on the same stream).
         ``method`` "t-test" / "t-test_overestim_var": Welch's t-test instead (``_run_batch_ttest``), same outputs.
+        ``lfc``, a device tensor ``[G, N_total]`` float64 (contiguous), receives scanpy's log fold change of every test at
+        ``lfc[:, result_gene0 + k]`` (``illico_log_fold_changes``, ``log_scale`` = ln of the log1p base, else 1), from the
+        group sums of a pass of its own (``illico_group_sums_*``, which then also writes ``nnz``) or of the t-test's moments.
         """
         b = ub - lb
         if b <= 0:
@@ -202,8 +206,11 @@ class Engine:
         with torch.cuda.device(self.device):
             M.ready()
         if method != WILCOXON:
-            return self._run_batch_ttest(M, lb, ub, flags, results, result_gene0, scores, nnz, check_method(method))
-        if nnz is not None:
+            return self._run_batch_ttest(M, lb, ub, flags, results, result_gene0, scores, nnz, check_method(method), lfc,
+                                         log_scale)
+        if lfc is not None:
+            self.log_fold_changes(M, lb, ub, lfc, result_gene0, log_scale, nnz)
+        elif nnz is not None:
             self.count_nonzero(M, lb, ub, nnz, result_gene0)
         if M.raw is not None:
             return self._run_batch_wide(M, lb, ub, flags, results, result_gene0, debug, scores)
@@ -258,10 +265,56 @@ class Engine:
                         Ntot, st)
         _lib.check(rc, f"illico_count_nonzero_{M.fmt}")
 
-    def _run_batch_ttest(self, M: DeviceMatrix, lb: int, ub: int, flags: _lib.Flags, results, result_gene0, scores, nnz, method):
+    def _scratch(self, name: str, G: int, b: int) -> torch.Tensor:
+        """This thread's float64 ``[G, >= b]`` scratch plane ``name`` (grown on demand), recorded on the current stream."""
+        t = self._tls
+        buf = getattr(t, name, None)
+        if buf is None or buf.shape[-1] < b:
+            setattr(t, name, None)
+            with torch.cuda.device(self.device):
+                buf = torch.empty((G, b), dtype=torch.float64, device=self.device)
+            setattr(t, name, buf)
+        buf.record_stream(torch.cuda.current_stream(self.device))
+        return buf
+
+    def log_fold_changes(self, M: DeviceMatrix, lb: int, ub: int, lfc: torch.Tensor, result_gene0: int, log_scale: float = 1.0,
+                         nnz: torch.Tensor | None = None) -> None:
+        """``lfc[:, result_gene0 + k]`` = scanpy's log fold change of gene ``lb + k`` of ``M`` in every group, on the current
+        stream: the group sums of the batch (``illico_group_sums_*``; with ``nnz``, its count plane in the same launch, as
+        ``count_nonzero``), then ``illico_log_fold_changes``.  A matrix kept as float64 (``M.raw``) is summed as it is."""
+        b = ub - lb
+        G, Ntot = lfc.shape
+        assert lfc.dtype == torch.float64 and lfc.is_contiguous() and G == self.n_groups and lfc.device == self.device
+        sums = self._scratch("sums", G, b)
+        vals, dtype = (M.raw, _lib.DTYPE_F64) if M.raw is not None else (M.data, _lib.DTYPE_F32)
+        cnt, cstride = (None, 0)
+        if nnz is not None:
+            assert nnz.dtype == torch.int32 and nnz.is_contiguous() and tuple(nnz.shape) == (G, Ntot)
+            cnt, cstride = nnz.data_ptr() + result_gene0 * 4, Ntot
+        with torch.cuda.device(self.device):
+            st = torch.cuda.current_stream(self.device).cuda_stream
+            if M.fmt == DENSE:
+                rc = self.lib.illico_group_sums_dense(vals.data_ptr(), dtype, int(vals.stride(0)), lb, b, C.byref(self.plan),
+                                                      sums.data_ptr(), cnt, cstride, sums.shape[1], st)
+            else:
+                fn = getattr(self.lib, f"illico_group_sums_{M.fmt}")
+                rc = fn(vals.data_ptr(), dtype, M.indices.data_ptr(), M.indptr.data_ptr(), lb, b, C.byref(self.plan), sums.data_ptr(),
+                        cnt, cstride, sums.shape[1], st)
+            _lib.check(rc, f"illico_group_sums_{M.fmt}")
+            self._lfc_from_sums(sums.data_ptr(), sums.shape[1], b, lfc, result_gene0, log_scale, st)
+
+    def _lfc_from_sums(self, s1: int, ms: int, b: int, lfc: torch.Tensor, result_gene0: int, log_scale: float, st) -> None:
+        hp = self.host_plan
+        G, Ntot = lfc.shape
+        rc = self.lib.illico_log_fold_changes(s1, ms, self._tables["group_size"].data_ptr(), G, b, hp.ref_group, hp.n_cells,
+                                              float(log_scale), lfc.data_ptr() + result_gene0 * 8, Ntot, st)
+        _lib.check(rc, "illico_log_fold_changes")
+
+    def _run_batch_ttest(self, M: DeviceMatrix, lb: int, ub: int, flags: _lib.Flags, results, result_gene0, scores, nnz, method,
+                         lfc=None, log_scale: float = 1.0):
         """Welch's t-test of genes ``[lb, ub)``: one pass over the batch for the per-(group, gene) moments (and the count
         plane when ``nnz`` is given) -- ``illico_group_moments_*`` -- then ``illico_welch_ttest`` into the same result and
-        score slabs.  float64 values (``M.raw``) are read as they are: no recoding, no staged lists."""
+        score slabs, and ``illico_log_fold_changes`` from the same sums when ``lfc`` is given.  float64 values (``M.raw``) are read as they are: no recoding, no staged lists."""
         b = ub - lb
         G, Ntot = results.shape[0], results.shape[1]
         assert results.dtype == torch.float64 and results.is_contiguous() and G == self.n_groups
@@ -301,6 +354,9 @@ class Engine:
                                              results.data_ptr() + result_gene0 * 3 * 8, Ntot * 3,
                                              scores.data_ptr() + result_gene0 * 8 if scores is not None else None, Ntot, st)
             _lib.check(rc, "illico_welch_ttest")
+            if lfc is not None:
+                assert lfc.dtype == torch.float64 and lfc.is_contiguous() and tuple(lfc.shape) == (G, Ntot)
+                self._lfc_from_sums(s1, ms, b, lfc, result_gene0, log_scale, st)
 
     def _run_batch_wide(self, M: DeviceMatrix, lb: int, ub: int, flags: _lib.Flags, results, result_gene0, debug, scores=None):
         """float64 input (values float32 cannot hold): every sub-batch is recoded on the device to order-preserving

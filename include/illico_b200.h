@@ -364,6 +364,23 @@ int illico_top_genes_filtered(const double* scores, int64_t score_group_stride, 
                               int32_t* out_gene, double* out_rec, int32_t* kept, void* workspace, size_t workspace_bytes,
                               void* stream);
 
+/* Bonferroni adjusted p-values (scanpy corr_method="bonferroni"): p_adj[g * n_genes + j] = min(p * n_genes, 1) of
+ * p = p_values[g * group_stride + j * gene_stride], NaN where p is NaN.  Same layout as illico_bh_adjust; a thread per test. */
+int illico_bonferroni_adjust(const double* p_values, int64_t group_stride, int64_t gene_stride, int32_t n_groups, int32_t n_genes,
+                             double* p_adj, void* stream);
+
+/* illico_top_genes' ranking (same keys, same stable sort, no filter) written in scanpy's rank_genes_groups layout: output
+ * column c (0 <= c < n_cols) ranks group group_rows[c] (device int32 [n_cols], each in [0, n_groups); NULL: group c, with
+ * n_cols <= n_groups), and rank r of it goes to element r * n_cols + c of five column-major [k, n_cols] planes: out_gene
+ * (int32 gene index), out_score (the score rounded to float32), out_lfc (lfc[g * lfc_group_stride + j] rounded to float32;
+ * lfc NULL: NaN), out_p (results[g * result_group_stride + 3 j], float64) and out_p_adj (p_adj[g * n_genes + j]; NULL: NaN).
+ * Each plane is then a record array with one field per column, without a copy.  Workspace:
+ * illico_top_genes_workspace_bytes(n_cols, n_genes). */
+int illico_top_genes_columns(const double* scores, int64_t score_group_stride, const double* results, int64_t result_group_stride,
+                             const double* p_adj, const double* lfc, int64_t lfc_group_stride, int32_t n_groups, int32_t n_genes,
+                             const int32_t* group_rows, int32_t n_cols, int32_t k, int32_t by_abs, int32_t* out_gene, float* out_score,
+                             float* out_lfc, double* out_p, double* out_p_adj, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- cells that express a gene (scanpy rank_genes_groups(pts=True): pct_nz_group / pct_nz_reference) -------------------
  * counts[g * count_group_stride + j] (int32) = cells of group g whose value in gene gene_lb + j satisfies x != 0: -0.0 and
  * explicitly stored zeros do not count, NaN does.  Every element of the batch's [n_groups, n_genes_batch] plane is written
@@ -407,6 +424,28 @@ int illico_group_moments_csc(const void* data, int32_t dtype, const int32_t* ind
                              int32_t n_genes_batch, const illico_plan_t* plan, int32_t is_log1p, double* sums, double* sumsq,
                              double* fsums, int32_t* counts, int64_t count_group_stride, int64_t group_stride,
                              void* stream);
+/* illico_group_moments_* with one accumulator: sums[g * group_stride + j] = sum of x (float64), and counts (may be NULL)
+ * the count plane in the same launch.  Every element of the [n_groups, n_genes_batch] planes is written; inputs, dtypes and
+ * summation as for illico_group_moments_*.  What scanpy's log fold change needs in a Wilcoxon run. */
+int illico_group_sums_dense(const void* X, int32_t dtype, int64_t ld, int32_t gene_lb, int32_t n_genes_batch,
+                            const illico_plan_t* plan, double* sums, int32_t* counts, int64_t count_group_stride,
+                            int64_t group_stride, void* stream);
+int illico_group_sums_csr(const void* data, int32_t dtype, const int32_t* indices, const int64_t* indptr, int32_t gene_lb,
+                          int32_t n_genes_batch, const illico_plan_t* plan, double* sums, int32_t* counts,
+                          int64_t count_group_stride, int64_t group_stride, void* stream);
+int illico_group_sums_csc(const void* data, int32_t dtype, const int32_t* indices, const int64_t* indptr, int32_t gene_lb,
+                          int32_t n_genes_batch, const illico_plan_t* plan, double* sums, int32_t* counts,
+                          int64_t count_group_stride, int64_t group_stride, void* stream);
+/* scanpy's logfoldchanges from the group sums of a batch (illico_group_sums_* / illico_group_moments_*' sums), in float64:
+ *   mean_g = S1_g / n_g;  mean_rest = mean_ref (ref_group >= 0) or (T - S1_g) / (n_cells - n_g) (ref_group < 0, T the gene's
+ *   total over the groups in illico_welch_ttest's fixed order);
+ *   lfc[g * lfc_group_stride + j] = log2((expm1(mean_g * log_scale) + 1e-9) / (expm1(mean_rest * log_scale) + 1e-9))
+ * log_scale = ln(base) of log1p data in another base, else 1.  group_size: device [n_groups].  CTA = 32 genes x 16 group
+ * lanes (csrc/ttest.cu). */
+int illico_log_fold_changes(const double* sums, int64_t group_stride, const int32_t* group_size, int32_t n_groups, int32_t n_genes,
+                            int32_t ref_group, int64_t n_cells, double log_scale, double* lfc, int64_t lfc_group_stride,
+                            void* stream);
+
 /* The moment planes of a batch of n_genes genes -> results[g * result_group_stride + 3 j ..] = (p, t, fold_change) and, when
  * scores is not NULL, scores[g * score_group_stride + j] = t with NaN -> 0.  One thread per gene (csrc/ttest.cu):
  *   mean = S1 / n;  var = S2 / n - mean * mean;  if n != 1: var *= n / (n - 1)        (scanpy 1.10 _get_mean_var, dense)
