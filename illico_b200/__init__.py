@@ -3,12 +3,12 @@
 Drop-in for the one hot path of remydubois/illico: ``asymptotic_wilcoxon(adata, ...)`` and the six
 batch dispatchers under it, plus ``rank_genes(adata, ...)`` (each group's genes ranked by score, selected on the GPU) and ``ttest(adata, ...)``
 (Welch's t-test, scanpy's ``method="t-test"``) and ``rank_genes_groups(adata, ...)`` (a drop-in for scanpy's, writing
-``adata.uns``), computed by hand-written sm_100a CUDA kernels behind a C ABI
+``adata.uns``) with its marker filter ``filter_rank_genes_groups(adata, ...)``, computed by hand-written sm_100a CUDA kernels behind a C ABI
 (``include/illico_b200.h``).  There is no CPU fallback.
 """
 __version__ = "0.1.0"
 
-__all__ = ["asymptotic_wilcoxon", "rank_genes", "rank_genes_groups", "ttest", "register_into_reference", "__version__"]
+__all__ = ["asymptotic_wilcoxon", "filter_rank_genes_groups", "rank_genes", "rank_genes_groups", "ttest", "register_into_reference", "__version__"]
 
 
 def __getattr__(name):
@@ -32,13 +32,14 @@ def __getattr__(name):
         # (importing .ttest binds the .ttest submodule to this name, and the .asymptotic_wilcoxon module to its own)
         globals().update(asymptotic_wilcoxon=aw, ttest=fn)
         return fn
-    if name == "rank_genes_groups":
+    if name in ("rank_genes_groups", "filter_rank_genes_groups"):
         from .asymptotic_wilcoxon import asymptotic_wilcoxon as aw
-        from .scanpy_compat import rank_genes_groups as fn
+        from .scanpy_compat import filter_rank_genes_groups, rank_genes_groups
 
         # (importing .scanpy_compat imports .asymptotic_wilcoxon, which binds that module to its name)
-        globals().update(asymptotic_wilcoxon=aw, rank_genes_groups=fn)
-        return fn
+        globals().update(asymptotic_wilcoxon=aw, rank_genes_groups=rank_genes_groups,
+                         filter_rank_genes_groups=filter_rank_genes_groups)
+        return globals()[name]
     if name == "register_into_reference":
         from .registry import register_into_reference as fn
 

@@ -121,12 +121,15 @@ SIGNATURES = {
     "illico_bonferroni_adjust": (C.c_int, [_vp, _i64, _i64, _i32, _i32, _vp, _vp]),
     "illico_top_genes_columns": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _vp, _i64, _i32, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _vp,
                                            _vp, _vp, _vp, _sz, _vp]),
-    "illico_welch_ttest": (C.c_int, [_vp, _vp, _vp, _i64, _vp, _i32, _i32, _i32, _i64, _i32, _i32, _vp, _i64, _vp, _i64, _vp]),
+    "illico_filter_marker_pairs": (C.c_int, [_vp, _vp, _i32, _i32, _i64, _vp, _i32, _vp, _i32, _vp, _i32, C.c_double, C.c_double,
+                                             C.c_double, _i32, _vp, _vp]),
+    "illico_welch_ttest":(C.c_int, [_vp, _vp, _vp, _i64, _vp, _i32, _i32, _i32, _i64, _i32, _i32, _vp, _i64, _vp, _i64, _vp]),
     "illico_student_t_batch": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _vp]),
     "illico_compute_pval_batch": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
 }
 
 DTYPE_F32, DTYPE_F64, DTYPE_F16, DTYPE_I8, DTYPE_U8, DTYPE_I16, DTYPE_I32, DTYPE_I64 = range(8)
+PAIRS_PLANE, PAIRS_F64, PAIRS_F32 = range(3)
 
 _lib = None
 

@@ -235,7 +235,7 @@ def _host_fractions(run: _Run):
 
 def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, alternative, use_continuity, tie_correct,
                layer, device, devices, score: bool, on_device: bool, pts: bool = False, method: str = WILCOXON,
-               groups=None, mask_var=None, lfc: bool = False, log_scale: float = 1.0) -> _Run:
+               groups=None, mask_var=None, lfc: bool = False, log_scale: float = 1.0, stats_only: bool = False) -> _Run:
     """Every (group, gene) test of ``adata``: validation, upload, group plan, one gene shard per GPU, batches, backed
     streaming.  ``on_device=False``: each shard's slabs are copied into pinned host arrays (``asymptotic_wilcoxon``).
     ``on_device=True``: they stay on the GPUs and meet in ``[G, N, 3]`` / ``[G, N]`` tensors on the first one
@@ -245,7 +245,9 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
     on every cell with the other groups collapsed into pseudo-groups whose rows are dropped.  ``mask_var``: the genes to
     test (``asymptotic_wilcoxon``); shards, batches and result planes then span the ``n_sel`` selected genes, and every
     batch runs on a matrix that holds only their columns (``select.ColumnSelection``).  ``lfc``: scanpy's log fold change
-    plane too (``Engine.run_batch(lfc=, log_scale=)``), allocated, sharded and gathered like the score plane."""
+    plane too (``Engine.run_batch(lfc=, log_scale=)``), allocated, sharded and gathered like the score plane.
+    ``stats_only``: no test is run -- each batch gets only the ``lfc`` / ``pts`` pass (``Engine.run_batch(stats_only=)``),
+    and neither the results nor the score plane is allocated (the run's ``results`` and ``scores`` are None)."""
     from .select import ColumnSelection, resolve_mask_var
 
     check_method(method)
@@ -338,8 +340,9 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
                     return
                 engine = Engine(shared["grpc"], sh.device, host_plan=shared["host_plan"])
                 flags = flags_for()
-                res = torch.empty((engine.n_groups, sh.ub - sh.lb, 3), dtype=torch.float64, device=sh.device)
-                sc = torch.empty((engine.n_groups, sh.ub - sh.lb), dtype=torch.float64, device=sh.device) if score else None
+                res = None if stats_only else torch.empty((engine.n_groups, sh.ub - sh.lb, 3), dtype=torch.float64, device=sh.device)
+                sc = torch.empty((engine.n_groups, sh.ub - sh.lb), dtype=torch.float64, device=sh.device) if score and not stats_only \
+                    else None
                 nz = torch.empty((engine.n_groups, sh.ub - sh.lb), dtype=torch.int32, device=sh.device) if pts else None
                 lf = torch.empty((engine.n_groups, sh.ub - sh.lb), dtype=torch.float64, device=sh.device) if lfc else None
                 if data_handler.in_ram:
@@ -362,16 +365,17 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
                     off = bounds[0] - sh.lb      # gene g of the run is column g + off of the device matrix
                     for lb, ub in _batches(sh.lb, sh.ub, batch_size, engine, True, method, lfc):
                         engine.run_batch(M, lb + off, ub + off, flags, res, lb - sh.lb, scores=sc, nnz=nz, method=method, lfc=lf,
-                                         log_scale=log_scale)
+                                         log_scale=log_scale, stats_only=stats_only)
                 else:
                     _run_backed(data_handler, _batches(sh.lb, sh.ub, batch_size, engine, False, method, lfc), engine, flags, res,
                                 max(1, int(n_threads)), gene0=sh.lb, scores=sc, nnz=nz, method=method, selection=selection,
-                                columns=colsel, lfc=lf, log_scale=log_scale)
+                                columns=colsel, lfc=lf, log_scale=log_scale, stats_only=stats_only)
                 if on_device and len(shards) == 1:
                     shared["out"], shared["out_scores"], shared["out_nnz"], shared["out_lfc"] = res, sc, nz, lf
                 else:
                     kind = "d2d" if on_device else "d2h"
-                    hostio.d2h_slab(shared["out"], res, sh.lb, kind)
+                    if res is not None:
+                        hostio.d2h_slab(shared["out"], res, sh.lb, kind)
                     if sc is not None:
                         hostio.d2h_slab(shared["out_scores"], sc, sh.lb, kind)
                     if nz is not None:
@@ -402,13 +406,15 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
         shared["grpc"], shared["host_plan"] = grpc, build_plan(grpc, seg_max)
         G = int(grpc.counts.size)
         if not on_device:
-            shared["out"] = torch.empty((G, n_genes, 3), dtype=torch.float64, pin_memory=True)
-            shared["out_scores"] = torch.empty((G, n_genes), dtype=torch.float64, pin_memory=True) if score else None
+            shared["out"] = None if stats_only else torch.empty((G, n_genes, 3), dtype=torch.float64, pin_memory=True)
+            shared["out_scores"] = torch.empty((G, n_genes), dtype=torch.float64, pin_memory=True) if score and not stats_only \
+                else None
             shared["out_nnz"] = torch.empty((G, n_genes), dtype=torch.int32, pin_memory=True) if pts else None
             shared["out_lfc"] = torch.empty((G, n_genes), dtype=torch.float64, pin_memory=True) if lfc else None
         elif len(shards) > 1:
-            shared["out"] = torch.empty((G, n_genes, 3), dtype=torch.float64, device=devs[0])
-            shared["out_scores"] = torch.empty((G, n_genes), dtype=torch.float64, device=devs[0]) if score else None
+            shared["out"] = None if stats_only else torch.empty((G, n_genes, 3), dtype=torch.float64, device=devs[0])
+            shared["out_scores"] = torch.empty((G, n_genes), dtype=torch.float64, device=devs[0]) if score and not stats_only \
+                else None
             shared["out_nnz"] = torch.empty((G, n_genes), dtype=torch.int32, device=devs[0]) if pts else None
             shared["out_lfc"] = torch.empty((G, n_genes), dtype=torch.float64, device=devs[0]) if lfc else None
     except BaseException:
@@ -428,12 +434,12 @@ def _run_tests(adata, is_log1p, group_keys, reference, n_threads, batch_size, al
             raise sh.error
     out, scores, nnz, lfcs = shared["out"], shared["out_scores"], shared.get("out_nnz"), shared.get("out_lfc")
     if not on_device:
-        out, scores = out.numpy(), (scores.numpy() if scores is not None else None)
+        out, scores = (out.numpy() if out is not None else None), (scores.numpy() if scores is not None else None)
         nnz = nnz.numpy() if nnz is not None else None
         lfcs = lfcs.numpy() if lfcs is not None else None
     S = len(unique_raw_groups)     # (fewer than G when one-versus-rest pseudo-groups follow the selected groups)
     var_names = adata.var_names if colsel is None else adata.var_names[colsel.cols]
-    return _Run(unique_raw_groups, grpc, shards[0].device, out[:S], scores[:S] if scores is not None else None, nnz, var_names,
+    return _Run(unique_raw_groups, grpc, shards[0].device, out[:S] if out is not None else None, scores[:S] if scores is not None else None, nnz, var_names,
                 lfcs[:S] if lfcs is not None else None)
 
 
@@ -509,7 +515,8 @@ class _PinnedSlot:
 
 
 def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, results, n_readers: int, gene0: int = 0,
-                scores=None, nnz=None, method: str = WILCOXON, selection=None, columns=None, lfc=None, log_scale: float = 1.0) -> None:
+                scores=None, nnz=None, method: str = WILCOXON, selection=None, columns=None, lfc=None, log_scale: float = 1.0,
+                stats_only: bool = False) -> None:
     """Out-of-core input (BASELINE config 4): gene batches stream disk -> pinned ring -> HBM -> kernels.
 
     Reader threads slice the next batches from the backed container straight into pinned staging buffers (a ring of
@@ -519,7 +526,7 @@ def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, resu
     ``asymptotic_wilcoxon.py:212-249``).  ``selection`` (``select.RowSelection``): only those rows are ranked -- the readers
     gather them out of dense batches, CSC batches are compacted on the device (``illico_select_rows_csc``).  ``columns``
     (``select.ColumnSelection``): the batches are ranges of the selected genes, and the readers fetch each one's runs of
-    consecutive columns as slices (``ColumnSelection.fetch``)."""
+    consecutive columns as slices (``ColumnSelection.fetch``).  ``stats_only``: ``Engine.run_batch``'s."""
     from .engine import DENSE, DeviceMatrix, _to_f32_or_wide
 
     dev = engine.device
@@ -605,7 +612,7 @@ def _run_backed(data_handler: DataHandler, iterator, engine: Engine, flags, resu
 
                 M, bounds = select_rows(M, bounds, selection)
         engine.run_batch(M, bounds[0], bounds[1], flags, results, lb - gene0, scores=scores, nnz=nnz, method=method, lfc=lfc,
-                         log_scale=log_scale)
+                         log_scale=log_scale, stats_only=stats_only)
 
     try:
         while done < n_readers:

@@ -12,6 +12,8 @@
 //   illico_bonferroni_adjust   Bonferroni adjusted p-values, min(p * n_genes, 1) (scanpy's corr_method="bonferroni").
 //   illico_top_genes_columns   illico_top_genes' ranking written column-major in scanpy's record layout ([k, groups]
 //                              planes of gene index, float32 score / log fold change, float64 p / p_adj).
+//   illico_filter_marker_pairs scanpy's filter_rank_genes_groups criteria on the listed (rank, group) pairs of a stored
+//                              result: a uint8 keep mask [k, groups], from device planes or from planes taken from `uns`.
 //   illico_compute_pval_batch  evaluates the epilogue's compute_pval (epilogue.cuh; reference illico/utils/math.py:64-118)
 //                              on arrays of arguments, so the known-answer vectors of tests/golden/primitives.npz can be
 //                              checked against the device code itself.
@@ -221,6 +223,47 @@ __global__ void __launch_bounds__(BH_THREADS) top_genes_kernel(const double* __r
     }
 }
 
+// One source of a filter_marker_pairs quantity (ILLICO_PAIRS_*): a float64 [groups, plane_stride] plane read at (group row,
+// gene), or a [k, n_cols] float64 / float32 plane read at the pair itself.
+struct PairSource {
+    const void* p;
+    int kind;
+};
+
+// v > bound (above) or v < bound, |v| first with absval; a float32 source is compared with the bound rounded to float32
+// (numpy's comparison of a float32 array with a Python float), a float64 one in float64.  NaN fails either way.
+__device__ __forceinline__ bool pair_passes(PairSource s, long long at_plane, long long at_pair, double bound, bool above,
+                                            bool absval) {
+    if (s.kind == ILLICO_PAIRS_F32) {
+        float v = static_cast<const float*>(s.p)[at_pair];
+        if (absval) v = fabsf(v);
+        const float b = __double2float_rn(bound);
+        return above ? v > b : v < b;
+    }
+    double v = static_cast<const double*>(s.p)[s.kind == ILLICO_PAIRS_PLANE ? at_plane : at_pair];
+    if (absval) v = fabs(v);
+    return above ? v > bound : v < bound;
+}
+
+// A thread per pair i = r * n_cols + c: gene[i] (-1: never kept) of output column c, whose group row is rows[c].
+__global__ void __launch_bounds__(256) filter_marker_pairs_kernel(const int32_t* __restrict__ gene, const int32_t* __restrict__ rows,
+                                                                  long long n_pairs, int n_cols, long long plane_stride,
+                                                                  PairSource in, PairSource out, PairSource fc, double min_in,
+                                                                  double max_out, double min_fc, int compare_abs,
+                                                                  uint8_t* __restrict__ keep) {
+    const long long i = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (i >= n_pairs) return;
+    const int j = gene[i];
+    bool ok = j >= 0;
+    if (ok) {
+        const bool planes = in.kind == ILLICO_PAIRS_PLANE || out.kind == ILLICO_PAIRS_PLANE || fc.kind == ILLICO_PAIRS_PLANE;
+        const long long at = planes ? (long long)rows[i % n_cols] * plane_stride + j : 0;
+        ok = pair_passes(in, at, i, min_in, true, false) && pair_passes(out, at, i, max_out, false, false) &&
+             pair_passes(fc, at, i, min_fc, true, compare_abs != 0);
+    }
+    keep[i] = ok ? 1 : 0;
+}
+
 __global__ void compute_pval_batch_kernel(const long long* n_ref, const long long* n_tgt, const long long* n, const double* tie,
                                           const double* U, const double* mu, const double* cc, const int* alt, double* out,
                                           long long count) {
@@ -377,6 +420,34 @@ int illico_top_genes_columns(const double* scores, int64_t score_group_stride, c
                   top_genes_kernel<true><<<ctas, BH_THREADS, 0, st>>>(scores, score_group_stride, results, result_group_stride, p_adj,
                                                                       n_groups, n_genes, k, by_abs ? 1 : 0, F, out_gene, nullptr,
                                                                       slab, O));
+    ILLICO_CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
+int illico_filter_marker_pairs(const int32_t* gene, const int32_t* group_rows, int32_t k, int32_t n_cols, int64_t plane_stride,
+                               const void* pct_in, int32_t pct_in_kind, const void* pct_out, int32_t pct_out_kind,
+                               const void* fold_change, int32_t fold_change_kind, double min_in_group_fraction,
+                               double max_out_group_fraction, double min_fold_change, int32_t compare_abs, uint8_t* keep,
+                               void* stream) {
+    const char* who = "illico_filter_marker_pairs";
+    if (k <= 0 || n_cols <= 0) return 0;
+    const int kinds[3] = {pct_in_kind, pct_out_kind, fold_change_kind};
+    bool planes = false;
+    for (int q = 0; q < 3; ++q) {
+        if (kinds[q] < ILLICO_PAIRS_PLANE || kinds[q] > ILLICO_PAIRS_F32) { set_error("%s: unknown source kind %d", who, kinds[q]); return 1; }
+        planes = planes || kinds[q] == ILLICO_PAIRS_PLANE;
+    }
+    if (!gene || !keep || !pct_in || !pct_out || !fold_change || (planes && (!group_rows || plane_stride < 1))) {
+        set_error("%s: NULL argument, or a plane source without group_rows / plane_stride", who);
+        return 1;
+    }
+    const long long n_pairs = (long long)k * n_cols;
+    cudaStream_t st = (cudaStream_t)stream;
+    ILLICO_LAUNCH("filter_marker_pairs_kernel", st,
+                  filter_marker_pairs_kernel<<<(unsigned)((n_pairs + 255) / 256), 256, 0, st>>>(
+                      gene, group_rows, n_pairs, n_cols, (long long)plane_stride, PairSource{pct_in, pct_in_kind},
+                      PairSource{pct_out, pct_out_kind}, PairSource{fold_change, fold_change_kind}, min_in_group_fraction,
+                      max_out_group_fraction, min_fold_change, compare_abs ? 1 : 0, keep));
     ILLICO_CUDA_OK(cudaGetLastError());
     return 0;
 }

@@ -184,7 +184,7 @@ class Engine:
     def run_batch(self, M: DeviceMatrix, lb: int, ub: int, flags: _lib.Flags, results: torch.Tensor,
                   result_gene0: int, debug: dict | None = None, scores: torch.Tensor | None = None,
                   nnz: torch.Tensor | None = None, method: str = WILCOXON, lfc: torch.Tensor | None = None,
-                  log_scale: float = 1.0) -> None:
+                  log_scale: float = 1.0, stats_only: bool = False) -> None:
         """Enqueues stage + rank for genes ``[lb, ub)`` of ``M``; writes ``results[:, result_gene0 + k, :]``.
 
         ``results`` is a device tensor ``[G, N_total, 3]`` float64 (contiguous).  ``scores``, a device tensor ``[G, N_total]``
@@ -195,6 +195,8 @@ class Engine:
         ``lfc``, a device tensor ``[G, N_total]`` float64 (contiguous), receives scanpy's log fold change of every test at
         ``lfc[:, result_gene0 + k]`` (``illico_log_fold_changes``, ``log_scale`` = ln of the log1p base, else 1), from the
         group sums of a pass of its own (``illico_group_sums_*``, which then also writes ``nnz``) or of the t-test's moments.
+        ``stats_only``: no test -- only the ``lfc`` / ``nnz`` pass is enqueued (``results`` may be None; a float64 matrix is
+        summed and counted as it is, with no recoding).
         """
         b = ub - lb
         if b <= 0:
@@ -205,6 +207,12 @@ class Engine:
             raise ValueError(f"Invalid chunk bounds: {(lb, ub)} for data with {M.shape[1]} columns.")
         with torch.cuda.device(self.device):
             M.ready()
+        if stats_only:
+            if lfc is not None:
+                self.log_fold_changes(M, lb, ub, lfc, result_gene0, log_scale, nnz)
+            elif nnz is not None:
+                self.count_nonzero(M, lb, ub, nnz, result_gene0)
+            return
         if method != WILCOXON:
             return self._run_batch_ttest(M, lb, ub, flags, results, result_gene0, scores, nnz, check_method(method), lfc,
                                          log_scale)

@@ -7,20 +7,27 @@ one field per group), so ``sc.get.rank_genes_groups_df``, ``sc.pl.rank_genes_gro
 (``illico_group_sums_*`` or the t-test's moments, then ``illico_log_fold_changes``); the adjustment (``illico_bh_adjust`` /
 ``illico_bonferroni_adjust``) and the per-group selection in scanpy's column layout (``illico_top_genes_columns``) run on the
 device, so only the ``n_genes`` records of each group cross PCIe.
+
+``filter_rank_genes_groups``: scanpy 1.10's ``sc.tl.filter_rank_genes_groups`` over such a result (ours or scanpy's).
+Fractions and fold changes come from ``uns`` when the result is one-versus-rest on the same ``groupby`` and ``use_raw``;
+otherwise from one pass over the listed genes' columns of ``X`` (``illico_group_sums_*`` / ``illico_count_nonzero_*``, then
+``illico_log_fold_changes`` and ``illico_nonzero_fractions``, one-versus-rest).  The criteria are evaluated on the device
+(``illico_filter_marker_pairs``), so only a ``[k, groups]`` keep mask comes back.
 """
 from __future__ import annotations
 
 from typing import Literal
 
 import numpy as np
+import numpy.lib.recfunctions as rfn
 import pandas as pd
 import torch
 
 from . import _lib
-from .asymptotic_wilcoxon import _run_tests, check_flag, nonzero_fractions
+from .asymptotic_wilcoxon import _device_list, _run_tests, check_flag, nonzero_fractions
 from .ranking import _bh_on_device
 
-__all__ = ["rank_genes_groups"]
+__all__ = ["filter_rank_genes_groups", "rank_genes_groups"]
 
 METHODS = ("t-test", "t-test_overestim_var", "wilcoxon")
 CORR_METHODS = ("benjamini-hochberg", "bonferroni")
@@ -80,6 +87,13 @@ def group_order(labels, groups, reference) -> list:
         raise ValueError(f"Could not calculate statistics for groups {', '.join(map(str, small))} since they only contain one "
                          "sample.")
     return order
+
+
+def log1p_scale(adata) -> float:
+    """ln of ``adata.uns["log1p"]["base"]``, or 1 when no base is set (scanpy's ``expm1(x · ln base)``)."""
+    uns = getattr(adata, "uns", {})
+    base = uns.get("log1p", {}).get("base") if "log1p" in uns else None
+    return float(np.log(base)) if base is not None else 1.0
 
 
 def records(planes: np.ndarray, fields: list) -> np.recarray:
@@ -164,9 +178,7 @@ def rank_genes_groups(
         adata = adata.copy()
     use_raw = resolve_use_raw(adata, use_raw, layer)
     order = group_order(adata.obs[groupby], groups, reference)
-    uns = getattr(adata, "uns", {})
-    base = uns.get("log1p", {}).get("base") if "log1p" in uns else None
-    log_scale = float(np.log(base)) if base is not None else 1.0
+    log_scale = log1p_scale(adata)
     target = _RawView(adata) if use_raw else adata
     ref = None if reference == "rest" else reference
     run = _run_tests(target, False, groupby, ref, n_threads, batch_size, "two-sided", False, tie_correct, layer, device, devices,
@@ -233,3 +245,199 @@ def top_columns(results: torch.Tensor, scores: torch.Tensor, lfc: torch.Tensor, 
                                                     ws.numel(), st), "illico_top_genes_columns")
         return gene.cpu().numpy(), {key: p.cpu().numpy() for key, p in planes.items()}
 
+
+
+FILTER_KEY = "rank_genes_groups_filtered"
+
+
+def filter_rank_genes_groups(
+    adata,
+    *,
+    key: str | None = None,
+    groupby: str | None = None,
+    use_raw: bool | None = None,
+    key_added: str = FILTER_KEY,
+    min_in_group_fraction: float = 0.25,
+    min_fold_change: float = 1,
+    max_out_group_fraction: float = 0.5,
+    compare_abs: bool = False,
+    device=None,
+    devices=None,
+    n_threads: int = 1,
+    batch_size: int | Literal["auto"] = "auto",
+):
+    """Filters the marker genes of a stored ranking as ``scanpy.tl.filter_rank_genes_groups`` (scanpy 1.10) does, and
+    writes the result to ``adata.uns[key_added]``.  Returns None.
+
+    ``adata.uns[key]`` (``key=None``: ``"rank_genes_groups"``) is a result in scanpy's layout, written by
+    ``rank_genes_groups`` or by scanpy.  ``groupby`` and ``use_raw`` default to its ``params``.  A listed gene of group
+    ``cluster`` (a field of ``names``) is kept when its fraction of expressing cells in the group is ``>
+    min_in_group_fraction``, that among all other cells is ``< max_out_group_fraction`` and its log fold change (``|lfc|`` with
+    ``compare_abs``) is ``> min_fold_change``; NaN fails every criterion.  ``adata.uns[key_added]`` is a shallow copy of
+    ``adata.uns[key]`` whose ``names`` has ``nan`` in place of every dropped gene; ``adata.uns[key]`` is left as it is.
+
+    When the result is one-versus-rest (``reference="rest"``) on the same ``groupby`` and ``use_raw``, the fold change is its
+    ``logfoldchanges`` (float32, compared in float32) and the fractions its ``pts`` / ``pts_rest``; with both present the
+    matrix is not read at all.  Otherwise the missing quantities come from ``X`` (``adata.raw.X`` with ``use_raw``; never a
+    layer): one pass over the columns of the listed genes only, one-versus-rest over every cell, giving the fractions
+    (``illico_nonzero_fractions``) and ``log2((f(mean_in) + 1e-9) / (f(mean_out) + 1e-9))`` with ``f = expm1(x · ln base)``
+    (``adata.uns["log1p"]["base"]``, else ``expm1``) from float64 group sums (``illico_log_fold_changes``).
+
+    Errors, raised before any device work: ``key`` not in ``adata.uns`` or ``groupby`` not in ``adata.obs``
+    (``KeyError``); a bound that is not a real number, ``compare_abs`` not a bool, ``use_raw=True`` without ``adata.raw``,
+    non-unique gene names (``ValueError``); a listed name not among the genes (``KeyError``).  When ``X`` is read: a field
+    that matches no group of ``groupby`` by ``str``, two groups with the same ``str``, or a cell with a missing label
+    (``ValueError``).
+
+    Where it differs from scanpy: a recomputed fold change comes from float64 sums (scanpy averages in the matrix's dtype; on
+    integer counts both are the same double, otherwise they can differ in the last bits); fractions count values ``!= 0``,
+    not a sparse matrix's stored entries; a field is matched to a group by ``str(group)`` (scanpy's ``obs[groupby] ==
+    field`` matches nothing in a column that is not of strings and drops the whole group); a missing label is refused; a name
+    that is already ``nan`` (a filtered result filtered again) stays ``nan`` (scanpy raises).  scanpy's log message is not
+    given.  ``device``, ``devices``, ``n_threads`` and ``batch_size`` are those of ``asymptotic_wilcoxon``.
+    """
+    key = KEY if key is None else key
+    if key not in adata.uns:
+        raise KeyError(f"{key!r} is not in adata.uns: run rank_genes_groups first")
+    stored = adata.uns[key]
+    params = stored["params"]
+    groupby = params["groupby"] if groupby is None else groupby
+    use_raw = params["use_raw"] if use_raw is None else use_raw
+    bounds = {"min_in_group_fraction": min_in_group_fraction, "min_fold_change": min_fold_change,
+              "max_out_group_fraction": max_out_group_fraction}
+    for name, value in bounds.items():
+        if isinstance(value, (bool, np.bool_)) or not isinstance(value, (int, float, np.integer, np.floating)):
+            raise ValueError(f"{name} must be a real number, got {value!r}")
+    check_flag("compare_abs", compare_abs)
+    check_flag("use_raw", use_raw)
+    if groupby not in adata.obs:
+        raise KeyError(f"groupby = {groupby!r} is not a column of adata.obs")
+    if use_raw and getattr(adata, "raw", None) is None:
+        raise ValueError("Received `use_raw=True`, but `adata.raw` is empty.")
+    var_names = pd.Index(adata.raw.var_names if use_raw else adata.var_names)
+    if not var_names.is_unique:
+        raise ValueError("filter_rank_genes_groups needs unique gene names")
+    same = params.get("groupby") == groupby and params.get("reference") == "rest" and params.get("use_raw") == use_raw
+    use_logfolds, use_fraction = same and "logfoldchanges" in stored, same and "pts_rest" in stored
+
+    names = stored["names"]
+    fields = list(names.dtype.names)
+    k, C = len(names), len(fields)
+    plain = np.asarray(names)                       # (field access on a plain structured array, not a recarray)
+    listed = np.empty((k, C), dtype=object)
+    for c, f in enumerate(fields):
+        listed[:, c] = plain[f]
+    flat = listed.reshape(-1)
+    gene = var_names.get_indexer(pd.Index(flat, dtype=object)).reshape(k, C)
+    missing = pd.isna(listed)
+    absent = (gene < 0) & ~missing
+    if absent.any():
+        raise KeyError(f"{listed[absent][0]!r} is not among the genes of {'adata.raw' if use_raw else 'adata'}")
+
+    sources = {}      # quantity -> [k, C] host plane taken from uns (the others come from the device planes)
+    if use_fraction:
+        for q, frame in (("in", stored["pts"]), ("out", stored["pts_rest"])):
+            sources[q] = _pairs_plane(frame, listed, missing, fields)
+    if use_logfolds:
+        fc = _field_plane(stored["logfoldchanges"], fields)
+        sources["fc"] = fc if fc.dtype == np.float32 else fc.astype(np.float64)
+    read = not (use_logfolds and use_fraction)
+    rows = None
+    if read:
+        from .groups import _factorize_sorted
+
+        groups, _ = _factorize_sorted(adata.obs[groupby])     # (the run's np.unique order; missing labels are refused)
+        strs = [str(g) for g in groups]
+        if len(set(strs)) != len(strs):
+            raise ValueError(f"groupby = {groupby!r} has two groups with the same str: {strs}")
+        row_of = {s: i for i, s in enumerate(strs)}
+        missing = [f for f in fields if f not in row_of]
+        if missing:
+            raise ValueError(f"fields {missing} of {key!r} are not groups of groupby = {groupby!r}")
+        rows = np.array([row_of[f] for f in fields], dtype=np.int32)
+
+    dev = _device_list(device, devices)[0]
+    keep = np.zeros((k, C), dtype=np.uint8)
+    union = np.unique(gene[gene >= 0])
+    if k and C and union.size:
+        to_col = np.full(len(var_names), -1, dtype=np.int32)
+        to_col[union] = np.arange(union.size, dtype=np.int32)
+        col = np.where(gene >= 0, to_col[gene], -1).astype(np.int32)     # gene -> column of the run (over U)
+        planes = {}
+        if read:
+            mask = np.zeros(len(var_names), dtype=bool)
+            mask[union] = True
+            target = _RawView(adata) if use_raw else adata
+            run = _run_tests(target, False, groupby, None, n_threads, batch_size, "two-sided", False, False, None, device, devices,
+                             score=False, on_device=True, pts=not use_fraction, mask_var=mask, lfc=not use_logfolds,
+                             log_scale=log1p_scale(adata), stats_only=True)
+            dev = run.device
+            if not use_fraction:
+                planes["in"], planes["out"] = nonzero_fractions(run.nnz, run.grpc)
+            if not use_logfolds:
+                planes["fc"] = run.lfc
+        keep = _filter_pairs(col, rows, sources, planes, union.size, min_in_group_fraction, max_out_group_fraction,
+                             min_fold_change, compare_abs, dev)
+    kept = np.where(keep.astype(bool), listed, np.nan)
+    out = np.empty(k, dtype=[(f, object) for f in fields])
+    for c, f in enumerate(fields):
+        out[f] = kept[:, c]
+    out = out.view(np.recarray)
+    result = stored.copy()
+    result["names"] = out
+    adata.uns[key_added] = result
+
+
+def _field_plane(rec: np.ndarray, fields: list) -> np.ndarray:
+    """The numeric fields ``fields`` of a record array as the columns of a ``[k, C]`` array (a view where numpy can make
+    one: a result's float32 ``logfoldchanges`` in field order)."""
+    if not fields:
+        return np.empty((len(rec), 0), dtype=np.float32)
+    return rfn.structured_to_unstructured(np.asarray(rec)[fields])
+
+
+def _pairs_plane(frame: pd.DataFrame, listed: np.ndarray, missing: np.ndarray, fields: list) -> np.ndarray:
+    """``frame[field].loc[name]`` for every listed (rank, field) pair as a ``[k, C]`` plane (float32 if the frame is, else
+    float64); a ``nan`` name gives NaN, a field or name missing from the frame is a ``KeyError``."""
+    k, C = listed.shape
+    at = frame.index.get_indexer(pd.Index(listed.reshape(-1), dtype=object)).reshape(k, C)
+    absent = (at < 0) & ~missing
+    if absent.any():
+        raise KeyError(f"{listed[absent][0]!r} is not in the index of the stored fractions")
+    cols = frame.columns.get_indexer(pd.Index(fields, dtype=object))
+    if (cols < 0).any():
+        raise KeyError(f"{fields[int(np.argmax(cols < 0))]!r} is not a column of the stored fractions")
+    values = frame.to_numpy()
+    dtype = np.float32 if values.dtype == np.float32 else np.float64
+    out = values[np.maximum(at, 0), cols[None, :]].astype(dtype, copy=False)
+    out[at < 0] = np.nan
+    return out
+
+
+def _filter_pairs(col: np.ndarray, rows, sources: dict, planes: dict, stride: int, min_in: float, max_out: float,
+                  min_fc: float, compare_abs: bool, dev) -> np.ndarray:
+    """``illico_filter_marker_pairs`` on the listed pairs: each quantity from its device plane (``planes``, ``[G, stride]``
+    float64) or from its host ``[k, C]`` plane (``sources``).  Returns the host ``keep`` mask ``[k, C]`` uint8."""
+    lib = _lib.load()
+    k, C = col.shape
+    with torch.cuda.device(dev):
+        st = torch.cuda.current_stream(dev).cuda_stream
+        hold = []
+
+        def arg(q):
+            if q in planes:
+                p = planes[q]
+                assert p.dtype == torch.float64 and p.is_contiguous() and p.shape[1] == stride
+                return p.data_ptr(), _lib.PAIRS_PLANE
+            t = torch.from_numpy(np.ascontiguousarray(sources[q])).to(dev)
+            hold.append(t)
+            return t.data_ptr(), _lib.PAIRS_F32 if t.dtype == torch.float32 else _lib.PAIRS_F64
+
+        d_col = torch.from_numpy(np.ascontiguousarray(col)).to(dev)
+        d_rows = torch.from_numpy(rows).to(dev) if rows is not None else None
+        keep = torch.empty((k, C), dtype=torch.uint8, device=dev)
+        (pi, ki), (po, ko), (pf, kf) = arg("in"), arg("out"), arg("fc")
+        _lib.check(lib.illico_filter_marker_pairs(d_col.data_ptr(), d_rows.data_ptr() if d_rows is not None else None, k, C, stride,
+                                                  pi, ki, po, ko, pf, kf, float(min_in), float(max_out), float(min_fc),
+                                                  int(bool(compare_abs)), keep.data_ptr(), st), "illico_filter_marker_pairs")
+        return keep.cpu().numpy()

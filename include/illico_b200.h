@@ -381,6 +381,24 @@ int illico_top_genes_columns(const double* scores, int64_t score_group_stride, c
                              const int32_t* group_rows, int32_t n_cols, int32_t k, int32_t by_abs, int32_t* out_gene, float* out_score,
                              float* out_lfc, double* out_p, double* out_p_adj, void* workspace, size_t workspace_bytes, void* stream);
 
+/* scanpy's filter_rank_genes_groups criteria on the listed genes of a stored result, one thread per pair: pair i = r * n_cols
+ * + c (rank r, output column c) is gene[i] (device int32 [k, n_cols]; -1, a name already dropped, is never kept) of group row
+ * group_rows[c].  Each of the three quantities comes from its own source, by kind:
+ *   ILLICO_PAIRS_PLANE  float64 [groups, plane_stride] plane, read at group_rows[c] * plane_stride + gene[i]
+ *                       (illico_nonzero_fractions' pct_group / pct_ref, illico_log_fold_changes' plane);
+ *   ILLICO_PAIRS_F64    float64 [k, n_cols] plane, read at i;
+ *   ILLICO_PAIRS_F32    float32 [k, n_cols] plane, read at i and compared with the bound rounded to float32 (a stored float32
+ *                       logfoldchanges compared as numpy compares it with a Python float).
+ * keep[i] (uint8) = pct_in > min_in_group_fraction && pct_out < max_out_group_fraction && fc > min_fold_change, fc replaced by
+ * |fc| when compare_abs != 0; strict comparisons, a NaN fails each.  group_rows and plane_stride are read only when a source
+ * is a plane. */
+enum illico_pairs_kind { ILLICO_PAIRS_PLANE = 0, ILLICO_PAIRS_F64 = 1, ILLICO_PAIRS_F32 = 2 };
+int illico_filter_marker_pairs(const int32_t* gene, const int32_t* group_rows, int32_t k, int32_t n_cols, int64_t plane_stride,
+                               const void* pct_in, int32_t pct_in_kind, const void* pct_out, int32_t pct_out_kind,
+                               const void* fold_change, int32_t fold_change_kind, double min_in_group_fraction,
+                               double max_out_group_fraction, double min_fold_change, int32_t compare_abs, uint8_t* keep,
+                               void* stream);
+
 /* ---- cells that express a gene (scanpy rank_genes_groups(pts=True): pct_nz_group / pct_nz_reference) -------------------
  * counts[g * count_group_stride + j] (int32) = cells of group g whose value in gene gene_lb + j satisfies x != 0: -0.0 and
  * explicitly stored zeros do not count, NaN does.  Every element of the batch's [n_groups, n_genes_batch] plane is written
