@@ -808,22 +808,40 @@ __global__ void __launch_bounds__(256) fused_group_kernel(const illico_plan_t pl
     gt.gc[GC_INV_NT * gt.Gs + g] = 1.0 / (double)n_t;
 }
 
-// ---- 3c. epilogue: 24-byte histogram -> (p, U, fold change), in place ---------------------------------------------------
-// Thread = gene, looping over a slice of the groups: the gene's table (weights, multiplicities, f(value)) and scalars
-// stay in registers, so the unrolled 12-slot fold has no loads and no address arithmetic; records of adjacent genes
-// are adjacent, so every warp access is a contiguous 768-byte run.  The fold change is a ratio of means compared at 1e-10:
-// its divisions by the group sizes are multiplications by precomputed reciprocals; everything that feeds the p-value
-// keeps the reference's IEEE operations.
+// ---- 3c. epilogue: 24-byte record -> (p, U, fold change), in place ----------------------------------------------------
+// Thread = gene, looping over a slice of the groups; records of adjacent genes are adjacent, so every warp access is a
+// contiguous 768-byte run, and the next group's record is loaded before the current one is folded.  The gene's slot
+// constants (weight, control multiplicity, f(value)) sit in a private column of shared memory: in registers they would
+// be spilled to the stack.  A CTA none of whose genes has the launch's record kind leaves before any other load.
+// Narrow fold: slots past the warp's highest non-zero counter are skipped (a uniform trip count); every sum is an exact
+// integer below 2^53 and reordered as such, while the f64 `sum` keeps its order (ascending slot, zero counts add
+// nothing).  The fold change is a ratio of means compared at 1e-10: its divisions by the group sizes are multiplications
+// by precomputed reciprocals; everything that feeds the p-value keeps the reference's IEEE operations.
 constexpr int EPI_GROUPS = 16;   // groups per thread
+constexpr int EPI_THREADS = 256;
+struct __align__(16) EpiSlot {
+    uint32_t wgt;   // OVO: 2 #{control > v} + a; OVR: doubled mid-rank
+    uint32_t a;     // OVO: multiplicity in the control
+    double fval;    // f(value) for the fold change
+};
+constexpr int EPI_SMEM = DCAP * EPI_THREADS * (int)sizeof(EpiSlot);   // 48 KB: 4 CTAs per SM
 // SCORE: also writes the score plane (illico_flags_t::scores); a separate instantiation, so that the default call's
 // epilogue is the same code as without the plane.
 template <bool OVO, bool WIDE, bool SCORE>
-__global__ void __launch_bounds__(256, 3) fused_epilogue_kernel(int b, const illico_plan_t pl, const illico_flags_t fl, Gtab gt,
-                                                             int bs, double* __restrict__ results, long long gstride,
-                                                             long long* dbg_u2, double* dbg_tie, long long* dbg_tie_exact,
-                                                             int share_1024) {
+__global__ void __launch_bounds__(EPI_THREADS, 4) fused_epilogue_kernel(int b, const illico_plan_t pl, const illico_flags_t fl, Gtab gt,
+                                                                     int bs, double* __restrict__ results, long long gstride,
+                                                                     int share_1024) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    EpiSlot* const cst = reinterpret_cast<EpiSlot*>(smem) + threadIdx.x;   // slot q of this thread's gene: cst[q * EPI_THREADS]
     __shared__ double gcs[GC_N][EPI_GROUPS];
     __shared__ int nts[EPI_GROUPS];
+    // the batch is being handed back as a whole (the table step flagged too many genes): nothing here will be kept
+    if ((long long)gt.n_bad[0] * 1024 > (long long)b * share_1024) return;
+    // WIDE: the genes of the wide table, whose record is (2U_nz | non-zeros << 40, T_nz, sum) and not a histogram.
+    // The other genes stay in the loop without loads or stores: the narrow fold's trip count is a warp vote.
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool live = j < b && !gt.bad[j] && (gt.mode[j] == 1) == WIDE;
+    if (!__syncthreads_or(live)) return;
     const int G = pl.n_groups, ref = pl.ref_group;
     const int ga = blockIdx.y * EPI_GROUPS, gb = min(G, ga + EPI_GROUPS);
     if (threadIdx.x < GC_N * EPI_GROUPS) {
@@ -834,73 +852,79 @@ __global__ void __launch_bounds__(256, 3) fused_epilogue_kernel(int b, const ill
         if (ga + k < gb) nts[k] = pl.group_size[ga + k];
     }
     __syncthreads();
-    const int j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= b || gt.bad[j]) return;
-    // the batch is being handed back as a whole (the table step flagged too many genes): nothing here will be kept
-    if ((long long)gt.n_bad[0] * 1024 > (long long)b * share_1024) return;
-    // WIDE: the genes of the wide table, whose record is (2U_nz | non-zeros << 40, T_nz, sum) and not a histogram
-    if ((gt.mode[j] == 1) != WIDE) return;
-    uint32_t wgt[WIDE ? 1 : DCAP], mult[(OVO && !WIDE) ? DCAP : 1];
-    double fval[WIDE ? 1 : DCAP];
-    if (!WIDE) {
-#pragma unroll
-        for (int q = 0; q < DCAP; ++q) {
-            wgt[WIDE ? 0 : q] = gt.wgt[(long long)q * bs + j];
-            fval[WIDE ? 0 : q] = gt.fval[(long long)q * bs + j];
-            if (OVO) mult[(OVO && !WIDE) ? q : 0] = gt.mult[(long long)q * bs + j];
-        }
+    if (live && !WIDE) {
+#pragma unroll 4
+        for (int q = 0; q < DCAP; ++q)
+            cst[q * EPI_THREADS] = {gt.wgt[(long long)q * bs + j], OVO ? gt.mult[(long long)q * bs + j] : 0u, gt.fval[(long long)q * bs + j]};
     }
     const long long n = pl.n_cells;
     const double cc = fl.use_continuity ? 0.5 : 0.0;
-    const long long g_nnz = gt.nnz[j];                       // OVO: control non-zeros; OVR: doubled mid-rank of the zero block
-    const unsigned long long g_tie = gt.tie[j];              // OVO: control tie term; OVR: f64 bits of the gene's tie correction
-    const double g_sum = gt.sum[j];                          // OVO: control sum; OVR: whole-gene sum
+    const long long g_nnz = live ? gt.nnz[j] : 0;            // OVO: control non-zeros; OVR: doubled mid-rank of the zero block
+    const unsigned long long g_tie = live ? gt.tie[j] : 0;   // OVO: control tie term; OVR: f64 bits of the gene's tie correction
+    const double g_sum = live ? gt.sum[j] : 0.0;             // OVO: control sum; OVR: whole-gene sum
     const long long n_ref = OVO ? (long long)pl.group_size[ref] : 0;
     const double ovr_tie_corr = __longlong_as_double((long long)g_tie);
     // OVO: the control's mean is a per-gene constant
-    const double ovo_rsum = OVO ? (fl.group_sums ? fl.group_sums[(long long)ref * b + j] : g_sum) : 0.0;
+    const double ovo_rsum = (OVO && live) ? (fl.group_sums ? fl.group_sums[(long long)ref * b + j] : g_sum) : 0.0;
     const double ovo_mean_r = OVO ? ovo_rsum / (double)n_ref : 0.0;
     const double ovo_inv_mean_r = 1.0 / ovo_mean_r;
+    const unsigned long long* rec = reinterpret_cast<const unsigned long long*>(results) + (long long)j * 3;
+    unsigned long long nx0 = 0, nx1 = 0, nx2 = 0;           // the next group's record
+    if (live) { nx0 = rec[(long long)ga * gstride]; nx1 = rec[(long long)ga * gstride + 1]; nx2 = rec[(long long)ga * gstride + 2]; }
     for (int g = ga; g < gb; ++g) {
+        const unsigned long long w0 = nx0, w1 = nx1, w2 = nx2;
+        if (live && g + 1 < gb) {
+            const unsigned long long* r = rec + (long long)(g + 1) * gstride;
+            nx0 = r[0]; nx1 = r[1]; nx2 = r[2];
+        }
         const int k = g - ga;
         const long long n_t = nts[k];
         const long long n_r = OVO ? n_ref : n - n_t;         // the sample U is reported for
         double* o = results + (long long)g * gstride + (long long)j * 3;
-        const long long di = (long long)g * b + j;
         if (OVO && g == ref) {
             // control row: (1, -1, fold change of the control against itself), as ovo_kernel writes it
-            o[0] = 1.0; o[1] = -1.0; o[2] = (ovo_mean_r == 0.0) ? INFINITY : ovo_mean_r / ovo_mean_r;
-            if (SCORE) fl.scores[(long long)g * fl.score_group_stride + j] = 0.0;
-            if (dbg_u2) dbg_u2[di] = -2;
-            if (dbg_tie) dbg_tie[di] = 0.0;
-            if (dbg_tie_exact) dbg_tie_exact[di] = 0;
+            if (live) {
+                o[0] = 1.0; o[1] = -1.0; o[2] = (ovo_mean_r == 0.0) ? INFINITY : ovo_mean_r / ovo_mean_r;
+                if (SCORE) fl.scores[(long long)g * fl.score_group_stride + j] = 0.0;
+            }
             continue;
         }
-        const unsigned long long* r = reinterpret_cast<const unsigned long long*>(o);
-        const unsigned long long wds[3] = {r[0], r[1], r[2]};
         unsigned long long acc = 0, tie_nz = 0;              // acc: OVO 2U without the zero block, OVR 2R without it
         uint32_t m = 0;
         double sum = 0.0;
         if (WIDE) {
-            acc = wds[0] & ((1ull << WIDE_M_SHIFT) - 1ull);
-            m = (uint32_t)(wds[0] >> WIDE_M_SHIFT);
-            tie_nz = wds[1];
-            sum = (double)wds[2];
+            acc = w0 & ((1ull << WIDE_M_SHIFT) - 1ull);
+            m = (uint32_t)(w0 >> WIDE_M_SHIFT);
+            tie_nz = w1;
+            sum = (double)w2;
         } else {
+            int top = 0;                                     // slots to visit: up to the warp's highest non-zero counter
+            if (w0) top = 4 - (__clzll((long long)w0) >> 4);
+            if (w1) top = 8 - (__clzll((long long)w1) >> 4);
+            if (w2) top = 12 - (__clzll((long long)w2) >> 4);
+            top = __reduce_max_sync(FULL, top);
+            const unsigned long long wds[3] = {w0, w1, w2};
+            unsigned long long tq = 0;                       // OVO: sum of bq (3a^2 + bq (3a + bq))
 #pragma unroll
             for (int q = 0; q < DCAP; ++q) {
+                if (q == top) break;
                 const uint32_t bq = (uint32_t)(wds[q >> 2] >> (16 * (q & 3))) & 0xffffu;
-                if (bq) {
-                    acc += (unsigned long long)bq * wgt[WIDE ? 0 : q];
-                    sum += (double)bq * fval[WIDE ? 0 : q];
-                    m += bq;
-                    if (OVO) {
-                        const unsigned long long a = mult[(OVO && !WIDE) ? q : 0];
-                        tie_nz += bq * (3ull * a * a - 1ull + bq * (3ull * a + bq));   // (a+b)^3 - (a+b) - (a^3 - a)
-                    }
+                const EpiSlot c = cst[q * EPI_THREADS];
+                acc += (unsigned long long)bq * c.wgt;
+                const double t = (double)bq * c.fval;
+                sum = bq ? sum + t : sum;                    // (a select: f(value) can be inf, and 0 * inf is NaN)
+                m += bq;
+                if (OVO) {
+                    // (a+b)^3 - (a+b) - (a^3 - a) = b (3a^2 + b (3a + b)) - b; the - b of every slot is - m below.
+                    // 3a < 2^20 and b < 2^16, so every product is a 32 x 32 -> 64-bit multiply-add but the last.
+                    const uint32_t a3 = 3u * c.a;
+                    const unsigned long long x = (unsigned long long)a3 * c.a + (unsigned long long)bq * (a3 + bq);
+                    tq += bq * x;
                 }
             }
+            if (OVO) tie_nz = tq - m;
         }
+        if (!live) continue;
         const long long z_t = n_t - (long long)m;
         double p, U, fc;
         if (OVO) {
@@ -915,9 +939,6 @@ __global__ void __launch_bounds__(256, 3) fused_epilogue_kernel(int b, const ill
             p = pval_core(gcs[GC_NRNT][k], gcs[GC_MU][k], gcs[GC_PROD12][k], tie_corr, U, cc, fl.alternative);
             if (SCORE) fl.scores[(long long)g * fl.score_group_stride + j] = score_core(gcs[GC_MU][k], gcs[GC_PROD12][k], tie_corr, U);
             fc = (ovo_mean_r == 0.0) ? INFINITY : (sum * gcs[GC_INV_NT][k]) * ovo_inv_mean_r;
-            if (dbg_u2) dbg_u2[di] = (long long)u2;
-            if (dbg_tie) dbg_tie[di] = tie;
-            if (dbg_tie_exact) dbg_tie_exact[di] = (long long)tie_exact;
         } else {
             const unsigned long long R2 = acc + (unsigned long long)z_t * (unsigned long long)g_nnz;
             const long long u2 = 2 * n_r * n_t + n_t * (n_t + 1) - (long long)R2;
@@ -931,10 +952,23 @@ __global__ void __launch_bounds__(256, 3) fused_epilogue_kernel(int b, const ill
             const bool all_here = (long long)m == n - (g_nnz - 1);
             const double mu_t = sum * gcs[GC_INV_NT][k], mu_r = all_here ? 0.0 : (g_sum - sum) / (double)(n - n_t);
             fc = (mu_r == 0.0) ? INFINITY : mu_t / mu_r;
-            if (dbg_u2) dbg_u2[di] = u2;
         }
         o[0] = p; o[1] = U; o[2] = fc;
     }
+}
+
+// the epilogue of the narrow records (WIDE = false) or of the wide ones, for the dense and the CSR path
+template <bool OVO, bool WIDE>
+int launch_fused_epilogue(int b, const illico_plan_t* plan, const illico_flags_t* flags, Gtab gt, int bs, double* results,
+                          long long gstride, int share_1024, cudaStream_t stream) {
+    auto epi = flags->scores ? fused_epilogue_kernel<OVO, WIDE, true> : fused_epilogue_kernel<OVO, WIDE, false>;
+    const int smem = WIDE ? 0 : EPI_SMEM;
+    ILLICO_CUDA_OK(cudaFuncSetAttribute(epi, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    const dim3 grid((unsigned)((b + EPI_THREADS - 1) / EPI_THREADS), (unsigned)((plan->n_groups + EPI_GROUPS - 1) / EPI_GROUPS));
+    ILLICO_LAUNCH(WIDE ? "fused_wide_epilogue_kernel" : "fused_epilogue_kernel", stream,
+                  epi<<<grid, EPI_THREADS, smem, stream>>>(b, *plan, *flags, gt, bs, results, gstride, share_1024));
+    ILLICO_CUDA_OK(cudaGetLastError());
+    return 0;
 }
 
 // ===================== CSR input: the same histograms, built in shared memory ==========================================
@@ -1246,16 +1280,8 @@ int run_fused(const float* X, long long ld, int gene_lb, int b, const illico_pla
     ILLICO_LAUNCH("fused_group_kernel", stream, fused_group_kernel<OVO><<<(plan->n_groups + 255) / 256, 256, 0, stream>>>(*plan, gt));
     ILLICO_LAUNCH("fused_gene_kernel", stream, fused_gene_kernel<OVO><<<(b + 127) / 128, 128, 0, stream>>>(b, *plan, *flags, gt, bs, nullptr, nullptr));
     ILLICO_CUDA_OK(cudaGetLastError());
-    const bool score = flags->scores != nullptr;
-    auto epi = score ? fused_epilogue_kernel<OVO, false, true> : fused_epilogue_kernel<OVO, false, false>;
-    ILLICO_LAUNCH("fused_epilogue_kernel", stream, epi<<<dim3((unsigned)((b + 255) / 256), (unsigned)((plan->n_groups + EPI_GROUPS - 1) / EPI_GROUPS)), 256, 0, stream>>>(
-            b, *plan, *flags, gt, bs, results, gstride, nullptr, nullptr, nullptr, list_share_1024()));
-    if (wide_on) {
-        auto wepi = score ? fused_epilogue_kernel<OVO, true, true> : fused_epilogue_kernel<OVO, true, false>;
-        ILLICO_LAUNCH("fused_wide_epilogue_kernel", stream, wepi<<<dim3((unsigned)((b + 255) / 256), (unsigned)((plan->n_groups + EPI_GROUPS - 1) / EPI_GROUPS)), 256, 0, stream>>>(
-                b, *plan, *flags, gt, bs, results, gstride, nullptr, nullptr, nullptr, list_share_1024()));
-    }
-    ILLICO_CUDA_OK(cudaGetLastError());
+    if (launch_fused_epilogue<OVO, false>(b, plan, flags, gt, bs, results, gstride, list_share_1024(), stream)) return 1;
+    if (wide_on && launch_fused_epilogue<OVO, true>(b, plan, flags, gt, bs, results, gstride, list_share_1024(), stream)) return 1;
 
     // 4. genes handed back: listed on the device, staged from the matrix by a persistent kernel, ranked by the general
     // path with the device-side count (an empty list costs three nearly empty launches)
@@ -1345,10 +1371,7 @@ int run_fused_csr(const float* data, const int32_t* indices, const long long* in
     }
     ILLICO_LAUNCH("fused_group_kernel", stream, fused_group_kernel<OVO><<<(plan->n_groups + 255) / 256, 256, 0, stream>>>(*plan, gt));
     ILLICO_LAUNCH("fused_gene_kernel", stream, fused_gene_kernel<OVO><<<(b + 127) / 128, 128, 0, stream>>>(b, *plan, *flags, gt, bs, nullptr, nullptr));
-    auto epi = flags->scores ? fused_epilogue_kernel<OVO, false, true> : fused_epilogue_kernel<OVO, false, false>;
-    ILLICO_LAUNCH("fused_epilogue_kernel", stream, epi<<<dim3((unsigned)((b + 255) / 256), (unsigned)((G + EPI_GROUPS - 1) / EPI_GROUPS)), 256, 0, stream>>>(
-            b, *plan, *flags, gt, bs, results, gstride, nullptr, nullptr, nullptr, 128));   // (the CSR pass stops at an eighth)
-    ILLICO_CUDA_OK(cudaGetLastError());
+    if (launch_fused_epilogue<OVO, false>(b, plan, flags, gt, bs, results, gstride, 128, stream)) return 1;   // (the CSR pass stops at an eighth)
 
     // hand-back, decided on the device: a few scattered genes -> one filtered pass over the stored values (HB_LIST);
     // many (or a pass that stopped early: 8 n_bad > b) -> the general CSR staging of the whole batch (HB_ALL)
